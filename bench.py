@@ -7,7 +7,7 @@ Workload = configs[2]: Matern-5/2 ARD, d=16, N=32768 on one GPU; one "step" is
 one optimiser objective evaluation = set_hyper (Gram + Cholesky + solve) +
 loglikelihood(grad=True).  Synthetic data per SURVEY.md section 8d.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 (torchrun, one rank per GPU): the N = 32768 evaluation fits one GPU and its
 optimiser loop is sequential ("replicas only", DESIGN.md section 6) -- `value` is the
@@ -349,6 +349,11 @@ def run_ours(args):
     t_max = max_over_ranks(max(dev_s, 0.0), world)
     value = world*K/t_max
     assert np.isfinite(lZ) and np.all(np.isfinite(dlZ))
+    if args.dump_outputs and rank == 0:
+        # what the last timed step returned to its caller, for output-by-output comparison of two builds
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, 'lZ.npy'), np.asarray(lZ, dtype=np.float64))
+        np.save(os.path.join(args.dump_outputs, 'dlZ.npy'), np.asarray(dlZ, dtype=np.float64))
 
     # ---- e2e: public API with host buffers, H2D of X, y and D2H of (lZ, dlZ) each step --
     del gp
@@ -617,7 +622,13 @@ def main():
                     help='skip dist_chol_n65536 / predict_strong / mcmc_4096x2048')
     ap.add_argument('--predict-pts', type=int, default=16384, dest='predict_pts', help='test points per rank')
     ap.add_argument('--no-cpu', action='store_true', dest='no_cpu')
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR',
+                    help='write lZ and dlZ of the last timed step (rank 0) as DIR/lZ.npy, DIR/dlZ.npy in float64')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -1,11 +1,11 @@
 """
 TEST INFRASTRUCTURE ONLY -- import the UNMODIFIED reference (Python-2 era
-mwhoffman/pygp under /root/reference) in the build container.
+mwhoffman/pygp; PYGP_REFERENCE_ROOT names a source checkout of it).
 
-Nothing under /root/reference is edited or copied; the py2-isms are bridged at
-run time (SURVEY.md section 8c).  /root/reference does not exist on the GPU
-box, so this module is used only by ``oracle/make_golden.py`` (and by
-``tests/test_oracle.py::test_live_reference`` which skips when it is absent).
+Nothing in that checkout is edited or copied; the py2-isms are bridged at
+run time (SURVEY.md section 8c).  The reference is not part of this
+repository, so only ``oracle/make_golden.py`` uses this module: it records the
+reference's outputs under tests/golden, which the tests compare against.
 """
 
 import builtins

@@ -8,8 +8,7 @@ import numpy.testing as nt
 import pytest
 import scipy.optimize as spop
 
-from oracle import ref_loader
-from oracle.cases import (KERNEL_CASES, GP_CASES, SURVEY_KAT, GP_SN, GP_MEAN,
+from oracle.cases import (KERNEL_CASES, GP_CASES, DTC_CASES, SURVEY_KAT, GP_SN, GP_MEAN,
                           kernel_inputs, gp_inputs)
 from oracle.pygp_oracle import make_kernel, OExactGP, OFITC
 
@@ -113,13 +112,42 @@ def test_gp_grad_fd(name):
     nt.assert_allclose(g1, spop.approx_fprime(h, f, 1e-8), rtol=1e-4, atol=1e-4)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='reference tree absent (GPU box)')
-def test_live_reference():
-    """In the build container: the restatement equals the live reference."""
-    from oracle import make_golden
-    pygp = ref_loader.load()
-    make_golden.kernel_golden(pygp)
-    make_golden.gp_golden(pygp)
+@pytest.mark.parametrize('name', sorted(GP_CASES) + sorted(DTC_CASES))
+def test_reference_record(name, golden):
+    """The reference outputs in tests/golden that the other golden tests leave unchecked: the
+    hyper layout, the exact-GP factor R and whitened residual a, and the outputs after
+    set_hyper(hyper2), at the tolerances oracle/make_golden.py compared them with when it
+    recorded them (its default 1e-12 / 1e-13 for R, a and the exact/FITC posterior after
+    set_hyper, which it stored unchecked).  With them every stored reference array is compared."""
+    from oracle.pygp_oracle import ODTC
+    g = golden['gp']
+    if name in DTC_CASES:
+        spec, N, d = DTC_CASES[name]
+        X, y, Xs, U = gp_inputs(N, d, True)
+        gp = ODTC(GP_SN, make_kernel(spec), GP_MEAN, U)
+        gp.add_data(X, y)
+        nt.assert_allclose(gp.full_posterior(Xs)[1], g[name + '/full_Sigma'], rtol=1e-8, atol=1e-11)
+        gp.set_hyper(g[name + '/hyper2'])
+        lZ, dlZ = gp.loglikelihood(True)
+        mu, s2, dmu, ds2 = gp.posterior(Xs, grad=True)
+        nt.assert_allclose(lZ, g[name + '/lZ_h2'], rtol=1e-12)
+        nt.assert_allclose(dlZ, g[name + '/dlZ_h2'], rtol=1e-9, atol=1e-10)
+        nt.assert_allclose(mu, g[name + '/mu_h2'], rtol=1e-10, atol=1e-12)
+        nt.assert_allclose(s2, g[name + '/s2_h2'], rtol=1e-9, atol=1e-12)
+        nt.assert_allclose(dmu, g[name + '/dmu_h2'], rtol=1e-9, atol=1e-11)
+        nt.assert_allclose(ds2, g[name + '/ds2_h2'], rtol=1e-8, atol=1e-11)
+        nt.assert_allclose(gp.full_posterior(Xs)[1], g[name + '/full_Sigma_h2'], rtol=1e-8, atol=1e-11)
+        return
+    gp, Xs = _build(name)
+    nt.assert_array_equal(gp.get_hyper(), g[name + '/hyper'])
+    if not GP_CASES[name][3]:
+        R = g[name + '/R']
+        nt.assert_allclose(gp._R[:R.shape[0], :R.shape[1]], R, rtol=1e-12, atol=1e-13)
+        nt.assert_allclose(gp._a, g[name + '/a'], rtol=1e-12, atol=1e-13)
+    gp.set_hyper(g[name + '/hyper2'])
+    mu, s2 = gp.posterior(Xs)
+    nt.assert_allclose(mu, g[name + '/mu_h2'], rtol=1e-12, atol=1e-13)
+    nt.assert_allclose(s2, g[name + '/s2_h2'], rtol=1e-11, atol=1e-13)
 
 
 @pytest.mark.parametrize('name', ['fitc_se_2d', 'fitc_ard4_500'])
