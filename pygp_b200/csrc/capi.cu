@@ -854,7 +854,7 @@ extern "C" int pgp_exact_loglike(pgp_model* m, int want_grad, double* lZ, double
     H.p = m->d_H; H.ld = ld;
     PGP_TRY(inv_upper(ctx, G, F, n, H));                                     // V = L^-T
     PGP_TRY(launch_gemv_upper(ctx, m->d_G, ld, m->d_F + n * ld, n, m->d_alpha));  // alpha = V a
-    PGP_TRY(syrk_upper_lower(ctx, H, G, n));                                // K~^-1 = V V^T
+    PGP_TRY(syrk_upper_lower_single(ctx, H, G, n));                         // K~^-1 = V V^T
     TraceArgs t;
     t.spec = m->d_spec;
     t.Z = m->d_Z;

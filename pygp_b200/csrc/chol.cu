@@ -20,6 +20,7 @@
 #include <cstdlib>
 
 #include "chol.cuh"
+#include "ozaki.cuh"
 #include "spec.cuh"
 
 namespace pgp {
@@ -698,6 +699,17 @@ int syrk_upper_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n) {
     if (n <= 0) return 0;
     return gemm_update(ctx, G.p, G.ld, G.bstride, G.p, G.ld, G.bstride, H.p, H.ld, H.bstride, n, n, n, 1.0, 0.0,
                        /*tri=*/1, /*krow=*/1, G.batch);
+}
+
+// From this order on, the gradient of ONE model computes V V^T as the emulated-FP64 INT8 product of
+// ozaki.cu (split + residue products + merge beat one DMMA launch: tools/ozaki_sweep.py,
+// profiles/r03_ozaki_sweep.txt).  The batched gradient keeps syrk_upper_lower: it runs problems side by
+// side on several streams, and the emulated product's multi-GiB scratch is pooled for one stream only.
+constexpr int64_t kOzakiMinN = 8192;
+
+int syrk_upper_lower_single(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n) {
+    if (G.batch == 1 && n >= kOzakiMinN && n <= oz::kMaxK) return ozaki_syrk_lower(ctx, H, G, n);
+    return syrk_upper_lower(ctx, H, G, n);
 }
 
 // ---------------------------------------------------------------------------

@@ -66,6 +66,9 @@ int inv_upper(pgp_ctx* ctx, const Mat& G, const Mat& L, int64_t n, const Mat& S)
 
 // H lower triangle <- G G^T with G upper triangular (= K~^-1 when G = L^-T).
 int syrk_upper_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n);
+// the same for the gradient of one model on the context stream: the emulated-FP64 INT8 product (ozaki.cu)
+// for large n, syrk_upper_lower below
+int syrk_upper_lower_single(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n);
 
 // out[b] = -1/2 |a|^2 - n/2 log 2 pi - sum log L_ii, a = row n of F (exact.py:119-121)
 int launch_loglik(pgp_ctx* ctx, const Mat& F, int64_t n, double* d_out);
