@@ -703,8 +703,10 @@ int syrk_upper_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n) {
 
 // From this order on, the gradient of ONE model computes V V^T as the emulated-FP64 INT8 product of
 // ozaki.cu (split + residue products + merge beat one DMMA launch: tools/ozaki_sweep.py,
-// profiles/r03_ozaki_sweep.txt).  The batched gradient keeps syrk_upper_lower: it runs problems side by
-// side on several streams, and the emulated product's multi-GiB scratch is pooled for one stream only.
+// profiles/r04_ozaki_sweep.txt: 1.75x at 8192; at 4096 it wins by 1.09x, 0.07 ms of a call whose
+// gradient costs far more, which does not pay for changing the bits of H from 4096 on).  The batched
+// gradient keeps syrk_upper_lower: it runs problems side by side on several streams, and the emulated
+// product's multi-GiB scratch is pooled for one stream only.
 constexpr int64_t kOzakiMinN = 8192;
 
 int syrk_upper_lower_single(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n) {

@@ -20,7 +20,6 @@ constexpr int kStageB = 2 * kChunkBytes;             // 256 rows x 128 k
 constexpr int kStageBytes = kStageA + kStageB;
 constexpr size_t kSyrkSmem = (size_t)kStages * kStageBytes + 1024;   // + alignment slack
 constexpr int kSyrkThreads = 192;                    // warp 0 copies, warp 1 MMAs, warps 2-5 epilogue
-constexpr int64_t kStripBytes = (int64_t)4 << 30;
 
 // inverse of m_j modulo m_t (balanced), j < t
 __constant__ float kInv[kMods][kMods] = {
@@ -51,6 +50,7 @@ __global__ void __launch_bounds__(256) ozaki_rowexp_kernel(const double* __restr
     double a = 0.0;
     bool finite = true;
     if (i < n)
+#pragma unroll 4
         for (int64_t k = i + lane; k < n; k += 32) {
             const double v = G[i * ld + k];
             finite &= isfinite(v);
@@ -63,8 +63,10 @@ __global__ void __launch_bounds__(256) ozaki_rowexp_kernel(const double* __restr
 }
 
 // ---- split: one CTA per (kb, rb) chunk, all moduli ----------------------------------------------
-// thread: 4 units of 16 consecutive k of one row; each unit is one 16-byte store per modulus
-__global__ void __launch_bounds__(256) ozaki_split_kernel(const double* __restrict__ G, int64_t ld, Layout L,
+// thread: 4 units of 16 consecutive k of one row; each unit is eight 16-byte loads of V and one 16-byte
+// store per modulus.  A unit that starts below n lies inside the row's ld (a multiple of 16), so it is
+// loaded whole and the entries left of the diagonal or beyond n are zeroed after the load.
+__global__ void __launch_bounds__(256, 1) ozaki_split_kernel(const double* __restrict__ G, int64_t ld, Layout L,
                                                           const int* __restrict__ exps, int8_t* __restrict__ res) {
     const int64_t c = blockIdx.x;
     int kb = (int)((sqrt(9.0 + 8.0 * (double)c) - 3.0) * 0.5);
@@ -80,12 +82,15 @@ __global__ void __launch_bounds__(256) ozaki_split_kernel(const double* __restri
         const int64_t k0 = (int64_t)kb * kRB + s * 16;
         long long x[16];
         const int e = i < n ? exps[i] : kNonFinite;
-        if (e != kNonFinite) {
-            const double* g = G + i * ld;
+        if (e != kNonFinite && k0 < n) {
+            const double2* g = reinterpret_cast<const double2*>(G + i * ld + k0);
+            double2 p[8];
+#pragma unroll
+            for (int h = 0; h < 8; ++h) p[h] = g[h];
 #pragma unroll
             for (int h = 0; h < 16; ++h) {
                 const int64_t k = k0 + h;
-                const double v = (k >= i && k < n) ? g[k] : 0.0;
+                const double v = (k >= i && k < n) ? ((h & 1) ? p[h >> 1].y : p[h >> 1].x) : 0.0;
                 x[h] = __double2ll_rn(ldexp(v, e));
             }
         } else {
@@ -164,39 +169,38 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, int (&v)[32]) {
                  : "memory");
 }
 
-// item -> (t, tile): t outermost so that the CTAs in flight share operand chunks in L2; inside a
-// modulus the tiles run row block by row block, longest contraction (smallest I) first
+// item -> (t, tile): t outermost, inside a modulus the tiles in raster_tile order (ozaki.cuh)
 struct Item {
     int t, I, J;
-    int64_t tile_local;
+    int64_t tile_local;                      // row-block-major number in the strip (out_offset)
 };
 __device__ __forceinline__ Item decode_item(int64_t item, int64_t strip_tiles, int I0, int I1) {
     Item it;
     it.t = (int)(item / strip_tiles);
-    it.tile_local = item - (int64_t)it.t * strip_tiles;
-    const int64_t g = tiles_before(I0) + it.tile_local;
-    int lo = I0, hi = I1 - 1;                // largest I with tiles_before(I) <= g
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (tiles_before(mid) <= g) lo = mid;
-        else hi = mid - 1;
-    }
-    it.I = lo;
-    it.J = (int)(g - tiles_before(lo));
+    raster_tile(item - (int64_t)it.t * strip_tiles, I0, I1, it.I, it.J);
+    it.tile_local = tiles_before(it.I) - tiles_before(I0) + it.J;
     return it;
 }
 
 // ---- the residue products: persistent CTAs over (modulus, lower tile) items ---------------------
+// Items are handed out in order from a global counter, one at a time to whichever CTA is free, so the
+// tiles in flight stay a compact window of the raster order (a static stride lets CTAs drift apart by
+// many items, as item lengths differ).  The copy thread takes the item and passes it on through a ring
+// of kItemSlots shared-memory slots to the MMA thread and the epilogue warps.
 // warp 0: one thread streams the A chunk (row block I) and the B chunk pair (row blocks 2J, 2J + 1) of
 //         every k-block into a kStages-deep ring (bulk copies, completion on full[s]);
 // warp 1: allocates 512 tensor-memory columns (two 128 x 256 s32 accumulators); one thread issues
 //         4 MMAs (K = 32 bytes each) per stage and frees the stage by tcgen05.commit to empty[s];
 // warps 2-5: epilogue of the other accumulator -- tcgen05.ld, mod m_t, one byte per entry.
+constexpr int kItemSlots = 8;
 __global__ void __launch_bounds__(kSyrkThreads, 1) ozaki_syrk_kernel(const int8_t* __restrict__ res, Layout L, int I0,
-                                                                     int I1, int64_t strip_tiles,
+                                                                     int I1, int64_t strip_tiles, int64_t chunk_mask,
+                                                                     unsigned* __restrict__ next_item,
                                                                      uint8_t* __restrict__ out) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t full[kStages], empty[kStages], tfull[2], tempty[2];
+    __shared__ __align__(8) uint64_t ifull[kItemSlots], iempty[kItemSlots];
+    __shared__ int64_t item_slot[kItemSlots];
     __shared__ uint32_t tmem_base_sh;
     const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -212,6 +216,10 @@ __global__ void __launch_bounds__(kSyrkThreads, 1) ozaki_syrk_kernel(const int8_
             mbar_init(&tfull[a], 1);
             mbar_init(&tempty[a], 4);
         }
+        for (int q = 0; q < kItemSlots; ++q) {
+            mbar_init(&ifull[q], 1);
+            mbar_init(&iempty[q], 5);            // the MMA thread and the four epilogue warps
+        }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -223,18 +231,33 @@ __global__ void __launch_bounds__(kSyrkThreads, 1) ozaki_syrk_kernel(const int8_
     tc_fence_after();
     const uint32_t tmem = tmem_base_sh;
 
+    // the item of the n-th turn, as the copy thread published it (>= items: no more)
+    auto take_item = [&](int n_it) {
+        const int q = n_it % kItemSlots;
+        mbar_wait(&ifull[q], (n_it / kItemSlots) & 1);
+        return item_slot[q];
+    };
+    auto release_item = [&](int n_it) { mbar_arrive(&iempty[n_it % kItemSlots]); };
+
     if (warp == 0) {
         if (lane == 0) {
             int s = 0;
             uint32_t ph = 0;
-            for (int64_t item = blockIdx.x; item < items; item += gridDim.x) {
+            for (int n_it = 0;; ++n_it) {
+                const int q = n_it % kItemSlots;
+                mbar_wait(&iempty[q], ((n_it / kItemSlots) & 1) ^ 1);
+                const int64_t item = atomicAdd(next_item, 1u);
+                item_slot[q] = item;
+                mbar_arrive(&ifull[q]);
+                if (item >= items) break;
                 const Item it = decode_item(item, strip_tiles, I0, I1);
                 for (int kb = it.I; kb < nkb; ++kb) {
                     mbar_wait(&empty[s], ph ^ 1);
                     mbar_expect_tx(&full[s], kStageBytes);
                     const uint32_t dst = sbase + s * kStageBytes;
-                    bulk_g2s(dst, res + L.chunk_index(it.t, kb, it.I) * kChunkBytes, kStageA, &full[s]);
-                    bulk_g2s(dst + kStageA, res + L.chunk_index(it.t, kb, 2 * it.J) * kChunkBytes, kStageB, &full[s]);
+                    bulk_g2s(dst, res + (L.chunk_index(it.t, kb, it.I) & chunk_mask) * kChunkBytes, kStageA, &full[s]);
+                    bulk_g2s(dst + kStageA, res + (L.chunk_index(it.t, kb, 2 * it.J) & chunk_mask) * kChunkBytes, kStageB,
+                             &full[s]);
                     if (++s == kStages) { s = 0; ph ^= 1; }
                 }
             }
@@ -243,8 +266,10 @@ __global__ void __launch_bounds__(kSyrkThreads, 1) ozaki_syrk_kernel(const int8_
         if (lane == 0) {
             int s = 0;
             uint32_t ph = 0;
-            int n_it = 0;
-            for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++n_it) {
+            for (int n_it = 0;; ++n_it) {
+                const int64_t item = take_item(n_it);
+                release_item(n_it);
+                if (item >= items) break;
                 const Item it = decode_item(item, strip_tiles, I0, I1);
                 const int a = n_it & 1;
                 mbar_wait(&tempty[a], ((n_it >> 1) & 1) ^ 1);
@@ -266,8 +291,11 @@ __global__ void __launch_bounds__(kSyrkThreads, 1) ozaki_syrk_kernel(const int8_
     } else {
         const int quarter = warp & 3;            // tcgen05.ld reaches lanes 32 (warp % 4) .. + 31
         const int row = quarter * 32 + lane;
-        int n_it = 0;
-        for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++n_it) {
+        for (int n_it = 0;; ++n_it) {
+            const int64_t item = take_item(n_it);
+            __syncwarp();
+            if (lane == 0) release_item(n_it);
+            if (item >= items) break;
             const Item it = decode_item(item, strip_tiles, I0, I1);
             const int a = n_it & 1;
             const int m = modulus(it.t);
@@ -313,8 +341,20 @@ __global__ void __launch_bounds__(kSyrkThreads, 1) ozaki_syrk_kernel(const int8_
 }
 
 // ---- merge: one CTA per tile; thread = 4 consecutive columns of every 4th row ---------------------
-__global__ void __launch_bounds__(256) ozaki_merge_kernel(const uint8_t* __restrict__ out, const int* __restrict__ exps,
-                                                          int64_t n, int I0, int I1, double* __restrict__ H, int64_t ldh) {
+// The four entries of a thread are reconstructed side by side (independent chains for the scheduler) and,
+// away from the diagonal and the edge, stored as two 16-byte stores.
+//
+// rint_neg(y) = -rint(y) for |y| < 2^22, as two FP32 adds (the sum with 1.5 2^23 rounds y to an integer,
+// ties to even like rintf) instead of FRND, which issues at a fraction of the FP32 rate.  A zero result is
+// +0 where -rintf gives -0 for y in [+0, 0.5]; it only feeds fmaf(rint_neg(y), m, x) with y = x / m, whose
+// value (x, or +0 for x = +-0) is the same either way, so every digit is the same bits as with rintf.
+__device__ __forceinline__ float rint_neg(float y) {
+    constexpr float kRound = 12582912.0f;    // 1.5 * 2^23
+    return __fsub_rn(kRound, __fadd_rn(y, kRound));
+}
+
+__global__ void __launch_bounds__(256, 1) ozaki_merge_kernel(const uint8_t* __restrict__ out, const int* __restrict__ exps,
+                                                             int64_t n, int I0, int I1, double* __restrict__ H, int64_t ldh) {
     const int64_t tile_local = blockIdx.x;
     const int64_t g = tiles_before(I0) + tile_local;
     int I = I0;
@@ -333,43 +373,51 @@ __global__ void __launch_bounds__(256) ozaki_merge_kernel(const uint8_t* __restr
         uint32_t w[kMods];
 #pragma unroll
         for (int t = 0; t < kMods; ++t) w[t] = *reinterpret_cast<const uint32_t*>(out + out_offset(tile_local, t, r, 4 * cg));
+        // balanced mixed-radix digits: v_t = ((r_t - v_0) / m_0 - v_1) / m_1 ... mod m_t, all in float:
+        // |operands| <= 383 * 126 < 2^24, and the rounded quotient leaves |v_t| <= m_t / 2
+        float v[4][kMods];
 #pragma unroll
-        for (int h = 0; h < 4; ++h) {
-            const int64_t j = j0 + h;
-            if (j > i || j >= n) continue;
-            // balanced mixed-radix digits: v_t = ((r_t - v_0) / m_0 - v_1) / m_1 ... mod m_t, all in
-            // float: |operands| <= 383 * 126 < 2^24, and the rounded quotient leaves |v_t| <= m_t / 2
-            float v[kMods];
+        for (int t = 0; t < kMods; ++t) {
+            const float m = (float)modulus(t), minv = 1.0f / m;
 #pragma unroll
-            for (int t = 0; t < kMods; ++t) {
-                const float m = (float)modulus(t), minv = 1.0f / m;
-                float u = (float)((w[t] >> (8 * h)) & 0xffu);
+            for (int h = 0; h < 4; ++h) {
+                // byte h of w[t] as a float: 2^23 + byte, exactly, minus 2^23
+                float u = __fsub_rn(__uint_as_float(__byte_perm(w[t], 0x4B000000u, 0x7654u & 0xfff0u | h)), 8388608.0f);
 #pragma unroll
                 for (int q = 0; q < t; ++q) {
-                    const float x = (u - v[q]) * kInv[t][q];
-                    u = fmaf(-rintf(x * minv), m, x);
+                    const float x = __fmul_rn(__fsub_rn(u, v[h][q]), kInv[t][q]);
+                    u = fmaf(rint_neg(__fmul_rn(x, minv)), m, x);
                 }
-                if (t == 0) u = fmaf(-rintf(u * minv), m, u);
-                v[t] = u;
+                if (t == 0) u = fmaf(rint_neg(__fmul_rn(u, minv)), m, u);
+                v[h][t] = u;
             }
-            double x = (double)v[kMods - 1];
+        }
+        double z[4];
 #pragma unroll
-            for (int t = kMods - 2; t >= 0; --t) x = fma(x, (double)modulus(t), (double)v[t]);
-            H[i * ldh + j] = (ei == kNonFinite || ej[h] == kNonFinite) ? __longlong_as_double(0x7ff8000000000000LL)
-                                                                      : ldexp(x, -(ei + ej[h]));
+        for (int h = 0; h < 4; ++h) {
+            double x = (double)v[h][kMods - 1];
+#pragma unroll
+            for (int t = kMods - 2; t >= 0; --t) x = fma(x, (double)modulus(t), (double)v[h][t]);
+            z[h] = (ei == kNonFinite || ej[h] == kNonFinite) ? __longlong_as_double(0x7ff8000000000000LL)
+                                                             : ldexp(x, -(ei + ej[h]));
+        }
+        double* o = H + i * ldh + j0;
+        if (j0 + 3 <= i && j0 + 3 < n && (ldh & 1) == 0) {
+            reinterpret_cast<double2*>(o)[0] = make_double2(z[0], z[1]);
+            reinterpret_cast<double2*>(o)[1] = make_double2(z[2], z[3]);
+        } else {
+#pragma unroll
+            for (int h = 0; h < 4; ++h)
+                if (j0 + h <= i && j0 + h < n) o[h] = z[h];
         }
     }
-}
-
-int64_t strip_end(int I0, int nrb, int64_t max_tiles) {
-    int I1 = I0 + 1;
-    while (I1 < nrb && tiles_before(I1 + 1) - tiles_before(I0) <= max_tiles) ++I1;
-    return I1;
 }
 
 }  // namespace
 
 int ozaki_split(pgp_ctx* ctx, const double* G, int64_t ld, int64_t n, int* exps, int8_t* res) {
+    if (ld % 16 || ld < n || reinterpret_cast<uintptr_t>(G) % 16)
+        return ctx->fail(PGP_E_ARG, "emulated V V^T: V needs a 16-byte aligned base and ld a multiple of 16");
     const Layout L = make_layout(n);
     const int64_t rows = (int64_t)L.nrbp * kRB;
     {
@@ -382,7 +430,7 @@ int ozaki_split(pgp_ctx* ctx, const double* G, int64_t ld, int64_t n, int* exps,
     return check_launch(ctx, "ozaki_split_kernel");
 }
 
-int ozaki_products(pgp_ctx* ctx, const int8_t* res, int64_t n, int I0, int I1, uint8_t* out) {
+int ozaki_products(pgp_ctx* ctx, const int8_t* res, int64_t n, int I0, int I1, uint8_t* out, int64_t resident_chunks) {
     const Layout L = make_layout(n);
     const int64_t strip_tiles = tiles_before(I1) - tiles_before(I0);
     if (strip_tiles <= 0) return 0;
@@ -391,9 +439,19 @@ int ozaki_products(pgp_ctx* ctx, const int8_t* res, int64_t n, int I0, int I1, u
     for (int I = I0; I < I1; ++I) macs += (double)(I / 2 + 1) * kRB * kBN * (double)(L.nrb - I) * kRB * kMods;
     const int64_t items = strip_tiles * kMods;
     const unsigned grid = (unsigned)std::min<int64_t>(items, ctx->sm_count);
-    Launch Lc(ctx, PC_OTHER, 2.0 * macs);
-    ozaki_syrk_kernel<<<grid, kSyrkThreads, kSyrkSmem, ctx->stream>>>(res, L, I0, I1, strip_tiles, out);
-    return check_launch(ctx, "ozaki_syrk_kernel");
+    unsigned* next_item = nullptr;               // the item counter, zero at the start of every launch
+    PGP_TRY(dev_alloc(ctx, &next_item, 1));
+    const cudaError_t e = cudaMemsetAsync(next_item, 0, sizeof(unsigned), ctx->stream);
+    int rc = e == cudaSuccess ? 0 : ctx->cuda_fail(e, "cudaMemsetAsync(item counter)", __FILE__, __LINE__);
+    if (!rc) {
+        Launch Lc(ctx, PC_OTHER, 2.0 * macs);
+        const int64_t mask = resident_chunks > 0 ? resident_chunks - 1 : -1;
+        ozaki_syrk_kernel<<<grid, kSyrkThreads, kSyrkSmem, ctx->stream>>>(res, L, I0, I1, strip_tiles, mask, next_item,
+                                                                          out);
+        rc = check_launch(ctx, "ozaki_syrk_kernel");
+    }
+    dev_free(ctx, next_item);
+    return rc;
 }
 
 int ozaki_merge(pgp_ctx* ctx, const uint8_t* out, const int* exps, int64_t n, int I0, int I1, double* H, int64_t ldh) {
@@ -404,15 +462,15 @@ int ozaki_merge(pgp_ctx* ctx, const uint8_t* out, const int* exps, int64_t n, in
     return check_launch(ctx, "ozaki_merge_kernel");
 }
 
-int ozaki_syrk_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n) {
+int ozaki_syrk_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n, int64_t strip_bytes) {
     if (n <= 0) return 0;
     if (n > kMaxK) return ctx->fail(PGP_E_ARG, "emulated V V^T: contraction longer than 65536 overflows int32");
     if (G.batch != 1 || H.batch != 1) return ctx->fail(PGP_E_ARG, "emulated V V^T: not batched");
     const Layout L = make_layout(n);
-    const int64_t max_tiles = std::max<int64_t>(1, kStripBytes / (kMods * kTileOutBytes));
+    const int64_t max_tiles = strip_max_tiles(strip_bytes);
     int64_t strip_max = 0;
     for (int I0 = 0; I0 < L.nrb;) {
-        const int I1 = (int)strip_end(I0, L.nrb, max_tiles);
+        const int I1 = strip_end(I0, L.nrb, max_tiles);
         strip_max = std::max(strip_max, tiles_before(I1) - tiles_before(I0));
         I0 = I1;
     }
@@ -424,7 +482,7 @@ int ozaki_syrk_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n) {
     if (!rc) rc = dev_alloc(ctx, &out, (size_t)strip_max * kMods * kTileOutBytes);
     if (!rc) rc = ozaki_split(ctx, G.p, G.ld, n, exps, res);
     for (int I0 = 0; !rc && I0 < L.nrb;) {
-        const int I1 = (int)strip_end(I0, L.nrb, max_tiles);
+        const int I1 = strip_end(I0, L.nrb, max_tiles);
         rc = ozaki_products(ctx, res, n, I0, I1, out);
         if (!rc) rc = ozaki_merge(ctx, out, exps, n, I0, I1, H.p, H.ld);
         I0 = I1;

@@ -16,6 +16,8 @@
 // Shared by ozaki.cu (the kernels) and tools/ozaki_check.cu (exactness harness and timer).
 #pragma once
 
+#include <algorithm>
+
 #include "chol.cuh"
 
 namespace pgp {
@@ -39,15 +41,16 @@ __host__ __device__ constexpr int modulus(int t) {
     }
 }
 
-// balanced residue of a signed integer |x| < 2^62, exact in integer arithmetic (an FP64 remainder of
-// a value above 2^53 is not): x = hi 2^31 + lo, 0 <= lo < 2^31, |hi| < 2^31
+// balanced residue of a signed integer |x| < 2^63, exact, with no division: x = l0 + l1 2^16 + l2 2^32 + l3 2^48
+// (l0, l1, l2 in [0, 2^16), l3 in [-2^15, 2^15)), so with c_j = 2^(16 j) mod m
+//   s = l0 + l1 c1 + l2 c2 + (l3 + 2^15) c3 + (m - 2^15 c3 mod m)  ==  x (mod m),  0 <= s < 2^26,
+// and s mod m for a constant m is a multiply-high and a multiply-add
 __host__ __device__ inline int residue(long long x, int m) {
-    const int hi = (int)(x >> 31);
-    const int lo = (int)(x & 0x7fffffffLL);
-    const int p31 = (int)((1LL << 31) % m);
-    int r = (hi % m) * p31 + lo % m;         // |r| < m^2 + m
-    r %= m;
-    if (r < 0) r += m;
+    const uint32_t lo = (uint32_t)x, hi = (uint32_t)(x >> 32);
+    const uint32_t c1 = (1u << 16) % m, c2 = (uint32_t)((1ull << 32) % m), c3 = (uint32_t)((1ull << 48) % m);
+    const uint32_t s = (lo & 0xffffu) + (lo >> 16) * c1 + (hi & 0xffffu) * c2 + ((hi >> 16) ^ 0x8000u) * c3 +
+                       (m - (0x8000u * c3) % m);
+    const int r = (int)(s % (uint32_t)m);
     return r > 127 ? r - m : r;              // [-128, 127]
 }
 
@@ -98,6 +101,46 @@ __host__ __device__ inline int64_t tiles_before(int I) {
     const int64_t q = I / 2;
     return (I & 1) ? (q + 1) * (q + 1) : q * (q + 1);
 }
+// The output residues go through a strip buffer of whole row blocks [I0, I1), at most kStripBytes (one row
+// block more if a single one is larger); the products of a strip all finish before its merge.
+constexpr int64_t kStripBytes = (int64_t)4 << 30;
+inline int64_t strip_max_tiles(int64_t strip_bytes) { return std::max<int64_t>(1, strip_bytes / (kMods * kTileOutBytes)); }
+inline int strip_end(int I0, int nrb, int64_t max_tiles) {
+    int I1 = I0 + 1;
+    while (I1 < nrb && tiles_before(I1 + 1) - tiles_before(I0) <= max_tiles) ++I1;
+    return I1;
+}
+// Order in which the residue products hand out the tiles of a strip (inside one modulus): bands of kBand row
+// blocks from I0, and inside a band column by column, the band's rows of a column one after the other.  The
+// ~148 tiles in flight then cover about kBand row blocks x 148 / kBand column tiles, so an A chunk (row block
+// I) and a B chunk pair (row blocks 2J, 2J + 1) are each read by ~12 tiles close together in time and come
+// from L2; their contractions start at most kBand - 1 k-blocks apart.  Row-block-major order shared B chunks
+// only ~2 ways at N = 32768.  g in [0, tiles_before(I1) - tiles_before(I0)) -> tile (I, J).
+constexpr int kBand = 12;
+__host__ __device__ inline void raster_tile(int64_t g, int I0, int I1, int& I, int& J) {
+    const int64_t t0 = tiles_before(I0);
+    int lo = 0, hi = (I1 - I0 - 1) / kBand;  // band: largest b with tiles_before(I0 + kBand b) - t0 <= g
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (tiles_before(I0 + kBand * mid) - t0 <= g) lo = mid;
+        else hi = mid - 1;
+    }
+    const int Ib = I0 + kBand * lo, Ie = Ib + kBand < I1 ? Ib + kBand : I1, G = Ie - Ib;
+    int64_t x = g - (tiles_before(Ib) - t0);
+    const int Jf = Ib / 2 + 1;               // columns J < Jf hold all G rows of the band (2 J <= Ib)
+    if (x < (int64_t)Jf * G) {
+        J = (int)(x / G);
+        I = Ib + (int)(x - (int64_t)J * G);
+        return;
+    }
+    x -= (int64_t)Jf * G;
+    J = Jf;                                  // then columns with rows 2 J .. Ie - 1
+    while (x >= Ie - 2 * J) {
+        x -= Ie - 2 * J;
+        ++J;
+    }
+    I = 2 * J + (int)x;
+}
 // residues of one strip: [tile - first tile of the strip][t][128 rows][256 columns] bytes, r in [0, m_t)
 __host__ __device__ inline int64_t out_offset(int64_t tile_local, int t, int r, int c) {
     return (tile_local * kMods + t) * kTileOutBytes + (int64_t)r * kBN + c;
@@ -108,11 +151,15 @@ __host__ __device__ inline int64_t out_offset(int64_t tile_local, int t, int r, 
 // The stages of the emulated product, in the order ozaki_syrk_lower runs them (tools/ozaki_check.cu
 // drives them one by one).  exps: nrbp * 128 int32; res: kMods * chunks * 16 KiB.
 int ozaki_split(pgp_ctx* ctx, const double* G, int64_t ld, int64_t n, int* exps, int8_t* res);
-// residue products of the lower tiles of row blocks [I0, I1) into `out` (oz::out_offset)
-int ozaki_products(pgp_ctx* ctx, const int8_t* res, int64_t n, int I0, int I1, uint8_t* out);
+// residue products of the lower tiles of row blocks [I0, I1) into `out` (oz::out_offset).
+// resident_chunks (a power of two, timing diagnostic only): every operand chunk index is taken modulo it, so
+// the same items and MACs read a window of resident_chunks * 16 KiB that stays in L2; `out` is then garbage
+int ozaki_products(pgp_ctx* ctx, const int8_t* res, int64_t n, int I0, int I1, uint8_t* out,
+                   int64_t resident_chunks = 0);
 // H (lower entries of rows [128 I0, 128 I1)) <- reconstruction of `out`, scaled by 2^-(e_i + e_j)
 int ozaki_merge(pgp_ctx* ctx, const uint8_t* out, const int* exps, int64_t n, int I0, int I1, double* H, int64_t ldh);
-// all of it: the lower triangle of H <- G G^T, G upper triangular, 1 <= n <= oz::kMaxK
-int ozaki_syrk_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n);
+// all of it: the lower triangle of H <- G G^T, G upper triangular, 1 <= n <= oz::kMaxK; strips of at most
+// strip_bytes of output residues (a smaller value only cuts more strips)
+int ozaki_syrk_lower(pgp_ctx* ctx, const Mat& H, const Mat& G, int64_t n, int64_t strip_bytes = oz::kStripBytes);
 
 }  // namespace pgp

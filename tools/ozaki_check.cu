@@ -12,6 +12,14 @@
 //   ozaki_check resid FILE       trap 2: residues of int64 values above 2^53; writes "x r_0 .. r_15" lines
 //   ozaki_check compare N [reps] V = L^-T of a Matern-5/2 Gram (d = 4): emulated vs DMMA V V^T,
 //                                max |dH| / sqrt(H_ii H_jj) and the time of each (CUDA events)
+//   ozaki_check strips N TILES   V = L^-T as for compare, products and merge cut into strips of at most TILES
+//                                tiles: the residue bytes of sampled tiles (first and last of every strip,
+//                                diagonal tiles, the last row block, random ones; all moduli) BIT-EXACT
+//                                against an independent dp4a product of the same residue rows, and H against
+//                                the DMMA product to 1e-13 of sqrt(H_ii H_jj)
+//   ozaki_check feed N [reps]    the residue products alone on random residues, strips as the library cuts
+//                                them: as laid out, and with every operand chunk read from a 32 MiB window
+//                                that stays in L2 (same items, same MACs) -- how much the operand feed costs
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
@@ -308,7 +316,8 @@ __global__ void maxrel_kernel(const double* He, const double* Hd, int64_t ld, in
     atomicMax(out, (unsigned long long)__double_as_longlong(m));
 }
 
-static int run_compare(int64_t n, int reps) {
+// V = L^-T of a Matern-5/2 Gram (d = 4) in G (ld = lead_dim(n)); F and Hs are n x ld scratch
+static void make_v(int64_t n, double* F, double* G, double* Hs) {
     const int64_t ld = lead_dim(n);
     const int d = 4;
     std::mt19937_64 rng(3);
@@ -316,35 +325,61 @@ static int run_compare(int64_t n, int reps) {
     std::vector<double> X((size_t)n * d);
     const double ell = 0.5 * std::pow((double)n, -1.0 / d) * 8;          // a few neighbours per length-scale
     for (auto& x : X) x = ud(rng) / ell;
-    double *dX, *F, *G, *Hd, *He;
+    double* dX;
     int* info;
-    unsigned long long* dmax;
     CK(cudaMalloc(&dX, sizeof(double) * X.size()));
-    CK(cudaMalloc(&F, sizeof(double) * n * ld));
-    CK(cudaMalloc(&G, sizeof(double) * n * ld));
-    CK(cudaMalloc(&Hd, sizeof(double) * n * ld));
-    CK(cudaMalloc(&He, sizeof(double) * n * ld));
     CK(cudaMalloc(&info, sizeof(int)));
-    CK(cudaMalloc(&dmax, sizeof(unsigned long long)));
     CK(cudaMemcpy(dX, X.data(), sizeof(double) * X.size(), cudaMemcpyHostToDevice));
     CK(cudaMemset(info, 0, sizeof(int)));
     CK(cudaMemset(G, 0, sizeof(double) * n * ld));
     matern_gram_kernel<<<dim3(64, (unsigned)n), 256>>>(dX, d, n, F, ld, 1e-2);
     CK(cudaGetLastError());
-    Mat Fm, Gm, Hm, Em;
+    Mat Fm, Gm, Hm;
     Fm.p = F; Fm.ld = ld;
     Gm.p = G; Gm.ld = ld;
-    Hm.p = Hd; Hm.ld = ld;
-    Em.p = He; Em.ld = ld;
+    Hm.p = Hs; Hm.ld = ld;
     LIB(potrf_lower(&ctx, Fm, n, 0, info));
-    LIB(inv_upper(&ctx, Gm, Fm, n, Hm));                                      // V = L^-T (Hd is scratch)
+    LIB(inv_upper(&ctx, Gm, Fm, n, Hm));                                      // V = L^-T (Hs is scratch)
     int hinfo = 0;
     CK(cudaMemcpy(&hinfo, info, sizeof(int), cudaMemcpyDeviceToHost));
-    if (hinfo) { fprintf(stderr, "Cholesky failed at %d\n", hinfo); return 2; }
+    if (hinfo) { fprintf(stderr, "Cholesky failed at %d\n", hinfo); exit(2); }
+    cudaFree(dX); cudaFree(info);
+}
 
-    GemmArgs g;                                                               // the DMMA V V^T
-    g.A = G; g.lda = ld; g.B = G; g.ldb = ld; g.C = Hd; g.ldc = ld;
+// the DMMA product H <- lower(G G^T)
+static void dmma_syrk(int64_t n, const double* G, double* H) {
+    const int64_t ld = lead_dim(n);
+    GemmArgs g;
+    g.A = G; g.lda = ld; g.B = G; g.ldb = ld; g.C = H; g.ldc = ld;
     g.M = n; g.N = n; g.K = n; g.alpha = 1.0; g.beta = 0.0; g.tri = 1; g.krow = 1;
+    LIB(launch_gemm_nt(&ctx, g));
+}
+
+static double max_rel(int64_t n, const double* He, const double* Hd) {
+    unsigned long long* dmax;
+    CK(cudaMalloc(&dmax, sizeof(unsigned long long)));
+    CK(cudaMemset(dmax, 0, sizeof(unsigned long long)));
+    maxrel_kernel<<<dim3(16, (unsigned)n), 256>>>(He, Hd, lead_dim(n), n, dmax);
+    unsigned long long bits;
+    CK(cudaMemcpy(&bits, dmax, sizeof bits, cudaMemcpyDeviceToHost));
+    cudaFree(dmax);
+    double m;
+    memcpy(&m, &bits, sizeof bits);
+    return m;
+}
+
+static int run_compare(int64_t n, int reps) {
+    const int64_t ld = lead_dim(n);
+    double *F, *G, *Hd, *He;
+    CK(cudaMalloc(&F, sizeof(double) * n * ld));
+    CK(cudaMalloc(&G, sizeof(double) * n * ld));
+    CK(cudaMalloc(&Hd, sizeof(double) * n * ld));
+    CK(cudaMalloc(&He, sizeof(double) * n * ld));
+    make_v(n, F, G, Hd);
+    Mat Gm, Em;
+    Gm.p = G; Gm.ld = ld;
+    Em.p = He; Em.ld = ld;
+
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));
@@ -364,7 +399,7 @@ static int run_compare(int64_t n, int reps) {
         std::sort(ms.begin(), ms.end());
         return (double)ms[ms.size() / 2];
     };
-    const double t_dmma = time_it([&] { LIB(launch_gemm_nt(&ctx, g)); });
+    const double t_dmma = time_it([&] { dmma_syrk(n, G, Hd); });
     const double t_emu = time_it([&] { LIB(ozaki_syrk_lower(&ctx, Em, Gm, n)); });
     // one more emulated run with the launch profile on: split / products / merge separately
     ctx.profile = true;
@@ -380,26 +415,198 @@ static int run_compare(int64_t n, int reps) {
         else t_merge += t;
     }
     ctx.profile = false;
-    CK(cudaMemset(dmax, 0, sizeof(unsigned long long)));
-    maxrel_kernel<<<dim3(16, (unsigned)n), 256>>>(He, Hd, ld, n, dmax);
-    unsigned long long bits;
-    CK(cudaMemcpy(&bits, dmax, sizeof bits, cudaMemcpyDeviceToHost));
-    double maxrel;
-    memcpy(&maxrel, &bits, sizeof bits);
+    const double maxrel = max_rel(n, He, Hd);
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, 0));
     printf("{\"n\": %ld, \"device\": \"%s\", \"dmma_ms\": %.3f, \"emulated_ms\": %.3f, \"speedup\": %.3f, "
            "\"split_ms\": %.3f, \"products_ms\": %.3f, \"merge_ms\": %.3f, \"products_int8_tops\": %.1f, "
            "\"max_rel_dH\": %.3e}\n",
            (long)n, prop.name, t_dmma, t_emu, t_dmma / t_emu, t_split, t_prod, t_merge, ops / (t_prod * 1e-3) / 1e12, maxrel);
-    cudaFree(dX); cudaFree(F); cudaFree(G); cudaFree(Hd); cudaFree(He);
+    cudaFree(F); cudaFree(G); cudaFree(Hd); cudaFree(He);
     pool_release(&ctx);
     return maxrel <= 1e-13 ? 0 : 1;
 }
 
+// ---- strips: sampled output tiles of every strip against an independent residue product ------------
+// one CTA per (sampled tile, modulus); thread = one column of the tile.  Residue rows are read from the
+// chunk layout 16 bytes (one swizzle unit) at a time and multiplied with dp4a: exact in int32.
+__global__ void ref_tiles_kernel(const int8_t* res, oz::Layout L, const int2* tiles, const int64_t* tile_local,
+                                 const uint8_t* out, unsigned long long* bad) {
+    const int s = blockIdx.x / oz::kMods, t = blockIdx.x % oz::kMods;
+    const int I = tiles[s].x, J = tiles[s].y, c = threadIdx.x;
+    const int64_t j = (int64_t)J * oz::kBN + c;
+    const int jb = (int)(j / oz::kRB), jr = (int)(j % oz::kRB);
+    const int m = oz::modulus(t);
+    for (int r0 = 0; r0 < oz::kRB; r0 += 16) {
+        int acc[16] = {0};
+        for (int kb = I; kb < L.nrb; ++kb) {
+            const int8_t* a = res + L.chunk_index(t, kb, I) * oz::kChunkBytes;
+            const int8_t* b = res + L.chunk_index(t, kb, jb) * oz::kChunkBytes;
+            for (int u = 0; u < 8; ++u) {
+                const int4 bv = *reinterpret_cast<const int4*>(b + oz::Layout::byte_in_chunk(jr, 16 * u));
+#pragma unroll
+                for (int r = 0; r < 16; ++r) {
+                    const int4 av = *reinterpret_cast<const int4*>(a + oz::Layout::byte_in_chunk(r0 + r, 16 * u));
+                    acc[r] = __dp4a(av.x, bv.x, acc[r]);
+                    acc[r] = __dp4a(av.y, bv.y, acc[r]);
+                    acc[r] = __dp4a(av.z, bv.z, acc[r]);
+                    acc[r] = __dp4a(av.w, bv.w, acc[r]);
+                }
+            }
+        }
+        for (int r = 0; r < 16; ++r) {
+            const int want = (acc[r] % m + m) % m;
+            if (out[oz::out_offset(tile_local[s], t, r0 + r, c)] != want) atomicAdd(bad, 1ull);
+        }
+    }
+}
+
+static int run_strips(int64_t n, int64_t max_tiles) {
+    const int64_t ld = lead_dim(n);
+    const oz::Layout L = oz::make_layout(n);
+    double *F, *G, *Hd, *He;
+    CK(cudaMalloc(&F, sizeof(double) * n * ld));
+    CK(cudaMalloc(&G, sizeof(double) * n * ld));
+    CK(cudaMalloc(&Hd, sizeof(double) * n * ld));
+    CK(cudaMalloc(&He, sizeof(double) * n * ld));
+    make_v(n, F, G, Hd);
+    dmma_syrk(n, G, Hd);
+    CK(cudaMemset(He, 0, sizeof(double) * n * ld));
+    std::vector<std::pair<int, int>> strips;
+    int64_t strip_max = 0;
+    for (int I0 = 0; I0 < L.nrb;) {
+        const int I1 = oz::strip_end(I0, L.nrb, max_tiles);
+        strips.push_back({I0, I1});
+        strip_max = std::max(strip_max, oz::tiles_before(I1) - oz::tiles_before(I0));
+        I0 = I1;
+    }
+    int* dexp;
+    int8_t* dres;
+    uint8_t* dout;
+    int2* dtiles;
+    int64_t* dlocal;
+    unsigned long long* dbad;
+    CK(cudaMalloc(&dexp, sizeof(int) * L.nrbp * oz::kRB));
+    CK(cudaMalloc(&dres, (size_t)oz::kMods * L.chunks * oz::kChunkBytes));
+    CK(cudaMalloc(&dout, (size_t)strip_max * oz::kMods * oz::kTileOutBytes));
+    CK(cudaMalloc(&dtiles, sizeof(int2) * strip_max));
+    CK(cudaMalloc(&dlocal, sizeof(int64_t) * strip_max));
+    CK(cudaMalloc(&dbad, sizeof(unsigned long long)));
+    CK(cudaMemset(dbad, 0, sizeof(unsigned long long)));
+    LIB(ozaki_split(&ctx, G, ld, n, dexp, dres));
+    std::mt19937_64 rng(9);
+    size_t checked = 0;
+    int64_t order_errors = 0;                                                  // raster_tile: each tile exactly once
+    for (auto& st : strips) {
+        const int I0 = st.first, I1 = st.second;
+        const int64_t t0 = oz::tiles_before(I0), cnt = oz::tiles_before(I1) - t0;
+        std::vector<char> hit(cnt, 0);
+        for (int64_t g = 0; g < cnt; ++g) {
+            int I, J;
+            oz::raster_tile(g, I0, I1, I, J);
+            const int64_t p = oz::tiles_before(I) + J - t0;
+            if (I < I0 || I >= I1 || J < 0 || J > I / 2 || hit[p]++) ++order_errors;
+        }
+        std::vector<int64_t> pick = {0, cnt - 1};                           // first and last tile of the strip
+        for (int I = I0; I < I1; ++I) {
+            if ((I - I0) % 8 == 0 || I == L.nrb - 1) pick.push_back(oz::tiles_before(I) + I / 2 - t0);   // diagonal
+            if (I == L.nrb - 1)                                                // the last (partial) row block
+                for (int J = 0; J <= I / 2; ++J) pick.push_back(oz::tiles_before(I) + J - t0);
+        }
+        std::uniform_int_distribution<int64_t> ut(0, cnt - 1);
+        for (int k = 0; k < 16; ++k) pick.push_back(ut(rng));
+        std::sort(pick.begin(), pick.end());
+        pick.erase(std::unique(pick.begin(), pick.end()), pick.end());
+        std::vector<int2> tl;
+        for (int64_t p : pick) {
+            int I = I0;
+            while (oz::tiles_before(I + 1) - t0 <= p) ++I;
+            tl.push_back(make_int2(I, (int)(p + t0 - oz::tiles_before(I))));
+        }
+        CK(cudaMemcpy(dtiles, tl.data(), sizeof(int2) * tl.size(), cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(dlocal, pick.data(), sizeof(int64_t) * pick.size(), cudaMemcpyHostToDevice));
+        LIB(ozaki_products(&ctx, dres, n, I0, I1, dout));
+        ref_tiles_kernel<<<(unsigned)(tl.size() * oz::kMods), oz::kBN>>>(dres, L, dtiles, dlocal, dout, dbad);
+        CK(cudaGetLastError());
+        LIB(ozaki_merge(&ctx, dout, dexp, n, I0, I1, He, ld));
+        checked += tl.size();
+    }
+    unsigned long long bad;
+    CK(cudaMemcpy(&bad, dbad, sizeof bad, cudaMemcpyDeviceToHost));
+    const double maxrel = max_rel(n, He, Hd);
+    printf("strips n=%ld strips=%zu order_errors=%ld tiles_checked=%zu residue_mismatches=%llu max_rel_dH=%.3e\n",
+           (long)n, strips.size(), (long)order_errors, checked, bad, maxrel);
+    cudaFree(F); cudaFree(G); cudaFree(Hd); cudaFree(He);
+    cudaFree(dexp); cudaFree(dres); cudaFree(dout); cudaFree(dtiles); cudaFree(dlocal); cudaFree(dbad);
+    pool_release(&ctx);
+    return (order_errors == 0 && bad == 0 && maxrel <= 1e-13) ? 0 : 1;
+}
+
+// ---- feed: residue products with operands from HBM vs from an L2-resident window -------------------
+__global__ void fill_kernel(int8_t* p, size_t bytes, uint64_t seed) {
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < bytes / 8; i += (size_t)gridDim.x * blockDim.x) {
+        uint64_t z = (i + 1) * 0x9E3779B97F4A7C15ull ^ seed;
+        z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+        z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+        reinterpret_cast<uint64_t*>(p)[i] = z ^ (z >> 31);
+    }
+}
+
+static int run_feed(int64_t n, int reps) {
+    const oz::Layout L = oz::make_layout(n);
+    const int64_t max_tiles = oz::strip_max_tiles(oz::kStripBytes);
+    std::vector<std::pair<int, int>> strips;
+    int64_t strip_max = 0;
+    for (int I0 = 0; I0 < L.nrb;) {
+        const int I1 = oz::strip_end(I0, L.nrb, max_tiles);
+        strips.push_back({I0, I1});
+        strip_max = std::max(strip_max, oz::tiles_before(I1) - oz::tiles_before(I0));
+        I0 = I1;
+    }
+    const size_t res_bytes = (size_t)oz::kMods * L.chunks * oz::kChunkBytes;
+    int8_t* dres;
+    uint8_t* dout;
+    CK(cudaMalloc(&dres, res_bytes));
+    CK(cudaMalloc(&dout, (size_t)strip_max * oz::kMods * oz::kTileOutBytes));
+    fill_kernel<<<4096, 256>>>(dres, res_bytes, 5);
+    CK(cudaGetLastError());
+    double macs = 0;
+    for (int I = 0; I < L.nrb; ++I) macs += (double)(I / 2 + 1) * oz::kRB * oz::kBN * (double)(L.nrb - I) * oz::kRB * oz::kMods;
+    const int64_t window = 2048;                                              // chunks: 32 MiB
+    cudaEvent_t e0, e1;
+    CK(cudaEventCreate(&e0));
+    CK(cudaEventCreate(&e1));
+    auto once = [&](int64_t resident) {
+        CK(cudaEventRecord(e0));
+        for (auto& st : strips) LIB(ozaki_products(&ctx, dres, n, st.first, st.second, dout, resident));
+        CK(cudaEventRecord(e1));
+        CK(cudaEventSynchronize(e1));
+        float t;
+        CK(cudaEventElapsedTime(&t, e0, e1));
+        return (double)t;
+    };
+    once(0);
+    once(window);
+    std::vector<double> a, b;
+    for (int r = 0; r < reps; ++r) {                                          // alternating
+        a.push_back(once(0));
+        b.push_back(once(window));
+    }
+    std::sort(a.begin(), a.end());
+    std::sort(b.begin(), b.end());
+    const double ta = a[a.size() / 2], tb = b[b.size() / 2];
+    cudaDeviceProp prop;
+    CK(cudaGetDeviceProperties(&prop, 0));
+    printf("{\"n\": %ld, \"device\": \"%s\", \"strips\": %zu, \"products_ms\": %.3f, \"resident_ms\": %.3f, "
+           "\"products_int8_tops\": %.1f, \"resident_int8_tops\": %.1f}\n",
+           (long)n, prop.name, strips.size(), ta, tb, 2 * macs / (ta * 1e-3) / 1e12, 2 * macs / (tb * 1e-3) / 1e12);
+    cudaFree(dres); cudaFree(dout);
+    return 0;
+}
+
 int main(int argc, char** argv) {
     if (argc < 3) {
-        fprintf(stderr, "usage: ozaki_check exact N [seed] | nonfinite 0 | merge FILE | resid FILE | compare N [reps]\n");
+        fprintf(stderr, "usage: ozaki_check exact N [seed] | nonfinite 0 | merge FILE | resid FILE | compare N [reps] | strips N TILES | feed N [reps]\n");
         return 2;
     }
     init_ctx();
@@ -409,6 +616,8 @@ int main(int argc, char** argv) {
     if (mode == "nonfinite") return run_nonfinite();
     if (mode == "resid") return run_resid(argv[2]);
     if (mode == "compare") return run_compare(atoll(argv[2]), argc > 3 ? atoi(argv[3]) : 3);
+    if (mode == "strips") return run_strips(atoll(argv[2]), argc > 3 ? atoll(argv[3]) : 2000);
+    if (mode == "feed") return run_feed(atoll(argv[2]), argc > 3 ? atoi(argv[3]) : 3);
     fprintf(stderr, "unknown mode %s\n", mode.c_str());
     return 2;
 }
