@@ -189,8 +189,6 @@ int alloc(pgp_ctx* ctx, DevBuf& b, size_t count) {
     return 0;
 }
 
-int single_type(const pgp_kernel_spec* s) { return s->n_parts == 1 ? s->parts[0].type : -1; }
-
 int upload_spec(pgp_ctx* ctx, const DevSpec& h, DevSpec* d) {
     // DevSpec is ~5 KB: stage through pageable memory (synchronous w.r.t. host)
     PGP_CUDA(ctx, cudaMemcpyAsync(d, &h, sizeof(DevSpec), cudaMemcpyHostToDevice, ctx->stream));
@@ -847,7 +845,7 @@ extern "C" int pgp_exact_loglike(pgp_model* m, int want_grad, double* lZ, double
         PGP_CUDA(ctx, cudaMemsetAsync(m->d_G, 0, sizeof(double) * n * ld, ctx->stream));
     }
     if (!m->d_H) PGP_TRY(dev_alloc(ctx, &m->d_H, (size_t)n * ld));
-    if (!m->d_partials) PGP_TRY(dev_alloc(ctx, &m->d_partials, (size_t)trace_cta_count(n) * (kMaxHyper + 1)));
+    if (!m->d_partials) PGP_TRY(dev_alloc(ctx, &m->d_partials, kTracePartialDoubles));
     Mat F, G, H;
     F.p = m->d_F; F.ld = ld;
     G.p = m->d_G; G.ld = ld;
@@ -857,7 +855,7 @@ extern "C" int pgp_exact_loglike(pgp_model* m, int want_grad, double* lZ, double
     PGP_TRY(syrk_upper_lower_single(ctx, H, G, n));                         // K~^-1 = V V^T
     TraceArgs t;
     t.spec = m->d_spec;
-    t.Z = m->d_Z;
+    t.Z1 = t.Z2 = m->d_Z;
     t.n = n;
     t.ndim = m->ndim;
     t.n_parts = m->spec.n_parts;
@@ -866,13 +864,13 @@ extern "C" int pgp_exact_loglike(pgp_model* m, int want_grad, double* lZ, double
     t.ldp = ld;
     t.alpha = m->d_alpha;
     t.partials = m->d_partials;
-    t.dlZ = m->d_res + 1;
+    t.sums = m->d_res + 1;
     t.single_type = single_type(&m->spec);
     PGP_TRY(launch_trace(ctx, t));
     double* hp = ctx->h_pin;
     PGP_CUDA(ctx, cudaMemcpyAsync(hp, m->d_res + 1, sizeof(double) * (nk + 2), cudaMemcpyDeviceToHost, ctx->stream));
     PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    for (int i = 0; i < nk + 2; ++i) dlZ[i] = hp[i];
+    trace_dlZ(hp, nk, m->hspec.h.sn2, dlZ);
     return 0;
 }
 
@@ -1164,7 +1162,7 @@ static int batched_impl(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double*
         }
         PGP_TRY(alloc<double>(ctx, dgrad, (size_t)chunk * nh));
         PGP_TRY(alloc<double>(ctx, dalpha, (size_t)kGradStreams * n));
-        PGP_TRY(alloc<double>(ctx, dpart, (size_t)kGradStreams * trace_cta_count(n) * (kMaxHyper + 1)));
+        PGP_TRY(alloc<double>(ctx, dpart, kGradStreams * kTracePartialDoubles));
         PGP_TRY(dG.get(ctx, (size_t)kGradStreams * n * ld));
         PGP_TRY(dH.get(ctx, (size_t)kGradStreams * n * ld));
         PGP_CUDA(ctx, cudaMemsetAsync(dG.p, 0, sizeof(double) * kGradStreams * n * ld, ctx->stream));
@@ -1240,12 +1238,12 @@ static int batched_impl(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double*
                 if (!rc2) {
                     TraceArgs t;
                     t.spec = dspec.as<DevSpec>() + b;
-                    t.Z = dZ.as<double>() + (size_t)b * z_doubles(np, d, n);
+                    t.Z1 = t.Z2 = dZ.as<double>() + (size_t)b * z_doubles(np, d, n);
                     t.n = n; t.ndim = d; t.n_parts = np; t.nhyper = nk;
                     t.P = H.p; t.ldp = ld;
                     t.alpha = alpha;
-                    t.partials = dpart.as<double>() + (size_t)si * trace_cta_count(n) * (kMaxHyper + 1);
-                    t.dlZ = dgrad.as<double>() + (size_t)b * nh;
+                    t.partials = dpart.as<double>() + si * kTracePartialDoubles;
+                    t.sums = dgrad.as<double>() + (size_t)b * nh;
                     t.single_type = single_type(spec);
                     rc2 = launch_trace(ctx, t);
                 }
@@ -1291,7 +1289,7 @@ static int batched_impl(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double*
         for (int b = 0; b < bc; ++b) {
             if (lZ) lZ[b0 + b] = hres[b];
             if (info) info[b0 + b] = hinfo[b];
-            if (grad) for (int h = 0; h < nh; ++h) dlZ[(b0 + b) * nh + h] = hgrad[(size_t)b * nh + h];
+            if (grad) trace_dlZ(&hgrad[(size_t)b * nh], nk, hspecs[b].h.sn2, dlZ + (b0 + b) * nh);
         }
     }
     return 0;

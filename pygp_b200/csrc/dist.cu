@@ -97,8 +97,7 @@ struct pgp_dist {
     int64_t v_nb = 0;
     double* d_B = nullptr;                  // gradient: (1 + owned rows, ld)
     size_t b_doubles = 0;
-    double* d_part = nullptr;
-    size_t part_doubles = 0;
+    double* d_part = nullptr;               // gradient trace: kTracePartialDoubles
     double* d_sums = nullptr;               // kMaxHyper + 4
     int64_t group = 0;                      // trailing-update grouping (0: default)
     int chunks = 0;                         // row chunks a panel travels in (0: default)
@@ -339,7 +338,7 @@ extern "C" int pgp_dist_exact_update(pgp_dist* d, pgp_model* m, const double* hy
     PGP_TRY(launch_set_residual(ctx, F, n, m->d_y, m->d_spec));            // row n = y - mean, all columns
 
     // owned block columns of K + sn2 I, built in place: rows [j0, n) x columns [j0, j0 + w)
-    const int st = single_type_of(&m->spec);
+    const int st = single_type(&m->spec);
     const int64_t zd = z_stride(n);
     for (int64_t j = rank; j < nblk; j += size) {
         const int64_t j0 = cols.j0(j), w = cols.w(j);
@@ -610,26 +609,6 @@ __global__ void stair_identity_kernel(double* B, int64_t ld, int64_t front, int6
     }
 }
 
-// sums[h] = sum over CTAs of partials[cta][h], h <= nh; sums[nh + 1] = sum(alpha)
-__global__ void partial_sums_kernel(const double* partials, int64_t n_cta, int nh, const double* alpha, int64_t n,
-                                    double* sums) {
-    __shared__ double red[256];
-    const int h = blockIdx.x;
-    double v = 0.0;
-    if (h <= nh) {
-        for (int64_t c = threadIdx.x; c < n_cta; c += blockDim.x) v += partials[c * (nh + 1) + h];
-    } else {
-        for (int64_t i = threadIdx.x; i < n; i += blockDim.x) v += alpha[i];
-    }
-    red[threadIdx.x] = v;
-    __syncthreads();
-    for (int s = blockDim.x / 2; s > 0; s >>= 1) {
-        if (threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) sums[h] = red[0];
-}
-
 }  // namespace
 
 extern "C" int pgp_dist_exact_loglike(pgp_dist* d, pgp_model* m, int64_t nb, int want_grad, double* lZ, double* dlZ) {
@@ -659,15 +638,7 @@ extern "C" int pgp_dist_exact_loglike(pgp_dist* d, pgp_model* m, int64_t nb, int
         PGP_TRY(dev_alloc(ctx, &d->d_B, need));
         d->b_doubles = need;
     }
-    const int64_t n_cta = trace_dist_cta_count(rows_local, n);
-    const size_t need_part = (size_t)std::max<int64_t>(n_cta, 1) * (kMaxHyper + 1);
-    if (d->part_doubles < need_part) {
-        PGP_CUDA(ctx, cudaStreamSynchronize(S));
-        dev_free(ctx, d->d_part);
-        d->d_part = nullptr;
-        PGP_TRY(dev_alloc(ctx, &d->d_part, need_part));
-        d->part_doubles = need_part;
-    }
+    if (!d->d_part) PGP_TRY(dev_alloc(ctx, &d->d_part, kTracePartialDoubles));
     PGP_CUDA(ctx, cudaMemsetAsync(d->d_B, 0, sizeof(double) * need, S));
     PGP_CUDA(ctx, cudaMemcpyAsync(d->d_B, m->d_F + n * ld, sizeof(double) * n, cudaMemcpyDeviceToDevice, S));
     if (rows_local > 0) {
@@ -731,8 +702,8 @@ extern "C" int pgp_dist_exact_loglike(pgp_dist* d, pgp_model* m, int64_t nb, int
 
     TraceDistArgs t;
     t.spec = m->d_spec;
-    t.Z = m->d_Z;
-    t.zd = z_stride(n);
+    t.Z1 = t.Z2 = m->d_Z;
+    t.zd1 = t.zd2 = z_stride(n);
     t.n = n;
     t.ndim = m->ndim;
     t.n_parts = m->spec.n_parts;
@@ -745,21 +716,14 @@ extern "C" int pgp_dist_exact_loglike(pgp_dist* d, pgp_model* m, int64_t nb, int
     t.size = size;
     t.alpha = m->d_alpha;
     t.partials = d->d_part;
-    t.single_type = single_type_of(&m->spec);
+    t.sums = d->d_sums;
+    t.single_type = single_type(&m->spec);
     PGP_TRY(launch_trace_dist(ctx, t));
-    {
-        Launch Lc(ctx, PC_OTHER, 8.0 * n);
-        partial_sums_kernel<<<nk + 2, 256, 0, S>>>(d->d_part, n_cta, nk, m->d_alpha, n, d->d_sums);
-        PGP_TRY(check_launch(ctx, "partial_sums_kernel"));
-    }
     if (size > 1)      // the ONE collective of the gradient: nhyper + 1 partial traces
         PGP_NCCL(d, g_nccl.AllReduce(d->d_sums, d->d_sums, (size_t)nk + 1, ncclDouble, ncclSum, d->comm, S));
     double* hp = ctx->h_pin;
     PGP_CUDA(ctx, cudaMemcpyAsync(hp, d->d_sums, sizeof(double) * (nk + 2), cudaMemcpyDeviceToHost, S));
     PGP_CUDA(ctx, cudaStreamSynchronize(S));
-    // exact.py:131-141: dlZ = [-sn2 tr(Q), -1/2 sum(Q o dK_h)..., sum(alpha)]
-    dlZ[0] = -m->hspec.h.sn2 * hp[0];
-    for (int h = 0; h < nk; ++h) dlZ[1 + h] = -0.5 * hp[1 + h];
-    dlZ[1 + nk] = hp[1 + nk];
+    trace_dlZ(hp, nk, m->hspec.h.sn2, dlZ);
     return 0;
 }

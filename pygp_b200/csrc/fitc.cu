@@ -17,7 +17,7 @@
 //     with its three M x N GEMMs per hyper is regrouped into elementwise traces
 //         dlZ_h = 1/2 [ dk_h(0) sum(q - 1/ell^2) + sum(dKuu_h o Cuu) + sum(dKxu_h o Cxu) ]
 //     (oracle/fitc_model.py derives and checks the regrouping against the
-//     oracle), so no dK matrix is ever materialised: trace_rect_kernel
+//     oracle), so no dK matrix is ever materialised: the trace kernel
 //     recomputes dK_h from the inputs while streaming Cuu / (Bt, T2).
 //   _marg_posterior(grad=False) (fitc.py:122-142): two right-solves per chunk of
 //     test points and one fused reduction.
@@ -438,8 +438,6 @@ int gemm(pgp_ctx* ctx, const double* A, int64_t lda, int tA, const double* B, in
     return launch_gemm(ctx, g);
 }
 
-int single_type(const pgp_kernel_spec* s) { return s->n_parts == 1 ? s->parts[0].type : -1; }
-
 void fitc_free(pgp_fitc* f) {
     pgp_ctx* ctx = f->ctx;
     cudaStreamSynchronize(ctx->stream);
@@ -739,8 +737,7 @@ extern "C" int pgp_fitc_loglike(pgp_fitc* f, int want_grad, double* lZ, double* 
                                                    f->d_q, f->d_w, f->d_P, ldp, dk0, f->d_res + 1);
         PGP_TRY(check_launch(ctx, "fitc_grad_scalars_kernel"));
     }
-    const size_t need = (size_t)std::max(trace_rect_cta_count(n, p), trace_rect_cta_count(p, p)) * (kMaxHyper + 1);
-    PGP_TRY(ensure_part(f, std::max(need, (size_t)kGemvBlocks * p)));
+    PGP_TRY(ensure_part(f, std::max(kTracePartialDoubles, (size_t)kGemvBlocks * p)));
     TraceRectArgs t;
     t.spec = f->d_spec;
     t.ndim = d; t.n_parts = np; t.nhyper = nk;

@@ -26,6 +26,8 @@
 //   + bulk-copy staging, 64 regs      0.525         0.78     1.06
 // i.e. the library sqrt / exp AND the strided per-thread staging both had to go.
 
+#include <type_traits>
+
 #include "fastmath.cuh"
 #include "gram.cuh"
 
@@ -735,6 +737,21 @@ __global__ void __launch_bounds__(kThreads, (MODE == 0 && is_fast_grad_type(PTYP
 // epilogue puts the eight warps of a CTA in lockstep; with one tile per CTA the four resident CTAs drift apart
 // and overlap their phases, which is worth more than the hidden copy latency.)
 
+// f(std::integral_constant<int, T>{}) with T = st, the leaf type of a one-leaf kernel, or -1: the
+// tile kernels' instantiation for that type (composite kernels: the tree interpreter)
+template <class F>
+static int with_leaf_type(int st, F&& f) {
+    switch (st) {
+        case PGP_SE: return f(std::integral_constant<int, PGP_SE>{});
+        case PGP_MATERN1: return f(std::integral_constant<int, PGP_MATERN1>{});
+        case PGP_MATERN3: return f(std::integral_constant<int, PGP_MATERN3>{});
+        case PGP_MATERN5: return f(std::integral_constant<int, PGP_MATERN5>{});
+        case PGP_PERIODIC: return f(std::integral_constant<int, PGP_PERIODIC>{});
+        case PGP_RQ: return f(std::integral_constant<int, PGP_RQ>{});
+        default: return f(std::integral_constant<int, -1>{});
+    }
+}
+
 template <int PTYPE, int MODE>
 static int launch_gram_t(pgp_ctx* ctx, const GramKArgs& a, size_t smem) {
     auto kern = gram_kernel<PTYPE, MODE>;
@@ -774,23 +791,11 @@ int launch_gram(pgp_ctx* ctx, const GramArgs& a0) {
         return ctx->fail(PGP_E_ARG, "gram: bad input-gradient request");
     if (mode == 3) return launch_gram_t<-1, 3>(ctx, a, smem);    // second derivatives: tree path only
     if (a.ostride != 1 && (a.symmetric || mode < 2)) return ctx->fail(PGP_E_ARG, "gram: strided output is for input-gradients only");
-    int st = a.n_parts == 1 ? a.single_type : -1;
-#define PGP_GRAM_CASE(T)                                                                  \
-    case T:                                                                               \
-        return mode == 2 ? launch_gram_t<T, 2>(ctx, a, smem)                              \
-                         : (mode == 1 ? launch_gram_t<T, 1>(ctx, a, smem) : launch_gram_t<T, 0>(ctx, a, smem));
-    switch (st) {
-        PGP_GRAM_CASE(PGP_SE)
-        PGP_GRAM_CASE(PGP_MATERN1)
-        PGP_GRAM_CASE(PGP_MATERN3)
-        PGP_GRAM_CASE(PGP_MATERN5)
-        PGP_GRAM_CASE(PGP_PERIODIC)
-        PGP_GRAM_CASE(PGP_RQ)
-        default:
-            return mode == 2 ? launch_gram_t<-1, 2>(ctx, a, smem)
-                             : (mode == 1 ? launch_gram_t<-1, 1>(ctx, a, smem) : launch_gram_t<-1, 0>(ctx, a, smem));
-    }
-#undef PGP_GRAM_CASE
+    return with_leaf_type(a.n_parts == 1 ? a.single_type : -1, [&](auto T) {
+        constexpr int PT = decltype(T)::value;
+        return mode == 2 ? launch_gram_t<PT, 2>(ctx, a, smem)
+                         : (mode == 1 ? launch_gram_t<PT, 1>(ctx, a, smem) : launch_gram_t<PT, 0>(ctx, a, smem));
+    });
 }
 
 // accumulate sum_{entries of one 64 x 64 tile} wq * dK_h for every hyper h into
@@ -885,91 +890,137 @@ __device__ __forceinline__ void trace_tile(const DevSpecHdr* S, const double* Zs
 }
 
 // ---------------------------------------------------------------------------
-// fused gradient trace: persistent CTAs over the lower-triangular tiles of
-// Q = K~^-1 - alpha alpha^T, recomputing K and every dK_h from the inputs.
-//   partial[cta][0]      = sum_i Q_ii
-//   partial[cta][1 + h]  = sum_ij Q_ij dK_h,ij   (full symmetric sum)
+// fused gradient trace: persistent CTAs over the tiles a policy W names, each accumulating
+// sum_ij W_ij dK_h,ij with K and every dK_h recomputed from the inputs.
+//   partials[cta][0]      = sum_i Q_ii when W::kExact, else not written
+//   partials[cta][1 + h]  = sum_ij W_ij dK_h,ij
+// A policy derives from the caller's arguments and adds
+//   kExact                 Q = K~^-1 - alpha alpha^T of an exact GP: one input set (Z2 = Z1), diagonal counted
+//   locate(tile, p)        tile index -> rows p.i0 of Z1 and p.j0 of Z2; false: skip (CTA-uniform)
+//   weights(p, t, wq, d)   the tile's weights, what it counts on the diagonal added to d
+// It is a template parameter: a runtime switch would cost registers in a kernel that sits at 128.
 // ---------------------------------------------------------------------------
-constexpr int kTraceCtasPerSm = 4;
+namespace {
 
-template <int PTYPE>
-__global__ void __launch_bounds__(kThreads) trace_kernel(TraceArgs a, int64_t n_tiles, int bulk) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int ndim = a.ndim, n_parts = a.n_parts, nh = a.nhyper, npd = n_parts * ndim;
-    const Smem sm(smem_raw, npd);
-    const DevSpecHdr* S = sm.S;
-    double* red = sm.extra;  // [8 warps][nhyper + 1]
-    uint32_t phase = 0;
-    bool first = true;
-    Tile t;
+struct TilePos {
+    int64_t i0, j0;
+};
 
-    double acc[kMaxHyper + 1];
-    for (int h = 0; h <= nh; ++h) acc[h] = 0.0;
-
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+// Q = K~^-1 - alpha alpha^T over the lower-triangular tiles: w Q_ij with w = 2 below the diagonal,
+// 1 on it, 0 above / outside
+struct SquareLower : TraceArgs {
+    static constexpr bool kExact = true;
+    using Pos = TilePos;
+    __device__ bool locate(int64_t tile, Pos& p) const {
         int ti, tj;
         tri_decode(tile, &ti, &tj);
-        const int64_t i0 = (int64_t)ti * kTile, j0 = (int64_t)tj * kTile;
-        if (first) {
-            smem_init_and_issue<true>(sm, a.spec, a.Z, a.Z, a.zd, a.zd, i0, j0, npd, bulk);
-            first = false;
-        } else {
-            __syncthreads();  // previous tile fully consumed
-            stage_issue(sm, a.Z, a.Z, a.zd, a.zd, i0, j0, npd, bulk);
-        }
-        stage_wait(sm, bulk, phase);
-
-        // weights: w Q_ij with w = 2 below the diagonal, 1 on it, 0 above / outside
-        double wq[4][4];
+        p.i0 = (int64_t)ti * kTile;
+        p.j0 = (int64_t)tj * kTile;
+        return true;
+    }
+    __device__ void weights(const Pos& p, const Tile& t, double (&wq)[4][4], double& diag) const {
 #pragma unroll
         for (int x = 0; x < 4; ++x) {
-            int64_t gi = i0 + t.row(x);
-            double ai = gi < a.n ? a.alpha[gi] : 0.0;
+            int64_t gi = p.i0 + t.row(x);
+            double ai = gi < n ? alpha[gi] : 0.0;
 #pragma unroll
             for (int y = 0; y < 4; ++y) {
-                int64_t gj = j0 + t.col(y);
+                int64_t gj = p.j0 + t.col(y);
                 double w = 0.0;
-                if (gi < a.n && gj <= gi) {
-                    double q = a.P[gi * a.ldp + gj] - ai * a.alpha[gj];
+                if (gi < n && gj <= gi) {
+                    double q = P[gi * ldp + gj] - ai * alpha[gj];
                     w = gi == gj ? q : 2.0 * q;
-                    if (gi == gj) acc[0] += q;
+                    if (gi == gj) diag += q;
                 }
                 wq[x][y] = w;
             }
         }
-
-        trace_tile<PTYPE>(S, sm.Zs1, sm.Zs2, sm.tab, ndim, n_parts, t, wq, acc);
     }
+};
 
-    // CTA reduction in a fixed order -> one row of partials per CTA
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    __syncthreads();
-    for (int h = 0; h <= nh; ++h) {
-        double v = acc[h];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == 0) red[warp * (nh + 1) + h] = v;
-    }
-    __syncthreads();
-    for (int h = threadIdx.x; h <= nh; h += kThreads) {
-        double v = 0.0;
-        for (int w = 0; w < kThreads / 32; ++w) v += red[w * (nh + 1) + h];
-        a.partials[(int64_t)blockIdx.x * (nh + 1) + h] = v;
-    }
-}
-
-// ---------------------------------------------------------------------------
-// rectangular trace: out[h] += scale * sum_ij W_ij dK_h(x1_i, x2_j) over a full
-// (n1, n2) block.  FITC's gradient is three of these (fitc.cu):
+// the full (n1, n2) rectangle (FITC's gradient is two of these, fitc.cu):
 //   mode 0: W = Wd (dense, ldw)                       -> sum(dKuu o Cuu)
 //   mode 1: W = 2 (al_i w_j - q_i Bt_ij + T2_ij)      -> sum(dKxu o Cxu),
 //           built on the fly so Cxu is never written.
-// partials[cta][h]; reduced by trace_rect_finish_kernel in a fixed order.
-// ---------------------------------------------------------------------------
-template <int PTYPE>
-__global__ void __launch_bounds__(kThreads) trace_rect_kernel(TraceRectArgs a, int64_t t2, int64_t n_tiles, int bulk) {
+struct Rect : TraceRectArgs {
+    static constexpr bool kExact = false;
+    using Pos = TilePos;
+    int64_t t2;  // tile columns
+    __device__ bool locate(int64_t tile, Pos& p) const {
+        const int64_t ti = tile / t2, tj = tile - ti * t2;
+        p.i0 = ti * kTile;
+        p.j0 = tj * kTile;
+        return true;
+    }
+    __device__ void weights(const Pos& p, const Tile& t, double (&wq)[4][4], double&) const {
+#pragma unroll
+        for (int x = 0; x < 4; ++x) {
+            const int64_t gi = p.i0 + t.row(x);
+            const bool rok = gi < n1;
+            double ai = 0.0, qi = 0.0;
+            if (mode == 1 && rok) { ai = al[gi]; qi = q ? q[gi] : 1.0; }
+#pragma unroll
+            for (int y = 0; y < 4; ++y) {
+                const int64_t gj = p.j0 + t.col(y);
+                double w = 0.0;
+                if (rok && gj < n2) {
+                    if (mode == 0) {
+                        // sym: only the lower triangle of a symmetric weight matrix is stored
+                        if (!sym) w = Wd[gi * ldw + gj];
+                        else if (gj < gi) w = 2.0 * Wd[gi * ldw + gj];
+                        else if (gj == gi) w = Wd[gi * ldw + gj];
+                    }
+                    else w = 2.0 * (ai * wv[gj] - qi * Bt[gi * ldw + gj] + T2[gi * ldw + gj]);
+                }
+                wq[x][y] = w;
+            }
+        }
+    }
+};
+
+// this rank's rows of K~^-1 (gram.cuh TraceDistArgs) x all columns: the rows of a tile are columns c of
+// K~^-1 (Z1 rows from c0), its columns are rows i; tiles wholly above the diagonal are skipped
+struct BlockColumn : TraceDistArgs {
+    static constexpr bool kExact = true;
+    struct Pos : TilePos {
+        int64_t r0, q;  // first local row, its block row
+    };
+    int64_t t2;
+    __device__ bool locate(int64_t tile, Pos& p) const {
+        const int64_t ti = tile / t2, tj = tile - ti * t2;
+        p.r0 = ti * kTile;
+        p.q = p.r0 / nb;
+        p.i0 = (rank + p.q * size) * nb + (p.r0 - p.q * nb);    // global column c0 of local row r0
+        p.j0 = tj * kTile;
+        return !(p.i0 >= n || p.j0 + kTile - 1 < p.i0);          // nothing on / below the diagonal
+    }
+    __device__ void weights(const Pos& p, const Tile& t, double (&wq)[4][4], double& diag) const {
+#pragma unroll
+        for (int x = 0; x < 4; ++x) {
+            const int64_t r = p.r0 + t.row(x), c = p.i0 + t.row(x);
+            const bool rok = r < rows_local && c < n && (r - p.q * nb) < nb;
+            const double ac = rok ? alpha[c] : 0.0;
+#pragma unroll
+            for (int y = 0; y < 4; ++y) {
+                const int64_t i = p.j0 + t.col(y);
+                double w = 0.0;
+                if (rok && i < n && i >= c) {
+                    const double qv = B[r * ldb + i] - ac * alpha[i];
+                    w = i == c ? qv : 2.0 * qv;
+                    if (i == c) diag += qv;
+                }
+                wq[x][y] = w;
+            }
+        }
+    }
+};
+
+}  // namespace
+
+template <int PTYPE, class W>
+__global__ void __launch_bounds__(kThreads) trace_kernel(W w, int64_t n_tiles, int bulk) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int ndim = a.ndim, n_parts = a.n_parts, nh = a.nhyper, npd = n_parts * ndim;
+    const int ndim = w.ndim, n_parts = w.n_parts, nh = w.nhyper, npd = n_parts * ndim;
     const Smem sm(smem_raw, npd);
     const DevSpecHdr* S = sm.S;
     double* red = sm.extra;  // [8 warps][nhyper + 1]
@@ -981,59 +1032,109 @@ __global__ void __launch_bounds__(kThreads) trace_rect_kernel(TraceRectArgs a, i
     for (int h = 0; h <= nh; ++h) acc[h] = 0.0;
 
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int64_t ti = tile / t2, tj = tile - ti * t2;
-        const int64_t i0 = ti * kTile, j0 = tj * kTile;
+        typename W::Pos p;
+        if (!w.locate(tile, p)) continue;
+        // one input set: the staging then computes the addresses of one array, not of two aliases
+        const double* Z2 = W::kExact ? w.Z1 : w.Z2;
+        const int64_t zd2 = W::kExact ? w.zd1 : w.zd2;
         if (first) {
-            smem_init_and_issue<true>(sm, a.spec, a.Z1, a.Z2, a.zd1, a.zd2, i0, j0, npd, bulk);
+            smem_init_and_issue<true>(sm, w.spec, w.Z1, Z2, w.zd1, zd2, p.i0, p.j0, npd, bulk);
             first = false;
         } else {
-            __syncthreads();
-            stage_issue(sm, a.Z1, a.Z2, a.zd1, a.zd2, i0, j0, npd, bulk);
+            __syncthreads();  // previous tile fully consumed
+            stage_issue(sm, w.Z1, Z2, w.zd1, zd2, p.i0, p.j0, npd, bulk);
         }
         stage_wait(sm, bulk, phase);
 
         double wq[4][4];
-#pragma unroll
-        for (int x = 0; x < 4; ++x) {
-            const int64_t gi = i0 + t.row(x);
-            const bool rok = gi < a.n1;
-            double ai = 0.0, qi = 0.0;
-            if (a.mode == 1 && rok) { ai = a.al[gi]; qi = a.q ? a.q[gi] : 1.0; }
-#pragma unroll
-            for (int y = 0; y < 4; ++y) {
-                const int64_t gj = j0 + t.col(y);
-                double w = 0.0;
-                if (rok && gj < a.n2) {
-                    if (a.mode == 0) {
-                        // sym: only the lower triangle of a symmetric weight matrix is stored
-                        if (!a.sym) w = a.Wd[gi * a.ldw + gj];
-                        else if (gj < gi) w = 2.0 * a.Wd[gi * a.ldw + gj];
-                        else if (gj == gi) w = a.Wd[gi * a.ldw + gj];
-                    }
-                    else w = 2.0 * (ai * a.wv[gj] - qi * a.Bt[gi * a.ldw + gj] + a.T2[gi * a.ldw + gj]);
-                }
-                wq[x][y] = w;
-            }
-        }
+        w.weights(p, t, wq, acc[0]);
         trace_tile<PTYPE>(S, sm.Zs1, sm.Zs2, sm.tab, ndim, n_parts, t, wq, acc);
     }
 
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    // CTA reduction in a fixed order -> one row of partials per CTA (reducing Rect's unused slot 0 as well
+    // cost its SE instantiation 29 registers)
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, h0 = W::kExact ? 0 : 1;
     __syncthreads();
-    for (int h = 1; h <= nh; ++h) {
+    for (int h = h0; h <= nh; ++h) {
         double v = acc[h];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
         if (lane == 0) red[warp * (nh + 1) + h] = v;
     }
     __syncthreads();
-    for (int h = 1 + threadIdx.x; h <= nh; h += kThreads) {
+    for (int h = h0 + threadIdx.x; h <= nh; h += kThreads) {
         double v = 0.0;
-        for (int w = 0; w < kThreads / 32; ++w) v += red[w * (nh + 1) + h];
-        a.partials[(int64_t)blockIdx.x * (nh + 1) + h] = v;
+        for (int k = 0; k < kThreads / 32; ++k) v += red[k * (nh + 1) + h];
+        w.partials[(int64_t)blockIdx.x * (nh + 1) + h] = v;
     }
 }
 
+template <class W>
+static int launch_trace_kernel(pgp_ctx* ctx, const W& w, int64_t n_tiles, int grid, double work) {
+    if (w.n_parts * w.ndim > 192)
+        return ctx->fail(PGP_E_ARG, "trace: n_parts * ndim > 192 exceeds the shared-memory tile");
+    const size_t smem = kSmemFixed + 2ull * w.n_parts * w.ndim * kTile * sizeof(double) +
+                        8ull * (w.nhyper + 1) * sizeof(double);
+    const int bulk = bulk_ok(w.Z1, w.zd1) && bulk_ok(w.Z2, w.zd2);
+    return with_leaf_type(w.n_parts == 1 ? w.single_type : -1, [&](auto T) {
+        auto kern = trace_kernel<decltype(T)::value, W>;
+        PGP_TRY(ensure_dyn_smem(ctx, kern, smem));
+        Launch L(ctx, PC_TRACE, work);
+        kern<<<grid, kThreads, smem, ctx->stream>>>(w, n_tiles, bulk);
+        return check_launch(ctx, "trace_kernel");
+    });
+}
+
+// sums[h] = sum over CTAs of partials[cta][h], h <= nh; sums[nh + 1] = sum(alpha)
+__global__ void trace_finish_kernel(const double* partials, int64_t n_cta, int nh, const double* alpha, int64_t n,
+                                    double* sums) {
+    __shared__ double red[256];
+    const int h = blockIdx.x;
+    double v = 0.0;
+    if (h <= nh) {
+        for (int64_t c = threadIdx.x; c < n_cta; c += blockDim.x) v += partials[c * (nh + 1) + h];
+    } else {
+        for (int64_t i = threadIdx.x; i < n; i += blockDim.x) v += alpha[i];
+    }
+    red[threadIdx.x] = v;
+    __syncthreads();
+    for (int s = blockDim.x / 2; s > 0; s >>= 1) {
+        if (threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) sums[h] = red[0];
+}
+
+static int launch_trace_finish(pgp_ctx* ctx, const TraceTiles& w, int n_cta, const double* alpha, int64_t n,
+                               double* sums, double work) {
+    Launch L(ctx, PC_OTHER, work);
+    trace_finish_kernel<<<w.nhyper + 2, 256, 0, ctx->stream>>>(w.partials, n_cta, w.nhyper, alpha, n, sums);
+    return check_launch(ctx, "trace_finish_kernel");
+}
+
+int launch_trace(pgp_ctx* ctx, const TraceArgs& a) {
+    SquareLower w;
+    static_cast<TraceArgs&>(w) = a;
+    if (!w.zd1) w.zd1 = z_stride(a.n);
+    if (!w.zd2) w.zd2 = z_stride(a.n);
+    const int64_t t = ceil_div(a.n, kTile), n_tiles = t * (t + 1) / 2;
+    const int grid = (int)std::min<int64_t>(n_tiles, kTraceMaxCtas);
+    PGP_TRY(launch_trace_kernel(ctx, w, n_tiles, grid, 4.0 * (double)a.n * (double)a.n));
+    return launch_trace_finish(ctx, a, grid, a.alpha, a.n, a.sums, 0.0);
+}
+
+int launch_trace_dist(pgp_ctx* ctx, const TraceDistArgs& a) {
+    if (a.nb <= 0 || a.nb % kTile) return ctx->fail(PGP_E_ARG, "trace: block width must be a multiple of 64");
+    BlockColumn w;
+    static_cast<TraceDistArgs&>(w) = a;
+    w.t2 = ceil_div(a.n, kTile);
+    const int64_t n_tiles = ceil_div(std::max<int64_t>(a.rows_local, 0), kTile) * w.t2;
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(n_tiles, kTraceMaxCtas));
+    PGP_TRY(launch_trace_kernel(ctx, w, n_tiles, grid, 8.0 * (double)a.rows_local * (double)a.n / 2));
+    return launch_trace_finish(ctx, a, grid, a.alpha, a.n, a.sums, 8.0 * a.n);
+}
+
+// out[h] += scale * s_h, accumulated on the device on top of what the caller put there
 __global__ void trace_rect_finish_kernel(const double* partials, int64_t n_cta, int nh, double scale, double* out) {
     __shared__ double red[256];
     const int h = blockIdx.x + 1;  // 1..nh
@@ -1048,227 +1149,21 @@ __global__ void trace_rect_finish_kernel(const double* partials, int64_t n_cta, 
     if (threadIdx.x == 0) out[h - 1] += scale * red[0];
 }
 
-int64_t trace_rect_cta_count(int64_t n1, int64_t n2) {
-    int64_t tiles = ceil_div(n1, kTile) * ceil_div(n2, kTile);
-    return std::min<int64_t>(tiles, 148 * kTraceCtasPerSm);
-}
-
-template <int PTYPE>
-static int launch_trace_rect_t(pgp_ctx* ctx, const TraceRectArgs& a, size_t smem, int64_t t2, int64_t n_tiles,
-                               int grid) {
-    auto kern = trace_rect_kernel<PTYPE>;
-    PGP_TRY(ensure_dyn_smem(ctx, kern, smem));
-    const int bulk = bulk_ok(a.Z1, a.zd1) && bulk_ok(a.Z2, a.zd2);
-    Launch L(ctx, PC_TRACE, (a.mode == 0 ? 8.0 : 16.0) * (double)a.n1 * (double)a.n2);
-    kern<<<grid, kThreads, smem, ctx->stream>>>(a, t2, n_tiles, bulk);
-    return check_launch(ctx, "trace_rect_kernel");
-}
-
-int launch_trace_rect(pgp_ctx* ctx, const TraceRectArgs& a0) {
-    if (a0.n1 <= 0 || a0.n2 <= 0) return 0;
-    TraceRectArgs a = a0;
-    if (!a.zd1) a.zd1 = z_stride(a.n1);
-    if (!a.zd2) a.zd2 = z_stride(a.n2);
-    if (a.n_parts * a.ndim > 192)
-        return ctx->fail(PGP_E_ARG, "trace: n_parts * ndim > 192 exceeds the shared-memory tile");
-    int64_t t2 = ceil_div(a.n2, kTile);
-    int64_t n_tiles = ceil_div(a.n1, kTile) * t2;
-    int grid = (int)trace_rect_cta_count(a.n1, a.n2);
-    size_t smem = kSmemFixed + 2ull * a.n_parts * a.ndim * kTile * sizeof(double) +
-                  8ull * (a.nhyper + 1) * sizeof(double);
-    int st = a.n_parts == 1 ? a.single_type : -1;
-    int rc;
-    switch (st) {
-        case PGP_SE: rc = launch_trace_rect_t<PGP_SE>(ctx, a, smem, t2, n_tiles, grid); break;
-        case PGP_MATERN1: rc = launch_trace_rect_t<PGP_MATERN1>(ctx, a, smem, t2, n_tiles, grid); break;
-        case PGP_MATERN3: rc = launch_trace_rect_t<PGP_MATERN3>(ctx, a, smem, t2, n_tiles, grid); break;
-        case PGP_MATERN5: rc = launch_trace_rect_t<PGP_MATERN5>(ctx, a, smem, t2, n_tiles, grid); break;
-        case PGP_PERIODIC: rc = launch_trace_rect_t<PGP_PERIODIC>(ctx, a, smem, t2, n_tiles, grid); break;
-        case PGP_RQ: rc = launch_trace_rect_t<PGP_RQ>(ctx, a, smem, t2, n_tiles, grid); break;
-        default: rc = launch_trace_rect_t<-1>(ctx, a, smem, t2, n_tiles, grid); break;
-    }
-    PGP_TRY(rc);
+int launch_trace_rect(pgp_ctx* ctx, const TraceRectArgs& a) {
+    if (a.n1 <= 0 || a.n2 <= 0) return 0;
+    Rect w;
+    static_cast<TraceRectArgs&>(w) = a;
+    if (!w.zd1) w.zd1 = z_stride(a.n1);
+    if (!w.zd2) w.zd2 = z_stride(a.n2);
+    w.t2 = ceil_div(a.n2, kTile);
+    const int64_t n_tiles = ceil_div(a.n1, kTile) * w.t2;
+    const int grid = (int)std::min<int64_t>(n_tiles, kTraceMaxCtas);
+    PGP_TRY(launch_trace_kernel(ctx, w, n_tiles, grid, (a.mode == 0 ? 8.0 : 16.0) * (double)a.n1 * (double)a.n2));
     {
         Launch L(ctx, PC_OTHER, 0.0);
         trace_rect_finish_kernel<<<a.nhyper, 256, 0, ctx->stream>>>(a.partials, grid, a.nhyper, a.scale, a.out);
     }
     return check_launch(ctx, "trace_rect_finish_kernel");
-}
-
-// dlZ[0] = -sn2 sum Q_ii ; dlZ[1+h] = -1/2 S_h ; dlZ[nh+1] = sum alpha
-__global__ void trace_finish_kernel(const DevSpec* spec, const double* partials, int64_t n_cta, int nh,
-                                    const double* alpha, int64_t n, double* dlZ) {
-    __shared__ double red[256];
-    const int h = blockIdx.x;  // 0..nh+1
-    double v = 0.0;
-    if (h <= nh) {
-        for (int64_t c = threadIdx.x; c < n_cta; c += blockDim.x) v += partials[c * (nh + 1) + h];
-    } else {
-        for (int64_t i = threadIdx.x; i < n; i += blockDim.x) v += alpha[i];
-    }
-    red[threadIdx.x] = v;
-    __syncthreads();
-    for (int s = blockDim.x / 2; s > 0; s >>= 1) {
-        if (threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-        double r = red[0];
-        if (h == 0) r = -spec->h.sn2 * r;
-        else if (h <= nh) r = -0.5 * r;
-        dlZ[h] = r;
-    }
-}
-
-int64_t trace_cta_count(int64_t n) {
-    int64_t t = ceil_div(n, kTile);
-    int64_t tiles = t * (t + 1) / 2;
-    return std::min<int64_t>(tiles, 148 * kTraceCtasPerSm);
-}
-
-template <int PTYPE>
-static int launch_trace_t(pgp_ctx* ctx, const TraceArgs& a, size_t smem, int64_t n_tiles, int grid) {
-    auto kern = trace_kernel<PTYPE>;
-    PGP_TRY(ensure_dyn_smem(ctx, kern, smem));
-    const int bulk = bulk_ok(a.Z, a.zd);
-    Launch L(ctx, PC_TRACE, 4.0 * (double)a.n * (double)a.n);
-    kern<<<grid, kThreads, smem, ctx->stream>>>(a, n_tiles, bulk);
-    return check_launch(ctx, "trace_kernel");
-}
-
-int launch_trace(pgp_ctx* ctx, const TraceArgs& a0) {
-    TraceArgs a = a0;
-    if (!a.zd) a.zd = z_stride(a.n);
-    if (a.n_parts * a.ndim > 192)
-        return ctx->fail(PGP_E_ARG, "trace: n_parts * ndim > 192 exceeds the shared-memory tile");
-    int64_t t = ceil_div(a.n, kTile);
-    int64_t n_tiles = t * (t + 1) / 2;
-    int grid = (int)trace_cta_count(a.n);
-    size_t smem = kSmemFixed + 2ull * a.n_parts * a.ndim * kTile * sizeof(double) +
-                  8ull * (a.nhyper + 1) * sizeof(double);
-    int st = a.n_parts == 1 ? a.single_type : -1;
-    int rc;
-    switch (st) {
-        case PGP_SE: rc = launch_trace_t<PGP_SE>(ctx, a, smem, n_tiles, grid); break;
-        case PGP_MATERN1: rc = launch_trace_t<PGP_MATERN1>(ctx, a, smem, n_tiles, grid); break;
-        case PGP_MATERN3: rc = launch_trace_t<PGP_MATERN3>(ctx, a, smem, n_tiles, grid); break;
-        case PGP_MATERN5: rc = launch_trace_t<PGP_MATERN5>(ctx, a, smem, n_tiles, grid); break;
-        case PGP_PERIODIC: rc = launch_trace_t<PGP_PERIODIC>(ctx, a, smem, n_tiles, grid); break;
-        case PGP_RQ: rc = launch_trace_t<PGP_RQ>(ctx, a, smem, n_tiles, grid); break;
-        default: rc = launch_trace_t<-1>(ctx, a, smem, n_tiles, grid); break;
-    }
-    PGP_TRY(rc);
-    {
-        Launch L(ctx, PC_OTHER, 0.0);
-        trace_finish_kernel<<<a.nhyper + 2, 256, 0, ctx->stream>>>(a.spec, a.partials, grid, a.nhyper, a.alpha,
-                                                                  a.n, a.dlZ);
-    }
-    return check_launch(ctx, "trace_finish_kernel");
-}
-
-// ---------------------------------------------------------------------------
-// block-column share of the gradient trace (gram.cuh: TraceDistArgs)
-// ---------------------------------------------------------------------------
-template <int PTYPE>
-__global__ void __launch_bounds__(kThreads) trace_dist_kernel(TraceDistArgs a, int64_t t2, int64_t n_tiles, int bulk) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int ndim = a.ndim, n_parts = a.n_parts, nh = a.nhyper, npd = n_parts * ndim;
-    const Smem sm(smem_raw, npd);
-    const DevSpecHdr* S = sm.S;
-    double* red = sm.extra;  // [8 warps][nhyper + 1]
-    uint32_t phase = 0;
-    bool first = true;
-    Tile t;
-
-    double acc[kMaxHyper + 1];
-    for (int h = 0; h <= nh; ++h) acc[h] = 0.0;
-
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int64_t ti = tile / t2, tj = tile - ti * t2;
-        const int64_t r0 = ti * kTile, q = r0 / a.nb;
-        const int64_t c0 = (a.rank + q * a.size) * a.nb + (r0 - q * a.nb);    // global column of local row r0
-        const int64_t j0 = tj * kTile;
-        if (c0 >= a.n || j0 + kTile - 1 < c0) continue;                       // (CTA-uniform) nothing on / below the diagonal
-        if (first) {
-            smem_init_and_issue<true>(sm, a.spec, a.Z + c0, a.Z + j0, a.zd, a.zd, 0, 0, npd, bulk);
-            first = false;
-        } else {
-            __syncthreads();
-            stage_issue(sm, a.Z + c0, a.Z + j0, a.zd, a.zd, 0, 0, npd, bulk);
-        }
-        stage_wait(sm, bulk, phase);
-
-        // rows of the tile = columns c of K~^-1 (this rank's), columns of the tile = rows i
-        double wq[4][4];
-#pragma unroll
-        for (int x = 0; x < 4; ++x) {
-            const int64_t r = r0 + t.row(x), c = c0 + t.row(x);
-            const bool rok = r < a.rows_local && c < a.n && (r - q * a.nb) < a.nb;
-            const double ac = rok ? a.alpha[c] : 0.0;
-#pragma unroll
-            for (int y = 0; y < 4; ++y) {
-                const int64_t i = j0 + t.col(y);
-                double w = 0.0;
-                if (rok && i < a.n && i >= c) {
-                    const double qv = a.B[r * a.ldb + i] - ac * a.alpha[i];
-                    w = i == c ? qv : 2.0 * qv;
-                    if (i == c) acc[0] += qv;
-                }
-                wq[x][y] = w;
-            }
-        }
-        trace_tile<PTYPE>(S, sm.Zs1, sm.Zs2, sm.tab, ndim, n_parts, t, wq, acc);
-    }
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    __syncthreads();
-    for (int h = 0; h <= nh; ++h) {
-        double v = acc[h];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == 0) red[warp * (nh + 1) + h] = v;
-    }
-    __syncthreads();
-    for (int h = threadIdx.x; h <= nh; h += kThreads) {
-        double v = 0.0;
-        for (int w = 0; w < kThreads / 32; ++w) v += red[w * (nh + 1) + h];
-        a.partials[(int64_t)blockIdx.x * (nh + 1) + h] = v;
-    }
-}
-
-int64_t trace_dist_cta_count(int64_t rows_local, int64_t n) {
-    int64_t tiles = ceil_div(rows_local, kTile) * ceil_div(n, kTile);
-    return std::max<int64_t>(1, std::min<int64_t>(tiles, 148 * kTraceCtasPerSm));
-}
-
-template <int PTYPE>
-static int launch_trace_dist_t(pgp_ctx* ctx, const TraceDistArgs& a, size_t smem, int64_t t2, int64_t n_tiles, int grid) {
-    auto kern = trace_dist_kernel<PTYPE>;
-    PGP_TRY(ensure_dyn_smem(ctx, kern, smem));
-    const int bulk = bulk_ok(a.Z, a.zd);
-    Launch L(ctx, PC_TRACE, 8.0 * (double)a.rows_local * (double)a.n / 2);
-    kern<<<grid, kThreads, smem, ctx->stream>>>(a, t2, n_tiles, bulk);
-    return check_launch(ctx, "trace_dist_kernel");
-}
-
-int launch_trace_dist(pgp_ctx* ctx, const TraceDistArgs& a) {
-    if (a.n_parts * a.ndim > 192)
-        return ctx->fail(PGP_E_ARG, "trace: n_parts * ndim > 192 exceeds the shared-memory tile");
-    if (a.nb <= 0 || a.nb % kTile) return ctx->fail(PGP_E_ARG, "trace: block width must be a multiple of 64");
-    const int64_t t2 = ceil_div(a.n, kTile);
-    const int64_t n_tiles = ceil_div(std::max<int64_t>(a.rows_local, 0), kTile) * t2;
-    const int grid = (int)trace_dist_cta_count(a.rows_local, a.n);
-    size_t smem = kSmemFixed + 2ull * a.n_parts * a.ndim * kTile * sizeof(double) + 8ull * (a.nhyper + 1) * sizeof(double);
-    int st = a.n_parts == 1 ? a.single_type : -1;
-    switch (st) {
-        case PGP_SE: return launch_trace_dist_t<PGP_SE>(ctx, a, smem, t2, n_tiles, grid);
-        case PGP_MATERN1: return launch_trace_dist_t<PGP_MATERN1>(ctx, a, smem, t2, n_tiles, grid);
-        case PGP_MATERN3: return launch_trace_dist_t<PGP_MATERN3>(ctx, a, smem, t2, n_tiles, grid);
-        case PGP_MATERN5: return launch_trace_dist_t<PGP_MATERN5>(ctx, a, smem, t2, n_tiles, grid);
-        case PGP_PERIODIC: return launch_trace_dist_t<PGP_PERIODIC>(ctx, a, smem, t2, n_tiles, grid);
-        case PGP_RQ: return launch_trace_dist_t<PGP_RQ>(ctx, a, smem, t2, n_tiles, grid);
-        default: return launch_trace_dist_t<-1>(ctx, a, smem, t2, n_tiles, grid);
-    }
 }
 
 // ---------------------------------------------------------------------------

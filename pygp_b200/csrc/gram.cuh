@@ -41,33 +41,44 @@ struct GramArgs {
 };
 int launch_gram(pgp_ctx* ctx, const GramArgs& a);
 
-struct TraceArgs {
+// Gradient traces sum_ij W_ij dK_h(x1_i, x2_j): one persistent tile kernel (gram.cu trace_kernel), whose
+// CTAs leave one row of partial sums each in `partials`, which needs kTracePartialDoubles doubles.
+constexpr int kTraceMaxCtas = 148 * 4;
+constexpr size_t kTracePartialDoubles = (size_t)kTraceMaxCtas * (kMaxHyper + 1);
+
+struct TraceTiles {
     const DevSpec* spec = nullptr;
-    const double* Z = nullptr;       // [parts][d][z_stride(n)]
-    int64_t n = 0;
-    int64_t zd = 0;                  // 0: z_stride(n)
+    const double* Z1 = nullptr;      // [parts][d][zd1]: inputs of the weight matrix's rows
+    const double* Z2 = nullptr;      // [parts][d][zd2]: inputs of its columns (may alias Z1)
+    int64_t zd1 = 0, zd2 = 0;
     int ndim = 0, n_parts = 0, nhyper = 0;
+    double* partials = nullptr;      // device scratch, kTracePartialDoubles
+    int single_type = -1;
+};
+
+// exact GP, Q = K~^-1 - alpha alpha^T over the lower-triangular tiles; Z1 = Z2, zd 0: z_stride(n).
+// sums = [sum Q_ii, sum(Q o dK_h)..., sum(alpha)] (device, nhyper + 2), scaled by trace_dlZ.
+struct TraceArgs : TraceTiles {
+    int64_t n = 0;
     const double* P = nullptr;       // lower triangle of K~^-1, (n, ldp)
     int64_t ldp = 0;
     const double* alpha = nullptr;   // (n)
-    double* partials = nullptr;      // [n_cta][nhyper + 1]
-    double* dlZ = nullptr;           // device (nhyper + 2): final gradient
-    int single_type = -1;
+    double* sums = nullptr;
 };
-// number of CTAs (= rows of `partials`) the trace launch will use
-int64_t trace_cta_count(int64_t n);
-// dlZ = [-sn2 tr(Q), -1/2 sum(Q o dK_h)..., sum(alpha)]   (exact.py:131-141)
 int launch_trace(pgp_ctx* ctx, const TraceArgs& a);
+
+// dlZ = [-sn2 tr(Q), -1/2 sum(Q o dK_h)..., sum(alpha)]   (exact.py:131-141) from the sums of an exact-GP trace
+inline void trace_dlZ(const double* sums, int nhyper, double sn2, double* dlZ) {
+    dlZ[0] = -sn2 * sums[0];
+    for (int h = 0; h < nhyper; ++h) dlZ[1 + h] = -0.5 * sums[1 + h];
+    dlZ[1 + nhyper] = sums[1 + nhyper];
+}
 
 // out[h] += scale * sum_ij W_ij dK_h(x1_i, x2_j), h < nhyper, over a full
 // rectangular block; W dense (mode 0) or FITC's Cxu built on the fly (mode 1).
-struct TraceRectArgs {
-    const DevSpec* spec = nullptr;
-    const double* Z1 = nullptr;      // [parts][d][z_stride(n1)]
-    const double* Z2 = nullptr;      // [parts][d][z_stride(n2)]
+// zd1 / zd2 0: z_stride(n1) / z_stride(n2).
+struct TraceRectArgs : TraceTiles {
     int64_t n1 = 0, n2 = 0;
-    int64_t zd1 = 0, zd2 = 0;        // 0: z_stride(n1) / z_stride(n2)
-    int ndim = 0, n_parts = 0, nhyper = 0;
     int mode = 0;
     int sym = 0;                     // mode 0, n1 == n2, X1 == X2: Wd holds the lower triangle of a symmetric W
     const double* Wd = nullptr;      // mode 0: (n1, ldw)
@@ -78,33 +89,25 @@ struct TraceRectArgs {
     const double* wv = nullptr;      // mode 1: (n2) w
     int64_t ldw = 0;
     double scale = 1.0;
-    double* partials = nullptr;      // [trace_rect_cta_count][nhyper + 1]
     double* out = nullptr;           // device (nhyper), accumulated into
-    int single_type = -1;
 };
-int64_t trace_rect_cta_count(int64_t n1, int64_t n2);
 int launch_trace_rect(pgp_ctx* ctx, const TraceRectArgs& a);
 
 // Block-column partition of the gradient trace (dist.cu): this rank holds the rows of K~^-1 that belong
 // to its block columns, B[r][i] = K~^-1[i][c(r)] valid for i >= c(r), where local row r = q nb + o is
-// global column c = (rank + q size) nb + o.  partials[cta][0] = sum of Q_cc, [1 + h] = the rank's
-// share of sum_ij Q_ij dK_h,ij (entries i > c counted twice, i == c once), Q = K~^-1 - alpha alpha^T.
-struct TraceDistArgs {
-    const DevSpec* spec = nullptr;
-    const double* Z = nullptr;       // [parts][d][zd], all n rows
-    int64_t zd = 0;
+// global column c = (rank + q size) nb + o.  Z1 = Z2 hold all n rows.  sums (device, nhyper + 2) =
+// [sum of Q_cc, the rank's share of sum_ij Q_ij dK_h,ij (entries i > c counted twice, i == c once)...,
+// sum(alpha)], Q = K~^-1 - alpha alpha^T.
+struct TraceDistArgs : TraceTiles {
     int64_t n = 0;
-    int ndim = 0, n_parts = 0, nhyper = 0;
     const double* B = nullptr;       // (rows_local, ldb)
     int64_t ldb = 0;
     int64_t rows_local = 0;
     int64_t nb = 0;
     int rank = 0, size = 1;
     const double* alpha = nullptr;   // (n)
-    double* partials = nullptr;      // [trace_dist_cta_count][nhyper + 1]
-    int single_type = -1;
+    double* sums = nullptr;
 };
-int64_t trace_dist_cta_count(int64_t rows_local, int64_t n);
 int launch_trace_dist(pgp_ctx* ctx, const TraceDistArgs& a);
 
 // out[h][i] = d k(x_i, x_i) / d hyper_h for h < nhyper (hmode=1) or k(x_i,x_i) (hmode=0)

@@ -33,8 +33,3 @@ struct pgp_model {
     double lZ = 0.0;
     int info = 0;
 };
-
-
-namespace pgp {
-inline int single_type_of(const pgp_kernel_spec* s) { return s->n_parts == 1 ? s->parts[0].type : -1; }
-}

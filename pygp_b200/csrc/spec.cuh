@@ -167,6 +167,9 @@ inline int compile_spec(const pgp_kernel_spec* s, const double* hyp, double sn2,
     return 0;
 }
 
+// leaf type of a one-leaf kernel, which the tile kernels instantiate for; -1 for a composite
+inline int single_type(const pgp_kernel_spec* s) { return s->n_parts == 1 ? s->parts[0].type : -1; }
+
 // ---- device: one leaf --------------------------------------------------------
 
 struct PartVal {

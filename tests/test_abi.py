@@ -59,8 +59,7 @@ def test_gram_tiles_are_staged_by_the_bulk_copy_engine(built):
     UBLKCP (bulk copy global -> shared) and SYNCS (mbarrier arrive / try_wait) in their SASS."""
     sass = subprocess.check_output(['cuobjdump', '-sass', built.LIB_PATH]).decode()
     funcs = sass.split('Function : ')
-    tiles = [f for f in funcs if f.split('\n', 1)[0].split('(')[0].find('gram_kernel') >= 0 or 'trace_kernel' in f.split('\n', 1)[0]
-             or 'trace_dist_kernel' in f.split('\n', 1)[0] or 'trace_rect_kernel' in f.split('\n', 1)[0]]
+    tiles = [f for f in funcs if f.split('\n', 1)[0].split('(')[0].find('gram_kernel') >= 0 or 'trace_kernel' in f.split('\n', 1)[0]]
     assert len(tiles) >= 20
     for f in tiles:
         assert 'UBLKCP' in f, f.split('\n', 1)[0]
