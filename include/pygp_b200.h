@@ -221,6 +221,26 @@ int pgp_batched_predict(pgp_ctx* ctx, const pgp_kernel_spec* spec,
                         const double* Xs, int64_t ms,
                         double* mu, double* s2, int32_t* info);
 
+/* ---- resident batch: meta/mcmc.py posterior(X, grad) over one chain ---------- */
+/* B ExactGP problems sharing X, y (hyps (B, nhyper_gp)), factored by the batched path's launches and kept in
+ * HBM.  The factors of as many problems as fit budget_bytes (0: half the free device memory) stay resident;
+ * the rest are factored again, chunk by chunk, at every predict.  info (B): per-problem potrf info, as
+ * pgp_batched_loglike.  The handle owns its device memory until pgp_batch_destroy. */
+typedef struct pgp_batch pgp_batch;
+int  pgp_batch_create(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double* X, const double* y, int64_t n,
+                      const double* hyps, int64_t B, int64_t budget_bytes, pgp_batch** out, int32_t* info);
+/* per-problem posterior at the same test points: mu, s2 (B, ms); input-gradients dmu, ds2 (B, ms, ndim), or
+ * both NULL.  mu and s2 are the bits pgp_batched_predict gives for the same problems and test points whenever
+ * both calls factor and solve a problem in the same kind of chunk: with other problems, or alone.  A problem
+ * alone in its chunk takes the single-model factorisation for 1536 <= n <= 20480 and the few-rows solve for
+ * ms <= 8 with n >= 512, which round differently from the batched ones; the chunks of the two calls depend on B,
+ * ms, the budget and the free memory. */
+int  pgp_batch_predict(pgp_batch* b, const double* Xs, int64_t ms, double* mu, double* s2,
+                       double* dmu, double* ds2);
+/* problems whose factor is resident */
+int64_t pgp_batch_resident(const pgp_batch* b);
+void pgp_batch_destroy(pgp_batch* b);
+
 /* ---- FITC: pygp/inference/fitc.py ----------------------------------------- */
 int pgp_fitc_create(pgp_ctx* ctx, const pgp_kernel_spec* spec,
                     const double* U, int64_t nu,

@@ -94,6 +94,10 @@ SIGNATURES = {
     'pgp_dist_exact_loglike': (C.c_int, [_vp, _vp, _i64, C.c_int, _dp, _dp]),
     'pgp_batched_loglike': (C.c_int, [_vp, _sp, _dp, _dp, _i64, _dp, _i64, _dp, _dp, _ip]),
     'pgp_batched_predict': (C.c_int, [_vp, _sp, _dp, _dp, _i64, _dp, _i64, _dp, _i64, _dp, _dp, _ip]),
+    'pgp_batch_create': (C.c_int, [_vp, _sp, _dp, _dp, _i64, _dp, _i64, _i64, C.POINTER(_vp), _ip]),
+    'pgp_batch_predict': (C.c_int, [_vp, _dp, _i64, _dp, _dp, _dp, _dp]),
+    'pgp_batch_resident': (_i64, [_vp]),
+    'pgp_batch_destroy': (None, [_vp]),
     'pgp_fitc_create': (C.c_int, [_vp, _sp, _dp, _i64, _dp, _dp, _i64, C.POINTER(_vp)]),
     'pgp_dtc_create': (C.c_int, [_vp, _sp, _dp, _i64, _dp, _dp, _i64, C.POINTER(_vp)]),
     'pgp_fitc_destroy': (None, [_vp]),

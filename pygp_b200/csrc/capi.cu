@@ -1105,12 +1105,123 @@ extern "C" int pgp_exact_get_factor(pgp_model* m, double* R_out, double* a_out) 
 // ---------------------------------------------------------------------------
 // batched small-N path
 // ---------------------------------------------------------------------------
+namespace {
+
+// bc problems sharing X, y in one set of buffers: per-problem specs, scaled inputs, factors (n + 1, ld)
+// with a in row n, potrf info and lZ
+struct ProblemChunk {
+    int bc = 0;
+    DevSpec* spec = nullptr;     // device [bc]
+    double* Z = nullptr;         // device [bc] z_doubles(np, d, n)
+    Mat F;                       // F.batch = bc, F.bstride = (n + 1) ld
+    int* info = nullptr;         // device [bc]
+    double* lZ = nullptr;        // device [bc]
+};
+
+// ExactGP._update (exact.py:50-55) of the problems hyps[0 .. c.bc) into the chunk's buffers, all in the same
+// launches; the host copies of the specs go to hspecs[0 .. bc)
+int factor_chunk(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double* dX, const double* dy, int64_t n,
+                 const double* hyps, const ProblemChunk& c, DevSpec* hspecs) {
+    const int d = spec->ndim, np = spec->n_parts, nk = spec->nhyper, nh = nk + 2;
+    const int bc = c.bc;
+    for (int b = 0; b < bc; ++b) {
+        const double* h = hyps + (size_t)b * nh;
+        PGP_TRY(compile_spec(spec, h + 1, std::exp(h[0] * 2), h[1 + nk], &hspecs[b], &ctx->err));
+    }
+    PGP_CUDA(ctx, cudaMemcpyAsync(c.spec, hspecs, sizeof(DevSpec) * bc, cudaMemcpyHostToDevice, ctx->stream));
+    PGP_CUDA(ctx, cudaMemsetAsync(c.info, 0, sizeof(int) * bc, ctx->stream));
+    PGP_TRY(launch_scale(ctx, c.spec, dX, n, d, np, c.Z, bc));
+    GramArgs g;
+    g.spec = c.spec;
+    g.Z1 = g.Z2 = c.Z;
+    g.n1 = g.n2 = n;
+    g.ndim = d;
+    g.n_parts = np;
+    g.out = c.F.p;
+    g.ldo = c.F.ld;
+    g.out_bstride = c.F.bstride;
+    g.lower_only = 1;
+    g.add_noise = 1;
+    g.batch = bc;
+    g.single_type = single_type(spec);
+    PGP_TRY(launch_gram(ctx, g));
+    PGP_TRY(launch_set_residual(ctx, c.F, n, dy, c.spec));
+    if (trsv_lower_supported(n)) {
+        // a = L^-1 r by its own batched substitution: as an extra row of the
+        // factorisation it would cost a 128-row tile in every trailing update
+        PGP_TRY(potrf_lower(ctx, c.F, n, 0, c.info));
+        PGP_TRY(launch_trsv_lower(ctx, c.F, n));
+    } else {
+        PGP_TRY(potrf_lower(ctx, c.F, n, 1, c.info));
+    }
+    return launch_loglik(ctx, c.F, n, c.lZ);
+}
+
+// Posterior of a factored chunk at ms test points dXs (exact.py:81-97): mu, s2 (bc, ms) on the device.  With
+// dmu, ds2 ((bc, ms, ndim), device) also the input-gradients (exact.py:99-116) in contraction form: after
+// predict_reduce has consumed V = (L^-1 k(X, X*))^T, the rows [V; a] are solved once more, [V; a] L^-1 =
+// [W; alpha^T], and xgrad_gram_kernel contracts them with the gradient Gram.
+// Scratch: Zs (bc z_doubles(np, d, ms)), Bm (bc, ms + 1 with gradients, ld).
+int predict_chunk(pgp_ctx* ctx, const pgp_kernel_spec* spec, int64_t n, const ProblemChunk& c, const double* dXs,
+                  int64_t ms, double* dZs, const Mat& Bm, double* mu, double* s2, double* dmu, double* ds2) {
+    const int d = spec->ndim, np = spec->n_parts;
+    const int64_t ld = c.F.ld;
+    PGP_TRY(launch_scale(ctx, c.spec, dXs, ms, d, np, dZs, c.bc));
+    GramArgs g;
+    g.spec = c.spec;
+    g.Z1 = dZs;
+    g.Z2 = c.Z;
+    g.n1 = ms;
+    g.n2 = n;
+    g.ndim = d;
+    g.n_parts = np;
+    g.out = Bm.p;
+    g.ldo = ld;
+    g.out_bstride = Bm.bstride;
+    g.batch = c.bc;
+    g.single_type = single_type(spec);
+    PGP_TRY(launch_gram(ctx, g));
+    PGP_TRY(trsm_right_lt(ctx, Bm, ms, c.F, n));
+    PGP_TRY(launch_predict_reduce(ctx, Bm.p, ld, ms, n, c.F.p + n * ld, c.spec, mu, s2, c.bc, Bm.bstride,
+                                  c.F.bstride, ms));
+    if (!dmu) return 0;
+    PGP_CUDA(ctx, cudaMemcpy2DAsync(Bm.p + ms * ld, sizeof(double) * Bm.bstride, c.F.p + n * ld,
+                                    sizeof(double) * c.F.bstride, sizeof(double) * n, c.bc, cudaMemcpyDeviceToDevice,
+                                    ctx->stream));
+    PGP_TRY(trsm_right_l(ctx, Bm, ms + 1, c.F, n));
+    XgradArgs x;
+    x.spec = c.spec;
+    x.Zs = dZs;
+    x.Z = c.Z;
+    x.ms = ms;
+    x.n = n;
+    x.ndim = d;
+    x.n_parts = np;
+    x.W = Bm.p;
+    x.ldw = ld;
+    x.w_bstride = Bm.bstride;
+    x.dmu = dmu;
+    x.ds2 = ds2;
+    x.out_bstride = ms * d;
+    x.batch = c.bc;
+    x.single_type = single_type(spec);
+    return launch_xgrad(ctx, x);
+}
+
+int check_batched_args(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double* X, const double* y, int64_t n,
+                       const double* hyps, int64_t B) {
+    if (!spec || !X || !y || !hyps || n <= 0 || B < 0) return ctx->fail(PGP_E_ARG, "null argument or bad size");
+    if (spec->n_parts * spec->ndim > 192) return ctx->fail(PGP_E_ARG, "n_parts * ndim > 192 not supported");
+    return 0;
+}
+
+}  // namespace
+
 static int batched_impl(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double* X, const double* y, int64_t n,
                         const double* hyps, int64_t B, const double* Xs, int64_t ms, double* lZ, double* dlZ, double* mu,
                         double* s2, int32_t* info) {
     if (!ctx) return PGP_E_ARG;
-    if (!spec || !X || !y || !hyps || n <= 0 || B < 0) return ctx->fail(PGP_E_ARG, "null argument or bad size");
-    if (spec->n_parts * spec->ndim > 192) return ctx->fail(PGP_E_ARG, "n_parts * ndim > 192 not supported");
+    PGP_TRY(check_batched_args(ctx, spec, X, y, n, hyps, B));
     PGP_TRY(set_device(ctx));
     if (B == 0) return 0;
     const int d = spec->ndim, np = spec->n_parts, nk = spec->nhyper, nh = nk + 2;
@@ -1180,43 +1291,19 @@ static int batched_impl(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double*
     } ev_guard{ev_main, ev_aux};
 
     for (int64_t b0 = 0; b0 < B; b0 += chunk) {
-        const int bc = (int)std::min<int64_t>(chunk, B - b0);
-        for (int b = 0; b < bc; ++b) {
-            const double* h = hyps + (b0 + b) * nh;
-            PGP_TRY(compile_spec(spec, h + 1, std::exp(h[0] * 2), h[1 + nk], &hspecs[b], &ctx->err));
-        }
-        PGP_CUDA(ctx, cudaMemcpyAsync(dspec.p, hspecs.data(), sizeof(DevSpec) * bc, cudaMemcpyHostToDevice, ctx->stream));
-        PGP_CUDA(ctx, cudaMemsetAsync(dinfo.p, 0, sizeof(int) * bc, ctx->stream));
-        PGP_TRY(launch_scale(ctx, dspec.as<DevSpec>(), dX.as<double>(), n, d, np, dZ.as<double>(), bc));
-        Mat F;
-        F.p = dF.p;
-        F.ld = ld;
-        F.bstride = (n + 1) * ld;
-        F.batch = bc;
-        GramArgs g;
-        g.spec = dspec.as<DevSpec>();
-        g.Z1 = g.Z2 = dZ.as<double>();
-        g.n1 = g.n2 = n;
-        g.ndim = d;
-        g.n_parts = np;
-        g.out = F.p;
-        g.ldo = ld;
-        g.out_bstride = F.bstride;
-        g.lower_only = 1;
-        g.add_noise = 1;
-        g.batch = bc;
-        g.single_type = single_type(spec);
-        PGP_TRY(launch_gram(ctx, g));
-        PGP_TRY(launch_set_residual(ctx, F, n, dy.as<double>(), dspec.as<DevSpec>()));
-        if (trsv_lower_supported(n)) {
-            // a = L^-1 r by its own batched substitution: as an extra row of the
-            // factorisation it would cost a 128-row tile in every trailing update
-            PGP_TRY(potrf_lower(ctx, F, n, 0, dinfo.as<int>()));
-            PGP_TRY(launch_trsv_lower(ctx, F, n));
-        } else {
-            PGP_TRY(potrf_lower(ctx, F, n, 1, dinfo.as<int>()));
-        }
-        PGP_TRY(launch_loglik(ctx, F, n, dres.as<double>()));
+        ProblemChunk c;
+        c.bc = (int)std::min<int64_t>(chunk, B - b0);
+        c.spec = dspec.as<DevSpec>();
+        c.Z = dZ.as<double>();
+        c.F.p = dF.p;
+        c.F.ld = ld;
+        c.F.bstride = (n + 1) * ld;
+        c.F.batch = c.bc;
+        c.info = dinfo.as<int>();
+        c.lZ = dres.as<double>();
+        const int bc = c.bc;
+        const Mat& F = c.F;
+        PGP_TRY(factor_chunk(ctx, spec, dX.as<double>(), dy.as<double>(), n, hyps + b0 * nh, c, hspecs.data()));
         PGP_CUDA(ctx, cudaMemcpyAsync(hres.data(), dres.p, sizeof(double) * bc, cudaMemcpyDeviceToHost, ctx->stream));
         PGP_CUDA(ctx, cudaMemcpyAsync(hinfo.data(), dinfo.p, sizeof(int) * bc, cudaMemcpyDeviceToHost, ctx->stream));
         if (grad) {
@@ -1257,31 +1344,15 @@ static int batched_impl(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double*
             PGP_CUDA(ctx, cudaMemcpyAsync(hgrad.data(), dgrad.p, sizeof(double) * bc * nh, cudaMemcpyDeviceToHost, main_s));
         }
         if (pred) {
-            PGP_TRY(launch_scale(ctx, dspec.as<DevSpec>(), dXs.as<double>(), ms, d, np, dZs.as<double>(), bc));
-            GramArgs c;
-            c.spec = dspec.as<DevSpec>();
-            c.Z1 = dZs.as<double>();
-            c.Z2 = dZ.as<double>();
-            c.n1 = ms;
-            c.n2 = n;
-            c.ndim = d;
-            c.n_parts = np;
-            c.out = dB.p;
-            c.ldo = ld;
-            c.out_bstride = ms * ld;
-            c.batch = bc;
-            c.single_type = single_type(spec);
-            PGP_TRY(launch_gram(ctx, c));
             Mat Bm;
             Bm.p = dB.p;
             Bm.ld = ld;
             Bm.bstride = ms * ld;
             Bm.batch = bc;
-            PGP_TRY(trsm_right_lt(ctx, Bm, ms, F, n));
             double* dmu = dout.as<double>();
             double* ds2 = dmu + (size_t)chunk * ms;
-            PGP_TRY(launch_predict_reduce(ctx, Bm.p, ld, ms, n, F.p + n * ld, dspec.as<DevSpec>(), dmu, ds2, bc,
-                                          Bm.bstride, F.bstride, ms));
+            PGP_TRY(predict_chunk(ctx, spec, n, c, dXs.as<double>(), ms, dZs.as<double>(), Bm, dmu, ds2, nullptr,
+                                  nullptr));
             PGP_CUDA(ctx, cudaMemcpyAsync(mu + b0 * ms, dmu, sizeof(double) * bc * ms, cudaMemcpyDeviceToHost, ctx->stream));
             PGP_CUDA(ctx, cudaMemcpyAsync(s2 + b0 * ms, ds2, sizeof(double) * bc * ms, cudaMemcpyDeviceToHost, ctx->stream));
         }
@@ -1306,6 +1377,203 @@ extern "C" int pgp_batched_predict(pgp_ctx* ctx, const pgp_kernel_spec* spec, co
                                    double* mu, double* s2, int32_t* info) {
     if (ctx && (!Xs || !mu || !s2 || ms < 0)) return ctx->fail(PGP_E_ARG, "null or negative argument");
     return batched_impl(ctx, spec, X, y, n, hyps, B, Xs, ms, nullptr, nullptr, mu, s2, info);
+}
+
+// ---------------------------------------------------------------------------
+// resident batch: B hyper vectors on one data set (meta/mcmc.py), factored once and kept in HBM
+// ---------------------------------------------------------------------------
+// Problems are held in chunks of `chunk` problems.  The first `resident` problems (whole chunks) keep their
+// factors in slots of their own; when not all fit the budget, the remaining chunks share one more slot and are
+// factored again, with the same launches, at every predict.
+struct pgp_batch {
+    pgp_ctx* ctx = nullptr;
+    pgp_kernel_spec spec;
+    int64_t n = 0, B = 0, ld = 0;
+    int64_t chunk = 0, resident = 0;
+    int64_t budget = 0;                // bytes
+    std::vector<double> hyps;          // (B, nhyper + 2)
+    double* d_X = nullptr;
+    double* d_y = nullptr;
+    // slots (ceil(resident / chunk), plus one when resident < B): spec, Z, F, info, lZ of `chunk` problems each
+    int64_t slots = 0;
+    DevSpec* d_spec = nullptr;
+    double* d_Z = nullptr;
+    double* d_F = nullptr;
+    int* d_info = nullptr;
+    double* d_lZ = nullptr;
+};
+
+namespace {
+
+size_t batch_problem_bytes(const pgp_kernel_spec* spec, int64_t n) {
+    const int64_t ld = lead_dim(n);
+    return sizeof(double) * ((size_t)(n + 1) * ld + z_doubles(spec->n_parts, spec->ndim, n) + 1) + sizeof(DevSpec) +
+           sizeof(int);
+}
+
+ProblemChunk batch_chunk(const pgp_batch* h, int64_t k) {
+    const int64_t slot = std::min<int64_t>(k, h->slots - 1);
+    const int d = h->spec.ndim, np = h->spec.n_parts;
+    ProblemChunk c;
+    c.bc = (int)std::min<int64_t>(h->chunk, h->B - k * h->chunk);
+    c.spec = h->d_spec + slot * h->chunk;
+    c.Z = h->d_Z + (size_t)slot * h->chunk * z_doubles(np, d, h->n);
+    c.F.p = h->d_F + (size_t)slot * h->chunk * (h->n + 1) * h->ld;
+    c.F.ld = h->ld;
+    c.F.bstride = (h->n + 1) * h->ld;
+    c.F.batch = c.bc;
+    c.info = h->d_info + slot * h->chunk;
+    c.lZ = h->d_lZ + slot * h->chunk;
+    return c;
+}
+
+void batch_free(pgp_batch* h) {
+    pgp_ctx* ctx = h->ctx;
+    cudaSetDevice(ctx->device);
+    cudaStreamSynchronize(ctx->stream);
+    dev_free(ctx, h->d_X);
+    dev_free(ctx, h->d_y);
+    dev_free(ctx, h->d_spec);
+    dev_free(ctx, h->d_Z);
+    dev_free(ctx, h->d_F);
+    dev_free(ctx, h->d_info);
+    dev_free(ctx, h->d_lZ);
+    delete h;
+}
+
+}  // namespace
+
+extern "C" int pgp_batch_create(pgp_ctx* ctx, const pgp_kernel_spec* spec, const double* X, const double* y,
+                                int64_t n, const double* hyps, int64_t B, int64_t budget_bytes, pgp_batch** out,
+                                int32_t* info) {
+    if (!ctx) return PGP_E_ARG;
+    if (!out || !info || B <= 0 || budget_bytes < 0) return ctx->fail(PGP_E_ARG, "null output or bad size");
+    *out = nullptr;
+    PGP_TRY(check_batched_args(ctx, spec, X, y, n, hyps, B));
+    PGP_TRY(set_device(ctx));
+    const int d = spec->ndim, np = spec->n_parts, nh = spec->nhyper + 2;
+    size_t budget = (size_t)budget_bytes;
+    if (!budget) {
+        size_t free_b = 0, total_b = 0;
+        PGP_CUDA(ctx, cudaMemGetInfo(&free_b, &total_b));
+        budget = free_b / 2;
+    }
+    // problems the budget holds; when that is not all of them, a quarter of it is the slot the others are
+    // refactored in (chunks of a quarter still batch well: N = 16384 takes 16 problems at 36 GB)
+    const int64_t fit = std::max<int64_t>(1, (int64_t)(budget / batch_problem_bytes(spec, n)));
+    pgp_batch* h = new (std::nothrow) pgp_batch();
+    if (!h) return PGP_E_NOMEM;
+    h->ctx = ctx;
+    h->spec = *spec;
+    h->n = n;
+    h->B = B;
+    h->ld = lead_dim(n);
+    h->budget = (int64_t)budget;
+    h->hyps.assign(hyps, hyps + (size_t)B * nh);
+    if (fit >= B) {
+        h->chunk = std::min<int64_t>(B, 32768);
+        h->resident = B;
+    } else {
+        h->chunk = std::min<int64_t>(std::max<int64_t>(1, fit / 4), 32768);
+        h->resident = (fit - h->chunk) / h->chunk * h->chunk;
+    }
+    // one slot per resident chunk (the last one may be partial: B need not be a multiple of the chunk), plus the
+    // shared slot of the refactored chunks; no slot holds more problems than there are
+    h->slots = (h->resident + h->chunk - 1) / h->chunk + (h->resident < B ? 1 : 0);
+    const size_t sp = (size_t)std::min<int64_t>(h->slots * h->chunk, B);
+    int rc = dev_alloc(ctx, &h->d_X, (size_t)n * d);
+    if (!rc) rc = dev_alloc(ctx, &h->d_y, (size_t)n);
+    if (!rc) rc = dev_alloc(ctx, &h->d_spec, sp);
+    if (!rc) rc = dev_alloc(ctx, &h->d_Z, sp * z_doubles(np, d, n));
+    if (!rc) rc = dev_alloc(ctx, &h->d_F, sp * (n + 1) * h->ld);
+    if (!rc) rc = dev_alloc(ctx, &h->d_info, sp);
+    if (!rc) rc = dev_alloc(ctx, &h->d_lZ, sp);
+    if (rc) {
+        batch_free(h);
+        return rc;
+    }
+    auto bail = [&](int code) { batch_free(h); return code; };
+    cudaError_t e = cudaMemcpyAsync(h->d_X, X, sizeof(double) * n * d, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h->d_y, y, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) return bail(ctx->cuda_fail(e, "batch upload", __FILE__, __LINE__));
+    // every problem is factored once here for its info; the chunks beyond the resident ones again at predict
+    std::vector<DevSpec> hspecs((size_t)h->chunk);
+    const int64_t nchunks = (B + h->chunk - 1) / h->chunk;
+    for (int64_t k = 0; k < nchunks; ++k) {
+        const ProblemChunk c = batch_chunk(h, k);
+        if ((rc = factor_chunk(ctx, spec, h->d_X, h->d_y, n, hyps + k * h->chunk * nh, c, hspecs.data()))) return bail(rc);
+        e = cudaMemcpyAsync(info + k * h->chunk, c.info, sizeof(int) * c.bc, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) return bail(ctx->cuda_fail(e, "batch factorisation", __FILE__, __LINE__));
+    }
+    *out = h;
+    return 0;
+}
+
+extern "C" int pgp_batch_predict(pgp_batch* h, const double* Xs, int64_t ms, double* mu, double* s2, double* dmu,
+                                 double* ds2) {
+    if (!h) return PGP_E_ARG;
+    pgp_ctx* ctx = h->ctx;
+    if (!Xs || !mu || !s2 || ms < 0 || (!dmu) != (!ds2)) return ctx->fail(PGP_E_ARG, "null or negative argument");
+    PGP_TRY(set_device(ctx));
+    if (ms == 0) return 0;
+    const pgp_kernel_spec* spec = &h->spec;
+    const int d = spec->ndim, np = spec->n_parts, nh = spec->nhyper + 2;
+    const int64_t n = h->n, ld = h->ld, B = h->B, chunk = h->chunk;
+    const bool grad = dmu != nullptr;
+    // test points per pass: the (chunk, points, ld) scratch within batched_impl's rule (24 GiB, half the free memory)
+    size_t free_b = 0, total_b = 0;
+    PGP_CUDA(ctx, cudaMemGetInfo(&free_b, &total_b));
+    const size_t budget = std::min<size_t>((size_t)24 << 30, free_b / 2);
+    const size_t per_point = sizeof(double) * ((size_t)ld + np * d + 2 + (grad ? 2 * d : 0)) * chunk;
+    const int64_t extra = grad ? 1 : 0;                   // row of a below the test points
+    int64_t mc = std::max<int64_t>(1, (int64_t)(budget / per_point) - extra);
+    mc = std::min(mc, ms);
+    DevBuf dXs, dZs, dout, dg, dB;
+    PGP_TRY(alloc<double>(ctx, dXs, (size_t)ms * d));
+    PGP_CUDA(ctx, cudaMemcpyAsync(dXs.p, Xs, sizeof(double) * ms * d, cudaMemcpyHostToDevice, ctx->stream));
+    PGP_TRY(alloc<double>(ctx, dZs, (size_t)chunk * z_doubles(np, d, mc)));
+    PGP_TRY(alloc<double>(ctx, dB, (size_t)chunk * (mc + extra) * ld));
+    PGP_TRY(alloc<double>(ctx, dout, (size_t)chunk * 2 * mc));
+    if (grad) PGP_TRY(alloc<double>(ctx, dg, (size_t)chunk * 2 * mc * d));
+    std::vector<DevSpec> hspecs((size_t)chunk);
+    const int64_t nchunks = (B + chunk - 1) / chunk;
+    for (int64_t k = 0; k < nchunks; ++k) {
+        const ProblemChunk c = batch_chunk(h, k);
+        const int64_t b0 = k * chunk;
+        if (b0 >= h->resident)
+            PGP_TRY(factor_chunk(ctx, spec, h->d_X, h->d_y, n, h->hyps.data() + b0 * nh, c, hspecs.data()));
+        for (int64_t s0 = 0; s0 < ms; s0 += mc) {
+            const int64_t mcs = std::min(mc, ms - s0);
+            Mat Bm;
+            Bm.p = dB.as<double>();
+            Bm.ld = ld;
+            Bm.bstride = (mcs + extra) * ld;
+            Bm.batch = c.bc;
+            double* dm = dout.as<double>();
+            double* dv = dm + (size_t)chunk * mcs;
+            double* gm = grad ? dg.as<double>() : nullptr;
+            double* gv = grad ? gm + (size_t)chunk * mcs * d : nullptr;
+            PGP_TRY(predict_chunk(ctx, spec, n, c, dXs.as<double>() + s0 * d, mcs, dZs.as<double>(), Bm, dm, dv, gm, gv));
+            cudaStream_t st = ctx->stream;
+            const size_t row = sizeof(double) * ms, w = sizeof(double) * mcs;
+            PGP_CUDA(ctx, cudaMemcpy2DAsync(mu + b0 * ms + s0, row, dm, w, w, c.bc, cudaMemcpyDeviceToHost, st));
+            PGP_CUDA(ctx, cudaMemcpy2DAsync(s2 + b0 * ms + s0, row, dv, w, w, c.bc, cudaMemcpyDeviceToHost, st));
+            if (grad) {
+                const size_t grow = row * d, gw = w * d;
+                PGP_CUDA(ctx, cudaMemcpy2DAsync(dmu + (b0 * ms + s0) * d, grow, gm, gw, gw, c.bc, cudaMemcpyDeviceToHost, st));
+                PGP_CUDA(ctx, cudaMemcpy2DAsync(ds2 + (b0 * ms + s0) * d, grow, gv, gw, gw, c.bc, cudaMemcpyDeviceToHost, st));
+            }
+            PGP_CUDA(ctx, cudaStreamSynchronize(st));     // the scratch is reused by the next pass
+        }
+    }
+    return 0;
+}
+
+extern "C" int64_t pgp_batch_resident(const pgp_batch* h) { return h ? h->resident : 0; }
+
+extern "C" void pgp_batch_destroy(pgp_batch* h) {
+    if (h) batch_free(h);
 }
 
 // ---------------------------------------------------------------------------

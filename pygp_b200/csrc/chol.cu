@@ -436,6 +436,9 @@ int trsm_nt_rec(pgp_ctx* ctx, const Mat& B, int64_t rows, const Mat& L, int64_t 
     g.alpha = -1.0; g.beta = 1.0;
     g.transB = 1;
     g.splitk = 1;
+    g.batch = B.batch;
+    g.strideA = g.strideC = B.bstride;
+    g.strideB = L.bstride;
     PGP_TRY(launch_gemm(ctx, g));
     return trsm_nt_rec(ctx, B, rows, L, j0, n1);
 }
@@ -642,7 +645,7 @@ int trsm_right_lt(pgp_ctx* ctx, const Mat& B, int64_t rows, const Mat& L, int64_
 
 int trsm_right_l(pgp_ctx* ctx, const Mat& B, int64_t rows, const Mat& L, int64_t n) {
     if (n <= 0 || rows <= 0) return 0;
-    if (B.batch != 1 || L.batch != 1) return ctx->fail(PGP_E_ARG, "trsm_right_l: not batched");
+    if (B.batch != L.batch) return ctx->fail(PGP_E_ARG, "trsm_right_l: B and L batches differ");
     return trsm_nt_rec(ctx, B, rows, L, 0, n);
 }
 

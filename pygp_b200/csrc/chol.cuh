@@ -32,7 +32,7 @@ bool trsv_lower_supported(int64_t n);
 // B[:, 0:n) <- B L^-T for `rows` rows of B (same column space as L).
 int trsm_right_lt(pgp_ctx* ctx, const Mat& B, int64_t rows, const Mat& L, int64_t n);
 
-// B[:, 0:n) <- B L^-1 (no transpose) for `rows` rows of B.
+// B[:, 0:n) <- B L^-1 (no transpose) for `rows` rows of B; batched as trsm_right_lt (B.batch == L.batch).
 int trsm_right_l(pgp_ctx* ctx, const Mat& B, int64_t rows, const Mat& L, int64_t n);
 
 // "Staircase" right-solves for the block-column partition of the gradient (dist.cu): the rows of B are

@@ -286,6 +286,27 @@ __device__ __forceinline__ double leaf_gradx(const DevPart& p, const PartVal& v,
     return -v.ardw * sdiff / ellk;
 }
 
+// leaf values and d k / d leaf of a composite at one entry (the input-gradients' tree pass)
+__device__ __forceinline__ void composite_adjoint(const DevSpecHdr& S, const double* z1, const double* z2, PartVal* pv,
+                                                  double* adj) {
+    double val[kMaxNodes];
+    eval_parts<true>(S, z1, z2, pv);
+    tree_forward(S, pv, val);
+    tree_backward(S, val, adj);
+}
+
+// d k / d x1[k] of a composite at one entry from its composite_adjoint
+__device__ __forceinline__ double composite_gradx(const DevSpecHdr& S, const DevSpec* gs, const double* z1,
+                                                  const double* z2, const PartVal* pv, const double* adj, int k) {
+    const int d = S.ndim;
+    double g = 0.0;
+    for (int p = 0; p < S.n_parts; ++p) {
+        double sd = z1[(p * d + k) * kTile] - z2[(p * d + k) * kTile];
+        g += adj[S.leaf_node[p]] * leaf_gradx(S.parts[p], pv[p], sd, gs->ell[p][k]);
+    }
+    return g;
+}
+
 // d^2 k / d x1_a d x2_b of a composite of SE leaves at one entry (se.py:88-99,
 // _real.py:102-103,129-156).  Every node carries (v, dv/dx1_a, dv/dx2_b, d2v/dx1_a dx2_b);
 // sums add them, products fold their children with the second-order product rule
@@ -666,16 +687,9 @@ __global__ void __launch_bounds__(kThreads, (MODE == 0 && is_fast_grad_type(PTYP
                     r = composite_gradxy(*S, a.spec + b, z1, z2, xdim, a.ydim);
                 } else if (GRADX) {
                     PartVal pv[kMaxParts];
-                    double val[kMaxNodes], adj[kMaxNodes];
-                    eval_parts<true>(*S, z1, z2, pv);
-                    tree_forward(*S, pv, val);
-                    tree_backward(*S, val, adj);
-                    double g = 0.0;
-                    for (int p = 0; p < n_parts; ++p) {
-                        double sd = z1[(p * ndim + xdim) * kTile] - z2[(p * ndim + xdim) * kTile];
-                        g += adj[S->leaf_node[p]] * leaf_gradx(S->parts[p], pv[p], sd, a.spec[b].ell[p][xdim]);
-                    }
-                    r = g;
+                    double adj[kMaxNodes];
+                    composite_adjoint(*S, z1, z2, pv, adj);
+                    r = composite_gradx(*S, a.spec + b, z1, z2, pv, adj, xdim);
                 } else if (GRAD1) {
                     r = composite_grad1(*S, z1, z2, gpart, gkind, gdim);
                 } else {
@@ -795,6 +809,138 @@ int launch_gram(pgp_ctx* ctx, const GramArgs& a0) {
         constexpr int PT = decltype(T)::value;
         return mode == 2 ? launch_gram_t<PT, 2>(ctx, a, smem)
                          : (mode == 1 ? launch_gram_t<PT, 1>(ctx, a, smem) : launch_gram_t<PT, 0>(ctx, a, smem));
+    });
+}
+
+// ---------------------------------------------------------------------------
+// posterior input-gradients in contraction form (gram.cuh XgradArgs): CTA (test tile, problem, dimension
+// group) walks the training tiles.  T = 2^lg_tpp threads (4 ... 32, one warp at most) share a test point:
+// thread T r + c owns test point r of the CTA's 256 / T and the columns c + T y of every training tile, and keeps
+// its kXgradDims sums of each kind in registers; the T threads of a test point reduce them by shuffles (fixed
+// order) at the end.  T = 4 fills the CTA with 64 test points; for fewer points (one per step of an
+// acquisition optimiser) the launcher takes a larger T, so that the training points of a tile are spread over
+// more threads instead of leaving most of them idle.  (A 4 x 4 micro-tile per thread, as in gram_kernel, needs
+// 4 x kXgradDims x 2 accumulators and ran into 250 registers.)
+// ---------------------------------------------------------------------------
+template <int PTYPE>
+__global__ void __launch_bounds__(kThreads) xgrad_gram_kernel(XgradArgs a, int bulk, int lg_tpp) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const int ndim = a.ndim, npd = a.n_parts * ndim;
+    const Smem sm(smem_raw, npd);
+    const int b = blockIdx.y;
+    const int tpp = 1 << lg_tpp;
+    const int64_t i0 = (int64_t)blockIdx.x * (kThreads >> lg_tpp);      // rows of the tile past the CTA's: unused
+    const int k0 = blockIdx.z * kXgradDims, kn = min(kXgradDims, ndim - k0);
+    const DevSpec* gs = a.spec + b;
+    const DevSpecHdr* S = PTYPE < 0 ? sm.S : &gs->h;
+    const double* Z1 = a.Zs + (int64_t)b * npd * a.zds;
+    const double* Z2 = a.Z + (int64_t)b * npd * a.zd;
+    const int r = threadIdx.x >> lg_tpp, c0 = threadIdx.x & (tpp - 1);
+    const int64_t gi = i0 + r;
+    const bool rok = gi < a.ms;
+    const double* Wr = a.W + (int64_t)b * a.w_bstride + (rok ? gi : 0) * a.ldw;
+    const double* alpha = a.W + (int64_t)b * a.w_bstride + a.ms * a.ldw;
+    double smu[kXgradDims], ss2[kXgradDims], ell[kXgradDims];
+#pragma unroll
+    for (int kk = 0; kk < kXgradDims; ++kk) {
+        ell[kk] = (PTYPE >= 0 && kk < kn) ? gs->ell[0][k0 + kk] : 1.0;
+        smu[kk] = ss2[kk] = 0.0;
+    }
+    uint32_t phase = 0;
+    const int64_t n_tiles = (a.n + kTile - 1) / kTile;
+    for (int64_t tj = 0; tj < n_tiles; ++tj) {
+        const int64_t j0 = tj * kTile;
+        if (tj == 0) {
+            smem_init_and_issue<(PTYPE < 0)>(sm, gs, Z1, Z2, a.zds, a.zd, i0, j0, npd, bulk);
+        } else {
+            __syncthreads();  // previous tile fully consumed
+            stage_issue(sm, Z1, Z2, a.zds, a.zd, i0, j0, npd, bulk);
+        }
+        stage_wait(sm, bulk, phase);
+        const int ny = rok ? (int)min((int64_t)(kTile >> lg_tpp), (a.n - j0 - c0 + tpp - 1) >> lg_tpp) : 0;   // c0 + T y < n
+        const double* z1 = sm.Zs1 + r;
+        if (PTYPE >= 0) {
+            DevPart part = S->parts[0];
+            part.type = PTYPE;
+#pragma unroll 4
+            for (int y = 0; y < ny; ++y) {
+                const int c = c0 + tpp * y;
+                const double al = alpha[j0 + c], w = Wr[j0 + c];
+                const double* z2 = sm.Zs2 + c;
+                double D = 0.0;
+                for (int k = 0; k < ndim; ++k) {
+                    const double df = z1[k * kTile] - z2[k * kTile];
+                    D = fma(df, df, D);
+                }
+                PartVal pv;
+                leaf_eval<PTYPE, true>(part, D, pv, sm.tab);
+#pragma unroll
+                for (int kk = 0; kk < kXgradDims; ++kk) {
+                    if (kk >= kn) break;
+                    const double sd = z1[(k0 + kk) * kTile] - z2[(k0 + kk) * kTile];
+                    const double g = leaf_gradx(part, pv, sd, ell[kk]);
+                    smu[kk] += g * al;
+                    ss2[kk] += g * w;
+                }
+            }
+        } else {
+#pragma unroll 1
+            for (int y = 0; y < ny; ++y) {
+                const int c = c0 + tpp * y;
+                const double al = alpha[j0 + c], w = Wr[j0 + c];
+                const double* z2 = sm.Zs2 + c;
+                PartVal pv[kMaxParts];
+                double adj[kMaxNodes];
+                composite_adjoint(*S, z1, z2, pv, adj);
+#pragma unroll
+                for (int kk = 0; kk < kXgradDims; ++kk) {
+                    if (kk >= kn) break;
+                    const double g = composite_gradx(*S, gs, z1, z2, pv, adj, k0 + kk);
+                    smu[kk] += g * al;
+                    ss2[kk] += g * w;
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int kk = 0; kk < kXgradDims; ++kk) {
+        if (kk >= kn) break;
+        double vm = smu[kk], vs = ss2[kk];
+        for (int o = 1; o < tpp; o <<= 1) {
+            vm += __shfl_xor_sync(0xffffffffu, vm, o);
+            vs += __shfl_xor_sync(0xffffffffu, vs, o);
+        }
+        if (c0 == 0 && rok) {
+            const int64_t o = (int64_t)b * a.out_bstride + gi * ndim + k0 + kk;
+            a.dmu[o] = vm;
+            a.ds2[o] = -2.0 * vs;
+        }
+    }
+}
+
+int launch_xgrad(pgp_ctx* ctx, const XgradArgs& a0) {
+    if (a0.ms <= 0 || a0.n <= 0 || a0.batch <= 0) return 0;
+    if (a0.n_parts * a0.ndim > 192)
+        return ctx->fail(PGP_E_ARG, "input-gradients: n_parts * ndim > 192 exceeds the shared-memory tile");
+    if (a0.batch > 65535) return ctx->fail(PGP_E_ARG, "input-gradients: more than 65535 problems in one launch");
+    // threads per test point: the largest of 4 ... 32 that still gives every thread of the CTA a test point
+    int lg_tpp = 2;
+    while (lg_tpp < 5 && a0.ms <= (kThreads >> (lg_tpp + 1))) ++lg_tpp;
+    const int64_t t1 = ceil_div(a0.ms, (int64_t)(kThreads >> lg_tpp));
+    if (t1 > 0x7fffffffLL) return ctx->fail(PGP_E_ARG, "input-gradients: too many test points in one launch");
+    XgradArgs a = a0;
+    if (!a.zds) a.zds = z_stride(a.ms);
+    if (!a.zd) a.zd = z_stride(a.n);
+    const int bulk = bulk_ok(a.Zs, a.zds) && bulk_ok(a.Z, a.zd);
+    const size_t smem = kSmemFixed + 2ull * a.n_parts * a.ndim * kTile * sizeof(double);
+    const dim3 grid((unsigned)t1, (unsigned)a.batch, (unsigned)ceil_div(a.ndim, kXgradDims));
+    return with_leaf_type(a.n_parts == 1 ? a.single_type : -1, [&](auto T) {
+        auto kern = xgrad_gram_kernel<decltype(T)::value>;
+        PGP_TRY(ensure_dyn_smem(ctx, kern, smem));
+        // work: the entries of the gradient Gram (one per test point, training point and dimension)
+        Launch L(ctx, PC_GRAM, 8.0 * (double)a.ms * (double)a.n * a.ndim * a.batch);
+        kern<<<grid, kThreads, smem, ctx->stream>>>(a, bulk, lg_tpp);
+        return check_launch(ctx, "xgrad_gram_kernel");
     });
 }
 

@@ -110,6 +110,30 @@ struct TraceDistArgs : TraceTiles {
 };
 int launch_trace_dist(pgp_ctx* ctx, const TraceDistArgs& a);
 
+// Posterior input-gradients of B exact GPs in contraction form (exact.py:99-116 with a = R^-T r):
+//     dmu[b][j][k] =      sum_i d k(x*_j, x_i) / d x*_jk  alpha_i
+//     ds2[b][j][k] = -2 * sum_i d k(x*_j, x_i) / d x*_jk  W_ji,     W = K~^-1 k(X, X*)
+// (stationary kernels: d k(x*, x*) / d x* = 0).  One tile kernel (gram.cu xgrad_gram_kernel) per
+// (problem, 8 ... 64 test points, group of kXgradDims input dimensions) walks the training tiles with the
+// gradient Gram recomputed from the inputs, never stored; every sum has a fixed order.
+constexpr int kXgradDims = 4;
+struct XgradArgs {
+    const DevSpec* spec = nullptr;   // device, [batch]
+    const double* Zs = nullptr;      // test inputs   [batch][parts][d][zds]
+    const double* Z = nullptr;       // training inputs [batch][parts][d][zd]
+    int64_t ms = 0, n = 0;
+    int64_t zds = 0, zd = 0;         // 0: z_stride(ms) / z_stride(n)
+    int ndim = 0, n_parts = 0;
+    const double* W = nullptr;       // [batch] rows [0, ms): W, row ms: alpha^T; (ms + 1, ldw)
+    int64_t ldw = 0, w_bstride = 0;
+    double* dmu = nullptr;           // device [batch] (ms, ndim)
+    double* ds2 = nullptr;
+    int64_t out_bstride = 0;
+    int batch = 1;
+    int single_type = -1;
+};
+int launch_xgrad(pgp_ctx* ctx, const XgradArgs& a);
+
 // out[h][i] = d k(x_i, x_i) / d hyper_h for h < nhyper (hmode=1) or k(x_i,x_i) (hmode=0)
 int launch_diag(pgp_ctx* ctx, const DevSpec* d_spec, int64_t n, int hmode, int nhyper, double* d_out);
 

@@ -10,7 +10,9 @@ plumbing.
                         meta/mcmc.py:75-93): each rank evaluates B/G of them; results
                         all-gathered.  No data-path collective.
   * mixture moments  -- MCMC.posterior (mcmc.py:84-93) over sharded samples needs two
-                        small all-reduces: sum mu_i, then sum (s2_i + (mu_i - mu)^2).
+                        small all-reduces: sum mu_i, then sum (s2_i + (mu_i - mu)^2); with
+                        input-gradients the same two carry sum dmu_i and
+                        sum (ds2_i + 2 (mu_i - mu)(dmu_i - dmu)) along.
 
 The optimiser / slice-sampler loops are sequential: replicas only (one restart or
 chain per GPU), nothing to do here.
@@ -182,23 +184,42 @@ def sharded_batched_loglike(gp, hypers, group=None, local_fn=None, grad=False):
     return (out[:, 0].copy(), out[:, 1:].copy()) if grad else out
 
 
-def sharded_mixture_posterior(gp, hypers, X, group=None, local_fn=None):
+def sharded_mixture_posterior(gp, hypers, X, group=None, local_fn=None, grad=False):
     """Moment-matched mixture posterior over hyper samples (mcmc.py:84-93):
     mu = mean_i mu_i, s2 = mean_i (s2_i + (mu_i - mu)^2), samples split across
-    the ranks.  `local_fn(hypers_slice, X) -> (mu_ (b, m), s2_ (b, m))`."""
+    the ranks.  `local_fn(hypers_slice, X) -> (mu_ (b, m), s2_ (b, m))`.
+    grad=True also returns the input-gradients dmu = mean_i dmu_i and
+    ds2 = mean_i (ds2_i + 2 (mu_i - mu)(dmu_i - dmu)); local_fn then returns
+    (mu_, s2_, dmu_ (b, m, d), ds2_ (b, m, d)).  Two all-reduces either way:
+    [sum mu_i, sum dmu_i], then the two centred sums."""
     rank, size = world(group)
     hypers = np.array(hypers, ndmin=2, dtype=float)
     X = np.array(X, ndmin=2, dtype=float)
-    B, m = len(hypers), len(X)
+    B, m, d = len(hypers), len(X), X.shape[1]
     lo, hi = shard_range(B, rank, size)
-    fn = local_fn or (lambda h, x: _batched('predict', gp, h, x))
-    err, mu_, s2_ = None, np.empty((0, m)), np.empty((0, m))
+    if local_fn is None:
+        if grad:
+            from .meta.mcmc import _DeviceBatch
+            local_fn = lambda h, x: _DeviceBatch(gp, h).predict(x, True)   # noqa: E731
+        else:
+            local_fn = lambda h, x: _batched('predict', gp, h, x)          # noqa: E731
+    err = None
+    parts = (np.empty((0, m)), np.empty((0, m))) + ((np.empty((0, m, d)), np.empty((0, m, d))) if grad else ())
     try:
         if hi > lo:
-            mu_, s2_ = fn(hypers[lo:hi], X)
+            parts = local_fn(hypers[lo:hi], X)
     except Exception as e:                # noqa: BLE001 -- e.g. LinAlgError on the one rank whose slice is non-PD
         err = e
     _raise_together(err, group)           # before the all-reduces: every rank raises, nobody deadlocks
-    mu = all_reduce_sum(np.sum(mu_, axis=0), group)/B
-    s2 = all_reduce_sum(np.sum(s2_ + (mu_ - mu)**2, axis=0), group)/B
-    return mu, s2
+    if not grad:
+        mu_, s2_ = parts
+        mu = all_reduce_sum(np.sum(mu_, axis=0), group)/B
+        s2 = all_reduce_sum(np.sum(s2_ + (mu_ - mu)**2, axis=0), group)/B
+        return mu, s2
+    mu_, s2_, dmu_, ds2_ = (np.asarray(p, dtype=float) for p in parts)
+    first = all_reduce_sum(np.concatenate([np.sum(mu_, axis=0), np.sum(dmu_, axis=0).ravel()]), group)/B
+    mu, dmu = first[:m], first[m:].reshape(m, d)
+    Mu = mu_ - mu
+    second = all_reduce_sum(np.concatenate([np.sum(s2_ + Mu**2, axis=0),
+                                            np.sum(ds2_ + 2*Mu[:, :, None]*(dmu_ - dmu), axis=0).ravel()]), group)/B
+    return mu, second[:m], dmu, second[m:].reshape(m, d)
