@@ -258,6 +258,12 @@ int pgp_dtc_create(pgp_ctx* ctx, const pgp_kernel_spec* spec,
 int pgp_fitc_update(pgp_fitc* f, const double* hyp);
 /* FITC.loglikelihood(grad) (fitc.py:167-232) */
 int pgp_fitc_loglike(pgp_fitc* f, int want_grad, double* lZ, double* dlZ);
+/* lZ, dlZ (nhyper + 2, as pgp_fitc_loglike with want_grad = 1) and dU = dlZ / dU (p, ndim, row-major
+   like U) at the current factorisation; FITC or DTC according to the create call.  lZ and dlZ are
+   bitwise those of pgp_fitc_loglike(f, 1, ...); repeated calls give bitwise-equal dU. */
+int pgp_fitc_loglike_pseudo(pgp_fitc* f, double* lZ, double* dlZ, double* dU);
+/* replace the p pseudo-inputs (same p, ndim); the state is unfactored until the next pgp_fitc_update */
+int pgp_fitc_set_pseudoinputs(pgp_fitc* f, const double* U);
 /* FITC._marg_posterior(X, grad=False) (fitc.py:122-142) */
 int pgp_fitc_predict(pgp_fitc* f, const double* Xs, int64_t ms,
                      double* mu, double* s2);

@@ -103,6 +103,8 @@ SIGNATURES = {
     'pgp_fitc_destroy': (None, [_vp]),
     'pgp_fitc_update': (C.c_int, [_vp, _dp]),
     'pgp_fitc_loglike': (C.c_int, [_vp, C.c_int, _dp, _dp]),
+    'pgp_fitc_loglike_pseudo': (C.c_int, [_vp, _dp, _dp, _dp]),
+    'pgp_fitc_set_pseudoinputs': (C.c_int, [_vp, _dp]),
     'pgp_fitc_predict': (C.c_int, [_vp, _dp, _i64, _dp, _dp]),
     'pgp_fitc_full_posterior': (C.c_int, [_vp, _dp, _i64, _dp, _dp]),
     'pgp_fitc_predict_grad': (C.c_int, [_vp, _dp, _i64, _dp, _dp, _dp, _dp]),

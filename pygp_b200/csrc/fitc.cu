@@ -653,14 +653,10 @@ extern "C" int pgp_fitc_update(pgp_fitc* f, const double* hyp) {
     return 0;
 }
 
-extern "C" int pgp_fitc_loglike(pgp_fitc* f, int want_grad, double* lZ, double* dlZ) {
-    if (!f) return PGP_E_ARG;
+// enqueue the gradient of lZ (fitc.py:167-232): dlZ lands in d_res[1 .. nk + 2], and Cuu, Bt, T2, alpha, q
+// (FITC) and w stay resident for pgp_fitc_loglike_pseudo
+static int fitc_grad_launch(pgp_fitc* f) {
     pgp_ctx* ctx = f->ctx;
-    if (!lZ || (want_grad && !dlZ)) return ctx->fail(PGP_E_ARG, "null output");
-    if (!f->factored) return ctx->fail(PGP_E_STATE, "loglike before a successful update");
-    *lZ = f->lZ;
-    if (!want_grad) return 0;
-    PGP_CUDA(ctx, cudaSetDevice(ctx->device));
     const int nk = f->spec.nhyper, d = f->ndim, np = f->spec.n_parts;
     const int64_t n = f->n, p = f->p, ldp = f->ldp;
     cudaStream_t s = ctx->stream;
@@ -753,11 +749,72 @@ extern "C" int pgp_fitc_loglike(pgp_fitc* f, int want_grad, double* lZ, double* 
     t.sym = 0;
     t.mode = 1; t.Bt = f->d_Bt; t.T2 = f->d_T; t.al = f->d_alpha; t.q = f->dtc ? nullptr : f->d_q; t.wv = f->d_w;
     if (f->dtc) t.scale = 0.5 / std::sqrt(f->hspec[0].h.sn2);      // the 2 / ell of M = 2 dKux / ell - dKuu B (dtc.py:189)
-    PGP_TRY(launch_trace_rect(ctx, t));
+    return launch_trace_rect(ctx, t);
+}
+
+extern "C" int pgp_fitc_loglike(pgp_fitc* f, int want_grad, double* lZ, double* dlZ) {
+    if (!f) return PGP_E_ARG;
+    pgp_ctx* ctx = f->ctx;
+    if (!lZ || (want_grad && !dlZ)) return ctx->fail(PGP_E_ARG, "null output");
+    if (!f->factored) return ctx->fail(PGP_E_STATE, "loglike before a successful update");
+    *lZ = f->lZ;
+    if (!want_grad) return 0;
+    PGP_CUDA(ctx, cudaSetDevice(ctx->device));
+    PGP_TRY(fitc_grad_launch(f));
+    const int nk = f->spec.nhyper;
+    double* hp = ctx->h_pin;
+    PGP_CUDA(ctx, cudaMemcpyAsync(hp, f->d_res + 1, sizeof(double) * (nk + 2), cudaMemcpyDeviceToHost, ctx->stream));
+    PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    for (int i = 0; i < nk + 2; ++i) dlZ[i] = hp[i];
+    return 0;
+}
+
+// d lZ / d U from the weights the gradient left resident (gram.cuh PseudoGradArgs): the hyper-gradient's
+// regrouped traces hold for any parameter Kuu, Kxu and kxx depend on; for these stationary kernels
+// d kxx / d U = 0 and d k(u, u) / d u = 0, and the su2 jitter does not depend on U, so only the two
+// contractions with d k(u_j, .) / d u_j remain (oracle/fitc_model.py fitc_pseudo_grad / dtc_pseudo_grad)
+extern "C" int pgp_fitc_loglike_pseudo(pgp_fitc* f, double* lZ, double* dlZ, double* dU) {
+    if (!f) return PGP_E_ARG;
+    pgp_ctx* ctx = f->ctx;
+    if (!lZ || !dlZ || !dU) return ctx->fail(PGP_E_ARG, "null output");
+    if (!f->factored) return ctx->fail(PGP_E_STATE, "loglike before a successful update");
+    *lZ = f->lZ;
+    PGP_CUDA(ctx, cudaSetDevice(ctx->device));
+    PGP_TRY(fitc_grad_launch(f));
+    const int nk = f->spec.nhyper, d = f->ndim;
+    const int64_t n = f->n, p = f->p;
+    cudaStream_t s = ctx->stream;
+    const size_t npart = pseudo_grad_partial_doubles(p, n, d);
+    PGP_TRY(ensure_part(f, npart + (size_t)p * d));
+    PseudoGradArgs g;
+    g.spec = f->d_spec;
+    g.ZU = f->d_ZU; g.ZX = f->d_ZX;
+    g.p = p; g.n = n;
+    g.ndim = d; g.n_parts = f->spec.n_parts;
+    g.Cuu = f->d_Cuu; g.Bt = f->d_Bt; g.T2 = f->d_T;
+    g.al = f->d_alpha; g.q = f->dtc ? nullptr : f->d_q; g.wv = f->d_w;
+    g.ldw = f->ldp;
+    g.sx = f->dtc ? 0.5 / std::sqrt(f->hspec[0].h.sn2) : 0.5;    // the trace scales of the Cxu term above
+    g.partials = f->d_part;
+    g.out = f->d_part + npart;
+    g.single_type = single_type(&f->spec);
+    PGP_TRY(launch_pseudo_grad(ctx, g));
     double* hp = ctx->h_pin;
     PGP_CUDA(ctx, cudaMemcpyAsync(hp, f->d_res + 1, sizeof(double) * (nk + 2), cudaMemcpyDeviceToHost, s));
+    PGP_CUDA(ctx, cudaMemcpyAsync(dU, g.out, sizeof(double) * p * d, cudaMemcpyDeviceToHost, s));
     PGP_CUDA(ctx, cudaStreamSynchronize(s));
     for (int i = 0; i < nk + 2; ++i) dlZ[i] = hp[i];
+    return 0;
+}
+
+extern "C" int pgp_fitc_set_pseudoinputs(pgp_fitc* f, const double* U) {
+    if (!f) return PGP_E_ARG;
+    pgp_ctx* ctx = f->ctx;
+    if (!U) return ctx->fail(PGP_E_ARG, "null pseudo-inputs");
+    PGP_CUDA(ctx, cudaSetDevice(ctx->device));
+    f->factored = false;
+    PGP_CUDA(ctx, cudaMemcpyAsync(f->d_U, U, sizeof(double) * f->p * f->ndim, cudaMemcpyHostToDevice, ctx->stream));
+    PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
 

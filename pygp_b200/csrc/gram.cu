@@ -944,6 +944,192 @@ int launch_xgrad(pgp_ctx* ctx, const XgradArgs& a0) {
     });
 }
 
+// ---------------------------------------------------------------------------
+// FITC / DTC pseudo-input gradient in contraction form (gram.cuh PseudoGradArgs).  CTA (dimension group,
+// split, tile of 64 pseudo-inputs) walks its slice of the column tiles: the ceil(p / 64) tiles of U first
+// (weight Cuu_sym), then the ceil(n / 64) tiles of X (weight Cxu).  Thread jj + 64 g owns pseudo-input jj
+// of the tile and the columns g + 4 y, y < 16, so the 32 lanes of a warp read one 256-byte row segment of
+// Bt and of T2 at a time (stored (n, ldw): one row per datum).  xgrad_gram_kernel puts its lanes along the
+// training index instead, which would make every lane of a warp stride by ldw through these weights; this
+// sibling keeps its staging and leaf_gradx / composite_gradx and only changes who owns which entry.  Each
+// thread keeps kPseudoDims sums; a single leaf's 1 / ell_k is taken out of the sum and applied once at the
+// end.  The four threads of a pseudo-input are added through shared memory in a fixed order, the splits by
+// pseudo_grad_reduce_kernel in a fixed order, so repeated calls give identical bits.
+// ---------------------------------------------------------------------------
+template <int PTYPE>
+__global__ void __launch_bounds__(kThreads) pseudo_gram_kernel(PseudoGradArgs a, int64_t nsplit, int bulk) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const int ndim = a.ndim, npd = a.n_parts * ndim;
+    const Smem sm(smem_raw, npd);
+    const int k0 = blockIdx.x * kPseudoDims, kn = min(kPseudoDims, ndim - k0);
+    const int64_t split = blockIdx.y, j0 = (int64_t)blockIdx.z * kTile;
+    const DevSpecHdr* S = PTYPE < 0 ? sm.S : &a.spec->h;
+    const int jj = threadIdx.x & (kTile - 1), g = threadIdx.x >> 6;
+    const int64_t gj = j0 + jj;
+    const bool rok = gj < a.p;
+    const double wj = rok ? a.wv[gj] : 0.0;
+    const bool hasq = a.q != nullptr;
+    const int64_t tu = (a.p + kTile - 1) / kTile, tx = (a.n + kTile - 1) / kTile, nct = tu + tx;
+    const int64_t zdu = (tu + 1) * kTile, zdx = (tx + 1) * kTile;     // z_stride(p), z_stride(n)
+    const int64_t c_begin = nct * split / nsplit, c_end = nct * (split + 1) / nsplit;   // nsplit <= nct: never empty
+    const double* z1 = sm.Zs1 + jj;
+    double acc[kPseudoDims];
+#pragma unroll
+    for (int kk = 0; kk < kPseudoDims; ++kk) acc[kk] = 0.0;
+    uint32_t phase = 0;
+    for (int64_t ct = c_begin; ct < c_end; ++ct) {
+        const bool xset = ct >= tu;
+        const int64_t i0 = (xset ? ct - tu : ct) * kTile, ncols = xset ? a.n : a.p;
+        const double* Z2 = xset ? a.ZX : a.ZU;
+        const int64_t zd2 = xset ? zdx : zdu;
+        if (ct == c_begin) {
+            smem_init_and_issue<(PTYPE < 0)>(sm, a.spec, a.ZU, Z2, zdu, zd2, j0, i0, npd, bulk);
+        } else {
+            __syncthreads();  // previous tile fully consumed
+            stage_issue(sm, a.ZU, Z2, zdu, zd2, j0, i0, npd, bulk);
+        }
+        stage_wait(sm, bulk, phase);
+        const int ny = rok ? (int)min((int64_t)(kTile / 4), (ncols - i0 - g + 3) / 4) : 0;    // g + 4 y < ncols - i0
+        if (PTYPE >= 0 && ndim <= kPseudoDims) {
+            // one group holds every dimension: the thread's pseudo-input stays in registers and the differences
+            // of the distance are the ones the gradient needs (CTA-uniform branch)
+            DevPart part = S->parts[0];
+            part.type = PTYPE;
+            double zu[kPseudoDims];
+#pragma unroll
+            for (int kk = 0; kk < kPseudoDims; ++kk) zu[kk] = kk < ndim ? z1[kk * kTile] : 0.0;
+            // four iterations in flight where they fit the registers (-Xptxas -v: Matern-1/2, 5/2 and RQ spill
+            // with four, SE spills with one)
+            constexpr int kUnroll = (PTYPE == PGP_SE || PTYPE == PGP_MATERN3 || PTYPE == PGP_PERIODIC) ? 4 : 1;
+#pragma unroll kUnroll
+            for (int y = 0; y < ny; ++y) {
+                const int c = g + 4 * y;
+                const int64_t gi = i0 + c;
+                const double w = xset ? a.sx * (2.0 * (a.al[gi] * wj - (hasq ? a.q[gi] : 1.0) * a.Bt[gi * a.ldw + gj] +
+                                                       a.T2[gi * a.ldw + gj]))
+                                      : (gi >= gj ? a.Cuu[gi * a.ldw + gj] : a.Cuu[gj * a.ldw + gi]);
+                const double* z2 = sm.Zs2 + c;
+                double df[kPseudoDims], D = 0.0;
+#pragma unroll
+                for (int kk = 0; kk < kPseudoDims; ++kk) {
+                    df[kk] = kk < ndim ? zu[kk] - z2[kk * kTile] : 0.0;
+                    D = fma(df[kk], df[kk], D);
+                }
+                PartVal pv;
+                leaf_eval<PTYPE, true>(part, D, pv, sm.tab);
+#pragma unroll
+                for (int kk = 0; kk < kPseudoDims; ++kk)
+                    if (kk < ndim) acc[kk] += w * leaf_gradx(part, pv, df[kk], 1.0);
+            }
+        } else if (PTYPE >= 0) {
+            DevPart part = S->parts[0];
+            part.type = PTYPE;
+#pragma unroll 4
+            for (int y = 0; y < ny; ++y) {
+                const int c = g + 4 * y;
+                const int64_t gi = i0 + c;
+                const double w = xset ? a.sx * (2.0 * (a.al[gi] * wj - (hasq ? a.q[gi] : 1.0) * a.Bt[gi * a.ldw + gj] +
+                                                       a.T2[gi * a.ldw + gj]))
+                                      : (gi >= gj ? a.Cuu[gi * a.ldw + gj] : a.Cuu[gj * a.ldw + gi]);
+                const double* z2 = sm.Zs2 + c;
+                double D = 0.0;
+                for (int k = 0; k < ndim; ++k) {
+                    const double df = z1[k * kTile] - z2[k * kTile];
+                    D = fma(df, df, D);
+                }
+                PartVal pv;
+                leaf_eval<PTYPE, true>(part, D, pv, sm.tab);
+#pragma unroll
+                for (int kk = 0; kk < kPseudoDims; ++kk) {
+                    if (kk >= kn) break;
+                    const double sd = z1[(k0 + kk) * kTile] - z2[(k0 + kk) * kTile];
+                    acc[kk] += w * leaf_gradx(part, pv, sd, 1.0);
+                }
+            }
+        } else {
+#pragma unroll 1
+            for (int y = 0; y < ny; ++y) {
+                const int c = g + 4 * y;
+                const int64_t gi = i0 + c;
+                const double w = xset ? a.sx * (2.0 * (a.al[gi] * wj - (hasq ? a.q[gi] : 1.0) * a.Bt[gi * a.ldw + gj] +
+                                                       a.T2[gi * a.ldw + gj]))
+                                      : (gi >= gj ? a.Cuu[gi * a.ldw + gj] : a.Cuu[gj * a.ldw + gi]);
+                const double* z2 = sm.Zs2 + c;
+                PartVal pv[kMaxParts];
+                double adj[kMaxNodes];
+                composite_adjoint(*S, z1, z2, pv, adj);
+#pragma unroll
+                for (int kk = 0; kk < kPseudoDims; ++kk) {
+                    if (kk >= kn) break;
+                    acc[kk] += w * composite_gradx(*S, a.spec, z1, z2, pv, adj, k0 + kk);
+                }
+            }
+        }
+    }
+    if (PTYPE >= 0 && PTYPE != PGP_PERIODIC) {   // leaf_gradx's -w (z1k - z2k) / ell_k with the division taken out
+#pragma unroll
+        for (int kk = 0; kk < kPseudoDims; ++kk)
+            if (kk < kn) acc[kk] /= a.spec->ell[0][k0 + kk];
+    }
+    double* red = sm.extra;  // [4][64][kPseudoDims]
+#pragma unroll
+    for (int kk = 0; kk < kPseudoDims; ++kk) red[(g * kTile + jj) * kPseudoDims + kk] = acc[kk];
+    __syncthreads();
+    if (g == 0 && rok) {
+        double* o = a.partials + (split * a.p + gj) * ndim + k0;
+        for (int kk = 0; kk < kn; ++kk) {
+            const double* r = red + jj * kPseudoDims + kk;
+            o[kk] = ((r[0] + r[kTile * kPseudoDims]) + r[2 * kTile * kPseudoDims]) + r[3 * kTile * kPseudoDims];
+        }
+    }
+}
+
+// out[e] = sum over splits s = 0, 1, ... of partials[s][e]
+__global__ void pseudo_grad_reduce_kernel(const double* partials, int64_t nsplit, int64_t total, double* out) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= total) return;
+    double s = 0.0;
+    for (int64_t sp = 0; sp < nsplit; ++sp) s += partials[sp * total + e];
+    out[e] = s;
+}
+
+// splits of the p + n columns: about 12 x 148 CTAs of equal work, several waves at two to four resident CTAs
+// per SM, so that the last wave leaves a short tail; at p = 2048 there are only 32 pseudo-input tiles
+static int64_t pseudo_splits(int64_t p, int64_t n, int ndim) {
+    const int64_t tiles = ceil_div(p, kTile) * ceil_div((int64_t)ndim, (int64_t)kPseudoDims);
+    const int64_t cols = ceil_div(p, kTile) + ceil_div(n, kTile);
+    return std::max<int64_t>(1, std::min<int64_t>(cols, ceil_div((int64_t)148 * 12, tiles)));
+}
+
+size_t pseudo_grad_partial_doubles(int64_t p, int64_t n, int ndim) {
+    return (size_t)pseudo_splits(p, n, ndim) * p * ndim;
+}
+
+int launch_pseudo_grad(pgp_ctx* ctx, const PseudoGradArgs& a) {
+    if (a.p <= 0 || a.n <= 0) return 0;
+    if (a.n_parts * a.ndim > 192)
+        return ctx->fail(PGP_E_ARG, "pseudo-input gradient: n_parts * ndim > 192 exceeds the shared-memory tile");
+    const int64_t tp = ceil_div(a.p, kTile), nsplit = pseudo_splits(a.p, a.n, a.ndim);
+    if (tp > 65535) return ctx->fail(PGP_E_ARG, "pseudo-input gradient: more than 65535 pseudo-input tiles");
+    const int bulk = bulk_ok(a.ZU, z_stride(a.p)) && bulk_ok(a.ZX, z_stride(a.n));
+    const size_t smem = kSmemFixed + 2ull * a.n_parts * a.ndim * kTile * sizeof(double) +
+                        4ull * kTile * kPseudoDims * sizeof(double);
+    const dim3 grid((unsigned)ceil_div((int64_t)a.ndim, (int64_t)kPseudoDims), (unsigned)nsplit, (unsigned)tp);
+    PGP_TRY(with_leaf_type(a.n_parts == 1 ? a.single_type : -1, [&](auto T) {
+        auto kern = pseudo_gram_kernel<decltype(T)::value>;
+        PGP_TRY(ensure_dyn_smem(ctx, kern, smem));
+        // work: the entries of the gradient Gram (one per pseudo-input, column and dimension)
+        Launch L(ctx, PC_GRAM, 8.0 * (double)a.p * (double)(a.p + a.n) * a.ndim);
+        kern<<<grid, kThreads, smem, ctx->stream>>>(a, nsplit, bulk);
+        return check_launch(ctx, "pseudo_gram_kernel");
+    }));
+    const int64_t total = a.p * a.ndim;
+    Launch L(ctx, PC_OTHER, 8.0 * (double)(nsplit + 1) * total);
+    pseudo_grad_reduce_kernel<<<(unsigned)ceil_div(total, (int64_t)256), 256, 0, ctx->stream>>>(a.partials, nsplit,
+                                                                                               total, a.out);
+    return check_launch(ctx, "pseudo_grad_reduce_kernel");
+}
+
 // accumulate sum_{entries of one 64 x 64 tile} wq * dK_h for every hyper h into
 // acc[1 + h] (the caller owns acc[0]); K and all dK_h are recomputed from the
 // staged inputs, nothing is read from memory.

@@ -134,6 +134,36 @@ struct XgradArgs {
 };
 int launch_xgrad(pgp_ctx* ctx, const XgradArgs& a);
 
+// Pseudo-input gradient of the FITC / DTC log marginal likelihood in contraction form (fitc.cu):
+//     out[j][k] =       sum_{i < p} Cuu_sym[j,i] d k(u_j, u_i) / d u_jk
+//               + sx * sum_{i < n} Cxu[i,j]     d k(u_j, x_i) / d u_jk
+// with Cuu_sym[j,i] = Cuu[max(i,j)][min(i,j)] (only the lower triangle of Cuu is read) and
+// Cxu = 2 (alpha w^T - diag(q) Bt + T2) built on the fly from its factors, as the Rect trace does.
+// One tile kernel (gram.cu pseudo_gram_kernel) per (64 pseudo-inputs, slice of the p + n columns,
+// group of kPseudoDims input dimensions) leaves partial sums [split][p][ndim] in `partials`; a second
+// kernel adds the splits in a fixed order into `out` (device, (p, ndim)).
+constexpr int kPseudoDims = 8;
+struct PseudoGradArgs {
+    const DevSpec* spec = nullptr;
+    const double* ZU = nullptr;      // [parts][d][z_stride(p)]
+    const double* ZX = nullptr;      // [parts][d][z_stride(n)]
+    int64_t p = 0, n = 0;
+    int ndim = 0, n_parts = 0;
+    const double* Cuu = nullptr;     // (p, ldw), lower triangle
+    const double* Bt = nullptr;      // (n, ldw)
+    const double* T2 = nullptr;      // (n, ldw)
+    const double* al = nullptr;      // (n) alpha
+    const double* q = nullptr;       // (n); nullptr = all ones (DTC)
+    const double* wv = nullptr;      // (p) w
+    int64_t ldw = 0;
+    double sx = 0.5;
+    double* partials = nullptr;      // device scratch, pseudo_grad_partial_doubles(p, n, ndim)
+    double* out = nullptr;
+    int single_type = -1;
+};
+size_t pseudo_grad_partial_doubles(int64_t p, int64_t n, int ndim);
+int launch_pseudo_grad(pgp_ctx* ctx, const PseudoGradArgs& a);
+
 // out[h][i] = d k(x_i, x_i) / d hyper_h for h < nhyper (hmode=1) or k(x_i,x_i) (hmode=0)
 int launch_diag(pgp_ctx* ctx, const DevSpec* d_spec, int64_t n, int hmode, int nhyper, double* d_out);
 

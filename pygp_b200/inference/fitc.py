@@ -5,6 +5,10 @@ Same constructor, properties and error behaviour as the reference; `_update`,
 `loglikelihood` and `_marg_posterior(grad=False)` are single C-ABI calls
 (pgp_fitc_update / _loglike / _predict).  X, y, U and every (n, p) intermediate
 stay in HBM; only the hyper vector goes in and (lZ, dlZ) / (mu, s2) come out.
+
+Beyond the reference: the pseudo-inputs can be moved (`set_pseudoinputs`) and
+`loglikelihood(grad=True, pseudoinputs=True)` also returns d lZ / d U, so that
+`learning.optimize(gp, pseudoinputs=True)` can fit the inducing set.
 """
 
 import ctypes as C
@@ -74,6 +78,27 @@ class FITC(GP):
         """The pseudo-input points."""
         return self._U
 
+    def set_pseudoinputs(self, U):
+        """Move the pseudo-inputs to the rows of U (a copy is kept) and, if data
+        is present, re-factorise, as `set_hyper` does.  U may have a different
+        number of rows; its columns must match the kernel's inputs."""
+        self._set_pseudoinputs(U)
+        if self.ndata > 0:
+            self._update()
+
+    def _set_pseudoinputs(self, U):
+        """Replace U without re-factorising: the device state stays unfactored
+        until the next `_update` (set_hyper / add_data)."""
+        U = np.array(U, ndmin=2, dtype=float, copy=True)
+        if U.shape[1] != self._kernel.ndim:
+            raise ValueError('pseudo-inputs have the wrong number of columns')
+        if self._dev is not None and U.shape[0] == self._U.shape[0]:
+            _lib.check(self._dev.ctx, _lib.lib().pgp_fitc_set_pseudoinputs(self._dev.handle, _lib.ptr(U)))
+        else:
+            self._dev = None            # a different p: rebuilt by the next _update
+            self._ndev = 0
+        self._U = U
+
     @classmethod
     def from_gp(cls, gp, U=None):
         if U is None:
@@ -103,9 +128,17 @@ class FITC(GP):
         if self._dev is None and self.ndata > 0:
             self._update()
 
-    def loglikelihood(self, grad=False):
+    def loglikelihood(self, grad=False, pseudoinputs=False):
+        """lZ; with `grad`, (lZ, dlZ); with `pseudoinputs`, (lZ, dlZ, dU), where
+        dU = d lZ / d U has the shape of `pseudoinputs` (lZ and dlZ are bitwise
+        those of `loglikelihood(True)`)."""
         self._ensure_dev()
         lZ = C.c_double()
+        if pseudoinputs:
+            dlZ, dU = np.empty(self.nhyper), np.empty(self._U.shape)
+            _lib.check(self._dev.ctx, _lib.lib().pgp_fitc_loglike_pseudo(
+                self._dev.handle, C.byref(lZ), _lib.ptr(dlZ), _lib.ptr(dU)))
+            return lZ.value, dlZ, dU
         dlZ = np.empty(self.nhyper) if grad else None
         _lib.check(self._dev.ctx, _lib.lib().pgp_fitc_loglike(
             self._dev.handle, int(bool(grad)), C.byref(lZ), None if dlZ is None else _lib.ptr(dlZ)))

@@ -1,7 +1,7 @@
 """Measure every BASELINE.json config at full size on ONE GPU (run on the GPU box):
   C1 SE 1-D N=1000 + 500 test points        C2 SE-ARD d=8 N=8192 under learning.optimize
   C3 -> bench.py                            C4 4096 hyper samples x N=2048 (batched)
-  C5 SE+Periodic 1-D N=65536 exact; FITC M=2048, N=2^20
+  C5 SE+Periodic 1-D N=65536 exact; FITC M=2048, N=2^20 (c5_fitc_pseudo: with d lZ / d U)
 Prints one JSON line per config (profiles/r01b_configs.jsonl).  Timing: wall clock
 around synchronous C-ABI calls (every call ends with a stream synchronise)."""
 
@@ -140,6 +140,50 @@ def c5_fitc():
         first_add_data_s=t_first, update_s=t_up, grad_s=t_gr, eval_s=t_up + t_gr,
         eff_fp64_tflops_8M2N=8.0*p*p*n/(t_up + t_gr)/1e12, predict_points_per_s=len(Xs)/t_pr, lZ=lZ,
         dlZ_finite=bool(np.all(np.isfinite(dlZ))))
+
+
+def card():
+    import subprocess
+    q = 'name,power.limit,clocks.sm,clocks.max.sm'
+    return subprocess.check_output(['nvidia-smi', '--query-gpu=' + q, '--format=csv,noheader']).decode().strip()
+
+
+def c5_fitc_pseudo():
+    """The C5-fitc shape with d lZ / d U: loglikelihood(True) and loglikelihood(True, pseudoinputs=True)
+    alternating, then one profiled call for the contraction kernel's own time (the only PC_GRAM launch
+    of a gradient call)."""
+    n, p, d = 1 << 20, 2048, 8
+    X, y = problem(n, d)
+    U = np.random.RandomState(3).rand(p, d)
+    gp = pygp.inference.FITC(pygp.likelihoods.Gaussian(0.1), pygp.kernels.SE(1.0, [0.6]*d), 0.0, U)
+    gp.add_data(X, y)
+    gp.loglikelihood(True)
+    gp.loglikelihood(True, pseudoinputs=True)
+    t_hyp, t_pse = [], []
+    for _ in range(4):
+        t0 = time.perf_counter()
+        gp.loglikelihood(True)
+        t_hyp.append(time.perf_counter() - t0)
+        t0 = time.perf_counter()
+        gp.loglikelihood(True, pseudoinputs=True)
+        t_pse.append(time.perf_counter() - t0)
+    ctx = _lib.context()
+    ctx.profile(True)
+    gp.loglikelihood(True, pseudoinputs=True)
+    launches, kern_ms, _ = ctx.profile_read(1)        # PC_GRAM: pseudo_gram_kernel
+    ctx.profile(False)
+    # algorithmic bytes: Bt and T2 once (n x p doubles each) plus Cuu, the inputs and alpha, q
+    nbytes = 16.0*n*p + 8.0*p*p + 8.0*(n + p)*d + 16.0*n
+    # FP64 operations per (pseudo-input, column) entry, counted from the SE instantiation's source: weight 5,
+    # distance 3 d, exp 11, gradient 4 d
+    flops = (16.0 + 7*d)*p*(n + p)
+    hbm_ms, fp64_ms = nbytes/7.7e12*1e3, flops/33.7e12*1e3   # data-sheet HBM3e; measured DFMA (profiles/fp64_peak.json)
+    say(config='C5-fitc-pseudo', workload='FITC SE-ARD d=8, M=2048, N=2^20: loglikelihood(True) vs loglikelihood(True, pseudoinputs=True), alternating',
+        card=card(), grad_s=sorted(t_hyp), grad_pseudo_s=sorted(t_pse),
+        added_ms_median=(float(np.median(t_pse)) - float(np.median(t_hyp)))*1e3,
+        pseudo_kernel_launches=launches, pseudo_kernel_ms=kern_ms, algorithmic_gb=nbytes/1e9, fp64_gflop=flops/1e9,
+        hbm_bound_ms=hbm_ms, fp64_bound_ms=fp64_ms, bound='fp64' if fp64_ms > hbm_ms else 'hbm',
+        share_of_bound=max(hbm_ms, fp64_ms)/kern_ms, target_added_ms=20.0)
 
 
 def next_rows():
