@@ -84,7 +84,8 @@ int  pgp_ctx_sync(pgp_ctx* ctx);
 /* kernels launched by this context since creation (bench.py gpu_launches) */
 int64_t pgp_ctx_launch_count(pgp_ctx* ctx);
 /* per-class device timing with CUDA events on the context stream.
- * classes: 0 gemm(DMMA) 1 gram 2 trace 3 potrf_base 4 trsm_base 5 other */
+ * classes: 0 gemm(DMMA) 1 gram 2 trace 3 potrf_base (and the panel chain of the rank-m
+ * update) 4 trsm_base (and the rows the rank-m update applies a panel to) 5 other */
 #define PGP_PROF_CLASSES 6
 int  pgp_ctx_profile(pgp_ctx* ctx, int enable);    /* enable also resets */
 int  pgp_ctx_profile_read(pgp_ctx* ctx, int cls, int64_t* launches,
@@ -256,6 +257,16 @@ int pgp_dtc_create(pgp_ctx* ctx, const pgp_kernel_spec* spec,
                    pgp_fitc** out);
 /* FITC._update (fitc.py:66-100) */
 int pgp_fitc_update(pgp_fitc* f, const double* hyp);
+/* GP.add_data of n_new rows onto a factored FITC / DTC handle (the reference has no incremental
+ * FITC update and refactors on all the data): append the rows AND update the factors by them in
+ * O(n_new p^2), independent of n -- Lc and the existing rows of the state do not change, the two
+ * p x p factors take a rank-n_new update (pgp_dev_chol_update).  Hypers and pseudo-inputs unchanged.
+ * 1 <= n_new <= pgp_fitc_inc_max_rows() (PGP_E_ARG otherwise, before any state is touched);
+ * PGP_E_STATE if the handle is not factored.  On any failure the handle is left unfactored, with
+ * its previous rows: the caller refactors from its own copy of the data. */
+int pgp_fitc_append_inc(pgp_fitc* f, const double* X, const double* y, int64_t n_new);
+/* the largest n_new pgp_fitc_append_inc and pgp_dev_chol_update accept */
+int pgp_fitc_inc_max_rows(void);
 /* FITC.loglikelihood(grad) (fitc.py:167-232) */
 int pgp_fitc_loglike(pgp_fitc* f, int want_grad, double* lZ, double* dlZ);
 /* lZ, dlZ (nhyper + 2, as pgp_fitc_loglike with want_grad = 1) and dU = dlZ / dU (p, ndim, row-major
@@ -298,6 +309,12 @@ int pgp_dev_copy2d(pgp_ctx* ctx, void* d_dst, int64_t dpitch, const void* d_src,
 /* in-place lower Cholesky of a device matrix (n, n) row-major with `extra`
  * further rows below it that receive the same right-solves (row n = r -> a). */
 int pgp_dev_potrf(pgp_ctx* ctx, double* d_F, int64_t n, int64_t ld, int64_t extra);
+/* in-place rank-m update of a lower factor, as pgp_dev_potrf leaves it: rows 0..n-1 of d_F hold L,
+ * rows n..n+extra-1 riding rows z_r = L^-1 g_r.  d_W (m, ldw), 1 <= m <= pgp_fitc_inc_max_rows():
+ * columns 0..n-1 the update vectors, column n + r the coefficients c_r of riding row r.  Afterwards
+ * L' L'^T = L L^T + W[:, :n]^T W[:, :n] and z_r' = L'^-1 (g_r + W[:, :n]^T c_r); d_W is overwritten. */
+int pgp_dev_chol_update(pgp_ctx* ctx, double* d_F, int64_t n, int64_t ld, int64_t extra,
+                        double* d_W, int64_t ldw, int64_t m);
 
 /* the short FP64 elementary functions of the covariance epilogues (csrc/fastmath.cuh),
  * elementwise on host arrays, for their accuracy sweep against libm

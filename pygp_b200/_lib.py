@@ -102,6 +102,8 @@ SIGNATURES = {
     'pgp_dtc_create': (C.c_int, [_vp, _sp, _dp, _i64, _dp, _dp, _i64, C.POINTER(_vp)]),
     'pgp_fitc_destroy': (None, [_vp]),
     'pgp_fitc_update': (C.c_int, [_vp, _dp]),
+    'pgp_fitc_append_inc': (C.c_int, [_vp, _dp, _dp, _i64]),
+    'pgp_fitc_inc_max_rows': (C.c_int, []),
     'pgp_fitc_loglike': (C.c_int, [_vp, C.c_int, _dp, _dp]),
     'pgp_fitc_loglike_pseudo': (C.c_int, [_vp, _dp, _dp, _dp]),
     'pgp_fitc_set_pseudoinputs': (C.c_int, [_vp, _dp]),
@@ -115,6 +117,7 @@ SIGNATURES = {
     'pgp_dev_trsm': (C.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, C.c_int]),
     'pgp_dev_copy2d': (C.c_int, [_vp, _vp, _i64, _vp, _i64, _i64, _i64]),
     'pgp_dev_potrf': (C.c_int, [_vp, _vp, _i64, _i64, _i64]),
+    'pgp_dev_chol_update': (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, _i64]),
     'pgp_dev_fastmath': (C.c_int, [_vp, C.c_int, _dp, _i64, _dp]),
 }
 

@@ -1646,6 +1646,20 @@ extern "C" int pgp_dev_potrf(pgp_ctx* ctx, double* d_F, int64_t n, int64_t ld, i
     return h;
 }
 
+extern "C" int pgp_dev_chol_update(pgp_ctx* ctx, double* d_F, int64_t n, int64_t ld, int64_t extra, double* d_W,
+                                   int64_t ldw, int64_t m) {
+    if (!ctx) return PGP_E_ARG;
+    if (!d_F || !d_W || n < 0 || extra < 0 || m < 1 || m > kIncRows || ld < n || ldw < n + extra)
+        return ctx->fail(PGP_E_ARG, "bad argument (1 <= m <= pgp_fitc_inc_max_rows())");
+    PGP_TRY(set_device(ctx));
+    Mat F, W;
+    F.p = d_F; F.ld = ld;
+    W.p = d_W; W.ld = ldw;
+    PGP_TRY(chol_update_lower(ctx, F, n, extra, W, m));
+    PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
 extern "C" int pgp_dev_fastmath(pgp_ctx* ctx, int which, const double* x, int64_t n, double* out) {
     if (!ctx) return PGP_E_ARG;
     if (!x || !out || n < 0 || which < 0 || which > 4) return ctx->fail(PGP_E_ARG, "bad argument");

@@ -1000,4 +1000,205 @@ int launch_extract_upper(pgp_ctx* ctx, const double* F, int64_t ld, int64_t n, d
     return check_launch(ctx, "extract_upper_kernel");
 }
 
+// ---- rank-m Cholesky update: L' L'^T = L L^T + W^T W -----------------------------------------------
+//
+// QR of M = [L^T; W] ((n + m) x n, M^T M = L L^T + W^T W): Q^T M = [L'^T; 0].  Reflector k acts on row k
+// of L^T (= column k of L) and the m rows of W, and is chosen from column k of M, (L_kk, W[:, k]):
+//     H (alpha, x) = (nrm, 0),  nrm = sqrt(alpha^2 + |x|^2) > 0 (so L'_kk > 0),
+//     H = I - 2 v v^T / (v^T v),  v = (alpha - nrm, x).
+// alpha = L_kk > 0, so alpha - nrm = -|x|^2 / (alpha + nrm) is formed without cancellation.  v is scaled by
+// mu = 2^e, e = ilogb(max |x_i|) (as LAPACK's dlarfg scales; a power of two, so the scaling is exact and
+// costs no division in the column chain): xs = x / mu, s = |xs|^2 in [1, 4m],
+//     v~ = v / mu = (v0, xs),   v0 = -mu s / (alpha + nrm),   tau = 2 / (v0^2 + s) in (0, 2],
+// so nothing of order 1/|x| is formed: entries of x far below alpha (kernel values of points many
+// length-scales away, down to the bottom of the double range) neither overflow nor lose accuracy.  For
+// |x| << alpha the reflector is not close to the identity: it reflects the W block about xs
+// (I - 2 xs xs^T / s) and leaves L_jk almost unchanged.  Applied to the entries (a, w) = (L_jk, W[:, j]) of a
+// later column j of M (row j of L with its m-vector):
+//     q = v0 a + xs.w,     a' = a - tau q v0,     w' = w - tau q xs.
+// mu = 0 is the identity (tau = 0).
+// Reflector k only touches L_jk (one entry of row j) and W[:, j]; L_kk itself is touched by reflector k
+// alone, so every row j is independent of the others once reflectors 0 .. j-1 are known.
+//
+// Riding rows: a row z = L^-1 g below the factor (potrf_lower's right-hand sides) with coefficients c
+// (W[:, n + r]) is one more column [z; c] of the same transform.  M^T [z; c] = L z + W^T c = g + W^T c =: g';
+// with Q orthogonal, M^T [z; c] = (Q^T M)^T Q^T [z; c] = [L' 0] [z'; c''] = L' z', so the transformed top
+// part is z' = L'^-1 g': the riding rows are rows like any other, applying every reflector, no pivot.
+//
+// Schedule per 64-column panel: one CTA generates the panel's 64 reflectors from the panel's own rows (a
+// dependent chain, one __syncthreads per column), then every row below the panel (and every riding row)
+// applies those 64 reflectors to its 64 entries and its m-vector.  m-vectors are spread over a group of
+// G lanes (2 entries per lane, G = the power of two with 2 G >= m), so x.w is G-lane shuffle sum.
+constexpr int kUpdPanelThreads = 1024;
+constexpr int kUpdApplyThreads = 128;
+constexpr int kUpdChunk = 8;           // L entries of a row loaded ahead of the reflector chain
+
+__device__ __forceinline__ double group_sum(double v, int G) {
+    for (int o = G >> 1; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// panel [k0, k0 + nb): reflectors into refl ((nb, kIncRows) scaled vectors xs) and scal ((nb, 2): v0, tau),
+// the panel's rows updated in place, L'_kk = nrm.  Each lane group owns rows grp and grp + groups of the panel.
+// The diagonal block is staged in shared memory, so the 64-step chain waits on no global load.
+__global__ void __launch_bounds__(kUpdPanelThreads) chol_update_panel_kernel(double* F, int64_t ld, int64_t k0, int nb,
+                                                                              const double* W, int64_t ldw, int m,
+                                                                              int G, double* refl, double* scal) {
+    __shared__ double xs[2][kIncRows];      // the pivot row's m-vector, double-buffered by column parity
+    __shared__ double Ls[kNB][kNB + 1];     // the diagonal block (lower triangle)
+    __shared__ double nrm_s[kNB];           // the new diagonal (the old one is alpha of each step)
+    const int lg = threadIdx.x & (G - 1), grp = threadIdx.x / G, groups = blockDim.x / G;
+    for (int idx = threadIdx.x; idx < nb * kNB; idx += blockDim.x) {
+        const int r = idx / kNB, c = idx - r * kNB;
+        if (c <= r) Ls[r][c] = F[(k0 + r) * ld + k0 + c];
+    }
+    double w[2][2];
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {
+        const int j = grp + r * groups;
+#pragma unroll
+        for (int t = 0; t < 2; ++t) {
+            const int i = lg + t * G;
+            w[r][t] = (j < nb && i < m) ? W[(int64_t)i * ldw + k0 + j] : 0.0;
+        }
+    }
+    if (grp == 0) {
+        xs[0][lg] = w[0][0];
+        xs[0][lg + G] = w[0][1];
+    }
+    __syncthreads();
+    for (int kk = 0; kk < nb; ++kk) {
+        const int b = kk & 1;
+        const double y0 = xs[b][lg], y1 = xs[b][lg + G];
+        const double alpha = Ls[kk][kk];                       // the diagonal is rewritten after the loop
+        double ym = fmax(fabs(y0), fabs(y1));
+        for (int o = G >> 1; o > 0; o >>= 1) ym = fmax(ym, __shfl_xor_sync(0xffffffffu, ym, o));
+        const int e = ym > 0.0 ? ilogb(ym) : 0;
+        const double mu = ym > 0.0 ? scalbn(1.0, e) : 0.0;
+        const double x0 = scalbn(y0, -e), x1 = scalbn(y1, -e);
+        double s = x0 * x0 + x1 * x1;
+        double d0 = x0 * w[0][0] + x1 * w[0][1];
+        double d1 = x0 * w[1][0] + x1 * w[1][1];
+        for (int o = G >> 1; o > 0; o >>= 1) {
+            s += __shfl_xor_sync(0xffffffffu, s, o);
+            d0 += __shfl_xor_sync(0xffffffffu, d0, o);
+            d1 += __shfl_xor_sync(0xffffffffu, d1, o);
+        }
+        const int ec = max(ilogb(alpha), e);                   // sqrt(alpha^2 + mu^2 s) without overflow
+        const double ac = scalbn(alpha, -ec), mc = scalbn(mu, -ec);
+        const double nrm = scalbn(sqrt(ac * ac + mc * mc * s), ec);
+        const double v0 = -(mu * s) / (alpha + nrm);
+        const double tau = mu > 0.0 ? 2.0 / (v0 * v0 + s) : 0.0;
+        if (grp == 0) {
+            refl[(int64_t)kk * kIncRows + lg] = x0;
+            refl[(int64_t)kk * kIncRows + lg + G] = x1;
+            if (lg == 0) {
+                scal[kk * 2 + 0] = v0;
+                scal[kk * 2 + 1] = tau;
+            }
+        }
+        double a[2];                                           // every lane of the group reads before lane 0 writes
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {
+            const int j = grp + r * groups;
+            a[r] = (j > kk && j < nb) ? Ls[j][kk] : 0.0;
+        }
+        __syncwarp();
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {
+            const int j = grp + r * groups;
+            if (j > kk && j < nb) {
+                const double t = tau * (v0 * a[r] + (r ? d1 : d0));
+                if (lg == 0) Ls[j][kk] = a[r] - t * v0;
+                w[r][0] -= t * x0;
+                w[r][1] -= t * x1;
+            }
+        }
+        const int nx = kk + 1;                                 // the next pivot publishes its m-vector
+        if (nx < nb && grp == nx % groups) {
+            const int r = nx / groups;
+            xs[b ^ 1][lg] = r ? w[1][0] : w[0][0];
+            xs[b ^ 1][lg + G] = r ? w[1][1] : w[0][1];
+        }
+        if (threadIdx.x == 0) nrm_s[kk] = nrm;
+        __syncthreads();
+    }
+    if (threadIdx.x < nb) Ls[threadIdx.x][threadIdx.x] = nrm_s[threadIdx.x];
+    __syncthreads();
+    for (int idx = threadIdx.x; idx < nb * kNB; idx += blockDim.x) {
+        const int r = idx / kNB, c = idx - r * kNB;
+        if (c <= r) F[(k0 + r) * ld + k0 + c] = Ls[r][c];
+    }
+}
+
+// rows [r0, r1) (below the panel, riding rows included) apply the panel's reflectors; one lane group per row
+__global__ void __launch_bounds__(kUpdApplyThreads) chol_update_apply_kernel(double* F, int64_t ld, int64_t k0, int nb,
+                                                                              int64_t r0, int64_t r1, double* W,
+                                                                              int64_t ldw, int m, int G,
+                                                                              const double* __restrict__ refl,
+                                                                              const double* __restrict__ scal) {
+    const int lg = threadIdx.x & (G - 1);
+    const int64_t j = r0 + ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
+    const bool valid = j < r1;                  // invalid lanes still join the group shuffles
+    double w0 = (valid && lg < m) ? W[(int64_t)lg * ldw + j] : 0.0;
+    double w1 = (valid && lg + G < m) ? W[(int64_t)(lg + G) * ldw + j] : 0.0;
+    double* row = F + (valid ? j : r0) * ld + k0;
+    for (int c0 = 0; c0 < nb; c0 += kUpdChunk) {
+        double av[kUpdChunk];
+#pragma unroll
+        for (int u = 0; u < kUpdChunk; ++u) av[u] = (valid && c0 + u < nb) ? row[c0 + u] : 0.0;
+#pragma unroll
+        for (int u = 0; u < kUpdChunk; ++u) {
+            const int kk = c0 + u;
+            if (kk < nb) {
+                const double x0 = __ldg(refl + (int64_t)kk * kIncRows + lg);
+                const double x1 = __ldg(refl + (int64_t)kk * kIncRows + lg + G);
+                const double v0 = __ldg(scal + kk * 2), tau = __ldg(scal + kk * 2 + 1);
+                const double d = group_sum(x0 * w0 + x1 * w1, G);
+                const double t = tau * (v0 * av[u] + d);
+                w0 -= t * x0;
+                w1 -= t * x1;
+                av[u] -= t * v0;
+            }
+        }
+        if (valid && lg == 0) {
+#pragma unroll
+            for (int u = 0; u < kUpdChunk; ++u)
+                if (c0 + u < nb) row[c0 + u] = av[u];
+        }
+    }
+    if (valid && lg < m) W[(int64_t)lg * ldw + j] = w0;
+    if (valid && lg + G < m) W[(int64_t)(lg + G) * ldw + j] = w1;
+}
+
+int chol_update_lower(pgp_ctx* ctx, const Mat& F, int64_t n, int64_t extra, const Mat& W, int64_t m) {
+    if (n <= 0 || m <= 0) return 0;
+    if (m > kIncRows) return ctx->fail(PGP_E_ARG, "chol_update_lower: more update rows than kIncRows");
+    int G = 1;
+    while (2 * G < m) G <<= 1;
+    double* refl = nullptr;                     // (kNB, kIncRows) reflector vectors, then (kNB, 2) scalars
+    PGP_TRY(dev_alloc(ctx, &refl, (size_t)kNB * kIncRows + 2 * kNB));
+    double* scal = refl + (size_t)kNB * kIncRows;
+    const int pthreads = std::min(kUpdPanelThreads, kNB * G);
+    int rc = 0;
+    for (int64_t k0 = 0; k0 < n && !rc; k0 += kNB) {
+        const int nb = (int)std::min<int64_t>(kNB, n - k0);
+        {
+            Launch L(ctx, PC_POTRF, 4.0 * nb * nb * m);
+            chol_update_panel_kernel<<<1, pthreads, 0, ctx->stream>>>(F.p, F.ld, k0, nb, W.p, W.ld, (int)m, G, refl,
+                                                                      scal);
+            rc = check_launch(ctx, "chol_update_panel_kernel");
+        }
+        const int64_t r0 = k0 + nb, r1 = n + extra;
+        if (rc || r0 >= r1) continue;
+        Launch L(ctx, PC_TRSM, 4.0 * nb * (double)(r1 - r0) * m);    // applies the panel to the rows below it
+        const unsigned blocks = (unsigned)ceil_div((r1 - r0) * G, kUpdApplyThreads);
+        chol_update_apply_kernel<<<blocks, kUpdApplyThreads, 0, ctx->stream>>>(F.p, F.ld, k0, nb, r0, r1, W.p, W.ld,
+                                                                              (int)m, G, refl, scal);
+        rc = check_launch(ctx, "chol_update_apply_kernel");
+    }
+    dev_free(ctx, refl);                        // stream-ordered reuse: safe before the kernels finish
+    return rc;
+}
+
 }  // namespace pgp

@@ -24,6 +24,14 @@ struct Mat {
 // style index of the first non-positive pivot (0 = ok).
 int potrf_lower(pgp_ctx* ctx, const Mat& F, int64_t n, int64_t extra, int* d_info);
 
+// Rank-m update of a factor in place: rows 0..n-1 of F hold L (lower), rows n..n+extra-1 riding rows
+// z_r = L^-1 g_r (as potrf_lower leaves them).  W: m <= kIncRows rows of width n + extra, columns [0, n) the
+// update vectors, column n + r riding row r's coefficients c_r.  Afterwards L' L'^T = L L^T + W[:, :n]^T W[:, :n]
+// and z_r' = L'^-1 (g_r + W[:, :n]^T c_r).  W is overwritten (scratch); the strict upper triangle of F is
+// not touched.  Householder QR of [L^T; W] in 64-column panels (chol.cu), O((n + extra) n m) FP64 FMAs.
+constexpr int kIncRows = 64;
+int chol_update_lower(pgp_ctx* ctx, const Mat& F, int64_t n, int64_t extra, const Mat& W, int64_t m);
+
 // row n of every batch member <- L^-1 (row n): a = L^-1 r as a separate batched
 // forward substitution (the batched small-N path; n <= 20480).
 int launch_trsv_lower(pgp_ctx* ctx, const Mat& F, int64_t n);

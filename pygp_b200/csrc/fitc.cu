@@ -41,6 +41,7 @@ struct pgp_fitc {
     pgp_kernel_spec spec;
     int ndim = 0;
     int64_t n = 0, p = 0, ldp = 0;
+    int64_t cap = 0;                // row capacity of every (n)-sized buffer (pgp_fitc_append_inc grows it)
     double *d_X = nullptr, *d_y = nullptr, *d_U = nullptr;
     double *d_ZX = nullptr, *d_ZU = nullptr;
     DevSpec* d_spec = nullptr;      // [0]: sn2 = noise; [1]: sn2 = su2 (Kuu jitter of fitc.py:68)
@@ -61,8 +62,11 @@ struct pgp_fitc {
     int* d_info = nullptr;
     double* d_pred = nullptr;       // (2, pc_rows, ldp) predict chunk
     int64_t pc_rows = 0;
+    double* d_lzs = nullptr;        // [0] sum log ell, [1] sum rs^2 over the n rows (lZ of an append)
+    double* d_inc = nullptr;        // append scratch: 2 x (kIncRows, ldw) update rows, scaled new inputs
     DevSpec hspec[2];
     bool factored = false;
+    bool zx_stale = false;          // d_ZX lacks appended rows (or has the stride of an older n)
     double lZ = 0.0;
 };
 
@@ -231,8 +235,10 @@ __global__ void rank1_sub_kernel(double* C, int64_t ld, int64_t p, const double*
 }
 
 // lZ = -sum log diag(Al) - sum log ell - 1/2 (rs.rs - beta.beta) - n/2 log 2 pi   (fitc.py:191-193)
+// The O(n) sums are carried in sums[0] = sum log ell, sums[1] = sum rs^2: rows [r0, n) are summed here and
+// replace (r0 == 0) or add to (an append of rows r0 .. n-1) the carried sums, so an append costs O(p + m).
 __global__ void fitc_lz_kernel(const double* A, int64_t ld, int64_t p, const double* ell, const double* rs,
-                               int64_t n, double* out) {
+                               int64_t r0, int64_t n, double* sums, double* out) {
     __shared__ double red[32];
     double sd = 0.0, sb = 0.0, sl = 0.0, sr = 0.0;
     for (int64_t j = threadIdx.x; j < p; j += blockDim.x) {
@@ -240,7 +246,7 @@ __global__ void fitc_lz_kernel(const double* A, int64_t ld, int64_t p, const dou
         double b = A[p * ld + j];
         sb += b * b;
     }
-    for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
+    for (int64_t i = r0 + threadIdx.x; i < n; i += blockDim.x) {
         sl += log(ell[i]);
         sr += rs[i] * rs[i];
     }
@@ -248,7 +254,39 @@ __global__ void fitc_lz_kernel(const double* A, int64_t ld, int64_t p, const dou
     sb = block_sum(sb, red);
     sl = block_sum(sl, red);
     sr = block_sum(sr, red);
-    if (threadIdx.x == 0) out[0] = -sd - sl - 0.5 * (sr - sb) - 0.5 * (double)n * log(2 * kPi);
+    if (threadIdx.x == 0) {
+        if (r0 > 0) {
+            sl += sums[0];
+            sr += sums[1];
+        }
+        sums[0] = sl;
+        sums[1] = sr;
+        out[0] = -sd - sl - 0.5 * (sr - sb) - 0.5 * (double)n * log(2 * kPi);
+    }
+}
+
+// update rows of an append, one warp per new row i (Kxu_i in W2 on entry):
+//   W1_i = [Vs_i | rs_i]                          -> Al Al^T += Vs_i^T Vs_i,  beta rides with c = rs_i
+//   W2_i = [Kxu_i / ell_i | rs_i]      (FITC)     -> Rl Rl^T = Kuu + su2 I + Kux diag(1/ell^2) Kxu,  b = Rl^-1 Kux (r/ell^2)
+//   W2_i = [Kxu_i / sqrt(sn2) | sn2 rs_i] (DTC)   -> Rux Rux^T = Kuu + su2 I + Kux Kxu / sn2,  b = Rux^-1 Kux r
+// (DTC: ell = sqrt(sn2), so the coefficient sn2 rs_i = sqrt(sn2) r_i makes W2^T c = Kux_new r_new)
+__global__ void fitc_inc_pack_kernel(const double* Vs, int64_t ld, int64_t m, int64_t p, const double* ell,
+                                     const double* rs, double* W1, double* W2, int64_t ldw, int dtc) {
+    const int lane = threadIdx.x & 31;
+    const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (row >= m) return;
+    const double l = ell[row], r = rs[row];
+    const double* v = Vs + row * ld;
+    double* w1 = W1 + row * ldw;
+    double* w2 = W2 + row * ldw;
+    for (int64_t k = lane; k < p; k += 32) {
+        w1[k] = v[k];
+        w2[k] = w2[k] / l;
+    }
+    if (lane == 0) {
+        w1[p] = r;
+        w2[p] = dtc ? r * l * l : r;
+    }
 }
 
 // scalar sums of the gradient (fitc.py:203-210, 219-230) and its first/last entries.
@@ -450,13 +488,77 @@ void fitc_free(pgp_fitc* f) {
     dev_free_null(ctx, f->d_pred);
     double** small[] = {&f->d_X, &f->d_y, &f->d_U, &f->d_ZX, &f->d_ZU, &f->d_L, &f->d_A, &f->d_R, &f->d_ell,
                         &f->d_rs, &f->d_c, &f->d_alpha, &f->d_q, &f->d_cw, &f->d_bb, &f->d_a, &f->d_b, &f->d_t,
-                        &f->d_w, &f->d_P, &f->d_Cuu, &f->d_VW, &f->d_part, &f->d_res};
+                        &f->d_w, &f->d_P, &f->d_Cuu, &f->d_VW, &f->d_part, &f->d_res, &f->d_lzs, &f->d_inc};
     for (double** q : small) {
         dev_free(ctx, *q);
         *q = nullptr;
     }
     dev_free(ctx, f->d_spec);
     dev_free(ctx, f->d_info);
+}
+
+inline int64_t kc_rows_for(int64_t rows, int64_t ldp) {
+    return std::min<int64_t>(rows, std::max<int64_t>(1024, ((int64_t)1 << 30) / (ldp * 8)));
+}
+
+// Row capacity for n rows.  Every (n)-sized buffer has f->cap rows (exact fit at create); when an append
+// outgrows it, the buffers are reallocated with n / 8 + 256 rows of slack (at most ~1 GiB of extra rows
+// per (n, ldp) buffer, at least 256), as pgp_exact_append_inc does, so a loop adding one datum at a time
+// reallocates once in hundreds of steps.  The first n rows of X, y, Vs, ell, rs, c move over; ZX is
+// rebuilt lazily (zx_stale) and the gradient buffers are allocated again at the new capacity on first use.
+// On failure the handle keeps its old buffers.
+int fitc_reserve(pgp_fitc* f, int64_t n) {
+    if (n <= f->cap) return 0;
+    pgp_ctx* ctx = f->ctx;
+    const int d = f->ndim, np = f->spec.n_parts;
+    const int64_t ldp = f->ldp, n_old = f->n;
+    const int64_t slack = std::min<int64_t>(n / 8 + 256, std::max<int64_t>(256, ((int64_t)1 << 27) / ldp));
+    const int64_t cap = round_up(n + slack, 256);
+    double *X = nullptr, *y = nullptr, *ZX = nullptr, *Vs = nullptr, *ell = nullptr, *rs = nullptr, *c = nullptr,
+           *alpha = nullptr;
+    int rc = 0;
+    auto A = [&](double** q, size_t cnt) { if (!rc) rc = dev_alloc(ctx, q, cnt); };
+    A(&X, (size_t)cap * d); A(&y, cap); A(&ZX, z_doubles(np, d, cap)); A(&Vs, (size_t)cap * ldp);
+    A(&ell, cap); A(&rs, cap); A(&c, cap); A(&alpha, cap);
+    double** fresh[] = {&X, &y, &ZX, &Vs, &ell, &rs, &c, &alpha};
+    if (rc) {
+        for (double** q : fresh) dev_free(ctx, *q);
+        return rc;
+    }
+    cudaStream_t s = ctx->stream;
+    const size_t b = sizeof(double);
+    cudaError_t e = cudaMemcpyAsync(X, f->d_X, b * n_old * d, cudaMemcpyDeviceToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(y, f->d_y, b * n_old, cudaMemcpyDeviceToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(Vs, f->d_Vs, b * n_old * ldp, cudaMemcpyDeviceToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ell, f->d_ell, b * n_old, cudaMemcpyDeviceToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(rs, f->d_rs, b * n_old, cudaMemcpyDeviceToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(c, f->d_c, b * n_old, cudaMemcpyDeviceToDevice, s);
+    if (e != cudaSuccess) {
+        cudaStreamSynchronize(s);
+        for (double** q : fresh) dev_free(ctx, *q);
+        return ctx->cuda_fail(e, "FITC row buffers", __FILE__, __LINE__);
+    }
+    // stream-ordered reuse: the old buffers may go back to the pool before the copies finish
+    std::swap(f->d_X, X); std::swap(f->d_y, y); std::swap(f->d_ZX, ZX); std::swap(f->d_Vs, Vs);
+    std::swap(f->d_ell, ell); std::swap(f->d_rs, rs); std::swap(f->d_c, c); std::swap(f->d_alpha, alpha);
+    for (double** q : fresh) dev_free(ctx, *q);
+    dev_free_null(ctx, f->d_Bt);
+    dev_free_null(ctx, f->d_Wt);
+    dev_free_null(ctx, f->d_T);
+    dev_free_null(ctx, f->d_q);
+    dev_free_null(ctx, f->d_cw);
+    dev_free_null(ctx, f->d_bb);
+    f->cap = cap;
+    f->zx_stale = true;
+    const int64_t kc = kc_rows_for(cap, ldp);        // Kxu chunks follow the data, not the size at create
+    if (kc > f->kc_rows) {
+        double* Kc = nullptr;
+        PGP_TRY(dev_alloc(ctx, &Kc, (size_t)kc * ldp));
+        dev_free(ctx, f->d_Kc);
+        f->d_Kc = Kc;
+        f->kc_rows = kc;
+    }
+    return 0;
 }
 
 }  // namespace
@@ -485,7 +587,8 @@ extern "C" int pgp_fitc_create(pgp_ctx* ctx, const pgp_kernel_spec* spec, const 
     f->ldp = lead_dim(nu);
     const int d = f->ndim, np = spec->n_parts;
     const int64_t p = nu, ldp = f->ldp;
-    f->kc_rows = std::min<int64_t>(n, std::max<int64_t>(1024, ((int64_t)1 << 30) / (ldp * 8)));
+    f->cap = n;                     // exact fit; pgp_fitc_append_inc adds slack when it has to grow
+    f->kc_rows = kc_rows_for(n, ldp);
     int rc = 0;
     auto A = [&](double** q, size_t cnt) { if (!rc) rc = dev_alloc(ctx, q, cnt); };
     A(&f->d_X, (size_t)n * d); A(&f->d_y, n); A(&f->d_U, (size_t)p * d);
@@ -493,7 +596,7 @@ extern "C" int pgp_fitc_create(pgp_ctx* ctx, const pgp_kernel_spec* spec, const 
     A(&f->d_L, (size_t)p * ldp); A(&f->d_A, (size_t)(p + 1) * ldp); A(&f->d_R, (size_t)(p + 1) * ldp);
     A(&f->d_ell, n); A(&f->d_rs, n); A(&f->d_c, n); A(&f->d_alpha, n);
     A(&f->d_a, ldp); A(&f->d_b, ldp); A(&f->d_t, ldp); A(&f->d_w, ldp);
-    A(&f->d_res, (size_t)2 * kMaxHyper + kScal);
+    A(&f->d_res, (size_t)2 * kMaxHyper + kScal); A(&f->d_lzs, 2);
     if (!rc) rc = dev_alloc(ctx, &f->d_spec, 2);
     if (!rc) rc = dev_alloc(ctx, &f->d_info, 4);
     if (!rc) rc = dev_alloc(ctx, &f->d_Vs, (size_t)n * ldp);
@@ -545,6 +648,7 @@ extern "C" int pgp_fitc_update(pgp_fitc* f, const double* hyp) {
     PGP_CUDA(ctx, cudaMemcpyAsync(f->d_spec, f->hspec, sizeof(DevSpec) * 2, cudaMemcpyHostToDevice, s));
     PGP_CUDA(ctx, cudaMemsetAsync(f->d_info, 0, sizeof(int) * 4, s));
     PGP_TRY(launch_scale(ctx, f->d_spec, f->d_X, n, d, np, f->d_ZX, 1));
+    f->zx_stale = false;
     PGP_TRY(launch_scale(ctx, f->d_spec, f->d_U, p, d, np, f->d_ZU, 1));
     const int st = single_type(&f->spec);
 
@@ -629,10 +733,12 @@ extern "C" int pgp_fitc_update(pgp_fitc* f, const double* hyp) {
         PGP_CUDA(ctx, cudaMemcpyAsync(f->d_b, f->d_a, sizeof(double) * p, cudaMemcpyDeviceToDevice, s));
         Mat bv; bv.p = f->d_b; bv.ld = ldp;
         PGP_TRY(trsm_right_lt(ctx, bv, 1, R, p));
+        // b also rides as row p of Rl (DTC: it was formed there), for the rank updates of pgp_fitc_append_inc
+        PGP_CUDA(ctx, cudaMemcpyAsync(f->d_R + p * ldp, f->d_b, sizeof(double) * p, cudaMemcpyDeviceToDevice, s));
     }
     {
         Launch Lc(ctx, PC_OTHER, 16.0 * n);
-        fitc_lz_kernel<<<1, 1024, 0, s>>>(f->d_A, ldp, p, f->d_ell, f->d_rs, n, f->d_res);
+        fitc_lz_kernel<<<1, 1024, 0, s>>>(f->d_A, ldp, p, f->d_ell, f->d_rs, 0, n, f->d_lzs, f->d_res);
         PGP_TRY(check_launch(ctx, "fitc_lz_kernel"));
     }
     double* hp = ctx->h_pin;
@@ -653,6 +759,92 @@ extern "C" int pgp_fitc_update(pgp_fitc* f, const double* hyp) {
     return 0;
 }
 
+extern "C" int pgp_fitc_inc_max_rows(void) { return kIncRows; }
+
+// GP.add_data of m rows onto a factored handle, O(m p^2) and independent of n.  With hypers and U fixed,
+// Lc and the existing rows of Vs, ell, rs do not change, and the two p x p factors take rank-m updates:
+//   Al Al^T = I + Vs^T Vs                          += Vs_new^T Vs_new                 (beta rides, c = rs_new)
+//   Rl Rl^T = Lc A Lc^T = Kuu + su2 I + Kux diag(1/ell^2) Kxu += (Kxu_new/ell)^T (Kxu_new/ell)  (b, c = rs_new)
+//   DTC: Rux Rux^T = Kuu + su2 I + Kux Kxu / sn2   += Kxu_new^T Kxu_new / sn2          (b, c = sqrt(sn2) r_new)
+// (fitc_inc_pack_kernel, chol_update_lower).  lZ follows from the carried sums (fitc_lz_kernel).
+extern "C" int pgp_fitc_append_inc(pgp_fitc* f, const double* X, const double* y, int64_t n_new) {
+    if (!f) return PGP_E_ARG;
+    pgp_ctx* ctx = f->ctx;
+    if (!X || !y || n_new < 1 || n_new > kIncRows)
+        return ctx->fail(PGP_E_ARG, "null argument or n_new outside [1, pgp_fitc_inc_max_rows()]");
+    if (!f->factored) return ctx->fail(PGP_E_STATE, "incremental update before a successful update");
+    PGP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const int d = f->ndim, np = f->spec.n_parts;
+    const int64_t n_old = f->n, m = n_new, n = n_old + m, p = f->p, ldp = f->ldp, ldw = lead_dim(p + 1);
+    cudaStream_t s = ctx->stream;
+    // a failure leaves the handle unfactored with its n_old rows (the rows past n_old are not data yet):
+    // the host drops it and refactors from its own copy, as after a failed pgp_exact_append_inc
+    auto bail = [&](int code) {
+        cudaStreamSynchronize(s);
+        f->factored = false;
+        return code;
+    };
+    int rc = 0;
+    if (!f->d_inc && (rc = dev_alloc(ctx, &f->d_inc, (size_t)2 * kIncRows * ldw + z_doubles(np, d, kIncRows))))
+        return bail(rc);
+    if ((rc = fitc_reserve(f, n))) return bail(rc);
+    double* W1 = f->d_inc;
+    double* W2 = W1 + (size_t)kIncRows * ldw;
+    double* Zs = W2 + (size_t)kIncRows * ldw;
+    double* Vn = f->d_Vs + n_old * ldp;
+    cudaError_t e = cudaMemcpyAsync(f->d_X + n_old * d, X, sizeof(double) * m * d, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(f->d_y + n_old, y, sizeof(double) * m, cudaMemcpyHostToDevice, s);
+    if (e != cudaSuccess) return bail(ctx->cuda_fail(e, "FITC append upload", __FILE__, __LINE__));
+    // Kxu_new = k(X_new, U) (the new rows of Vs, and a copy in W2); Vt_new = Kxu_new Lc^-T   fitc.py:79-84
+    if ((rc = launch_scale(ctx, f->d_spec, f->d_X + n_old * d, m, d, np, Zs, 1))) return bail(rc);
+    GramArgs g;
+    g.spec = f->d_spec;
+    g.Z1 = Zs; g.n1 = m;
+    g.Z2 = f->d_ZU; g.n2 = p;
+    g.ndim = d; g.n_parts = np;
+    g.out = Vn; g.ldo = ldp;
+    g.single_type = single_type(&f->spec);
+    if ((rc = launch_gram(ctx, g))) return bail(rc);
+    e = cudaMemcpy2DAsync(W2, ldw * 8, Vn, ldp * 8, p * 8, m, cudaMemcpyDeviceToDevice, s);
+    if (e != cudaSuccess) return bail(ctx->cuda_fail(e, "FITC append copy", __FILE__, __LINE__));
+    Mat L; L.p = f->d_L; L.ld = ldp;
+    Mat V; V.p = Vn; V.ld = ldp;
+    if ((rc = trsm_right_lt(ctx, V, m, L, p))) return bail(rc);
+    {
+        Launch Lc(ctx, PC_OTHER, 16.0 * m * p);
+        fitc_ell_kernel<<<warp_rows_grid(m), 256, 0, s>>>(Vn, ldp, m, p, f->d_y + n_old, f->d_spec, f->d_ell + n_old,
+                                                          f->d_rs + n_old, f->d_c + n_old, f->dtc);
+        if ((rc = check_launch(ctx, "fitc_ell_kernel"))) return bail(rc);
+    }
+    {
+        Launch Lc(ctx, PC_OTHER, 24.0 * m * p);
+        fitc_inc_pack_kernel<<<warp_rows_grid(m), 256, 0, s>>>(Vn, ldp, m, p, f->d_ell + n_old, f->d_rs + n_old, W1, W2,
+                                                               ldw, f->dtc);
+        if ((rc = check_launch(ctx, "fitc_inc_pack_kernel"))) return bail(rc);
+    }
+    Mat A; A.p = f->d_A; A.ld = ldp;
+    Mat R; R.p = f->d_R; R.ld = ldp;
+    Mat M1; M1.p = W1; M1.ld = ldw;
+    Mat M2; M2.p = W2; M2.ld = ldw;
+    if ((rc = chol_update_lower(ctx, A, p, 1, M1, m))) return bail(rc);
+    if ((rc = chol_update_lower(ctx, R, p, 1, M2, m))) return bail(rc);
+    e = cudaMemcpyAsync(f->d_b, f->d_R + p * ldp, sizeof(double) * p, cudaMemcpyDeviceToDevice, s);
+    if (e != cudaSuccess) return bail(ctx->cuda_fail(e, "FITC append copy", __FILE__, __LINE__));
+    {
+        Launch Lc(ctx, PC_OTHER, 16.0 * (p + m));
+        fitc_lz_kernel<<<1, 1024, 0, s>>>(f->d_A, ldp, p, f->d_ell, f->d_rs, n_old, n, f->d_lzs, f->d_res);
+        if ((rc = check_launch(ctx, "fitc_lz_kernel"))) return bail(rc);
+    }
+    double* hp = ctx->h_pin;
+    e = cudaMemcpyAsync(hp, f->d_res, sizeof(double), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) return bail(ctx->cuda_fail(e, "FITC incremental update", __FILE__, __LINE__));
+    f->n = n;
+    f->lZ = hp[0];
+    f->zx_stale = true;                 // ZX has the stride of n_old and lacks the new rows
+    return 0;
+}
+
 // enqueue the gradient of lZ (fitc.py:167-232): dlZ lands in d_res[1 .. nk + 2], and Cuu, Bt, T2, alpha, q
 // (FITC) and w stay resident for pgp_fitc_loglike_pseudo
 static int fitc_grad_launch(pgp_fitc* f) {
@@ -660,13 +852,17 @@ static int fitc_grad_launch(pgp_fitc* f) {
     const int nk = f->spec.nhyper, d = f->ndim, np = f->spec.n_parts;
     const int64_t n = f->n, p = f->p, ldp = f->ldp;
     cudaStream_t s = ctx->stream;
-    const size_t np_ = (size_t)n * ldp;
+    const size_t np_ = (size_t)f->cap * ldp;        // row buffers follow the capacity (fitc_reserve)
     if (!f->d_Bt) PGP_TRY(dev_alloc(ctx, &f->d_Bt, np_));
     if (!f->d_Wt) PGP_TRY(dev_alloc(ctx, &f->d_Wt, np_));
     if (!f->d_T) PGP_TRY(dev_alloc(ctx, &f->d_T, np_));
-    if (!f->d_q) PGP_TRY(dev_alloc(ctx, &f->d_q, (size_t)n));
-    if (!f->d_cw) PGP_TRY(dev_alloc(ctx, &f->d_cw, (size_t)n));
-    if (!f->d_bb) PGP_TRY(dev_alloc(ctx, &f->d_bb, (size_t)n));
+    if (!f->d_q) PGP_TRY(dev_alloc(ctx, &f->d_q, (size_t)f->cap));
+    if (!f->d_cw) PGP_TRY(dev_alloc(ctx, &f->d_cw, (size_t)f->cap));
+    if (!f->d_bb) PGP_TRY(dev_alloc(ctx, &f->d_bb, (size_t)f->cap));
+    if (f->zx_stale) {                                 // appended rows: the traces read ZX of all n rows
+        PGP_TRY(launch_scale(ctx, f->d_spec, f->d_X, n, d, np, f->d_ZX, 1));
+        f->zx_stale = false;
+    }
     if (!f->d_P) PGP_TRY(dev_alloc(ctx, &f->d_P, (size_t)p * ldp));
     if (!f->d_Cuu) PGP_TRY(dev_alloc(ctx, &f->d_Cuu, (size_t)p * ldp));
     Mat L; L.p = f->d_L; L.ld = ldp;

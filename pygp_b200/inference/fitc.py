@@ -114,13 +114,36 @@ class FITC(GP):
 
     def _update(self):
         if self._dev is None or self._ndev != self.ndata:
-            # FITC has no incremental update in the reference either (every
-            # add_data re-runs _update on all the data, _base.py:133-141)
+            # new rows that did not go through _updateinc (the reference refactors
+            # on every add_data, _base.py:133-141): upload all the data again
             self._dev = None
             self._dev = _DeviceFITC.create(self._kernel, self._U, self._X, self._y, self._dtc)
             self._ndev = self.ndata
         hyp = _lib.as_f64(self.get_hyper())
         _lib.check(self._dev.ctx, _lib.lib().pgp_fitc_update(self._dev.handle, _lib.ptr(hyp)))
+
+    def _updateinc(self, X, y):
+        """Append rows to a factored device state by rank updates of its p x p
+        factors, O(len(X) p^2) whatever ndata is (pgp_fitc_append_inc; beyond the
+        reference, which refactors on all the data).  At most min(ndata, the
+        library's row cap) rows: past ndata new rows the full update costs less
+        than twice the incremental one, and it is the reference path."""
+        dev = self._dev
+        if dev is None or self._ndev != self.ndata or len(X) > self.ndata:
+            raise NotImplementedError
+        if len(X) > _lib.lib().pgp_fitc_inc_max_rows():
+            raise NotImplementedError
+        Xn, yn = _lib.as_f64(X, 2), _lib.as_f64(y, 1)
+        rc = _lib.lib().pgp_fitc_append_inc(dev.handle, _lib.ptr(Xn), _lib.ptr(yn), len(Xn))
+        if rc == -4:
+            raise NotImplementedError       # not factored (set_pseudoinputs): the full update takes over
+        try:
+            _lib.check(dev.ctx, rc)
+        except Exception:
+            # the handle is unfactored now: drop it, the next _update uploads the host's data again
+            self._dev, self._ndev = None, 0
+            raise
+        self._ndev += len(Xn)
 
     def _ensure_dev(self):
         """Device state of a copy made without a hyper argument (utils/models.py:47-55):
